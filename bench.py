@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ProdSearch embedding-scoring hot path on B200 (contract: see the task brief).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one TEM training step (ItemTransformerRanker.forward_dotproduct + backward + the
 reference's clipped Adam) on BASELINE.json configs[1]: Amazon-Sports-shaped synthetic data,
@@ -337,6 +337,22 @@ def timed(fn, iters, warmup=3):
     e.record()
     torch.cuda.synchronize()
     return s.elapsed_time(e) / iters * 1e-3
+
+
+def dump_outputs(path, loss, model):
+    """What a caller of the timed step receives from its last call: the loss it returned and the parameters it left
+    (the rank's own shards when the tables are row-sharded), each as ``path/<name>.npy`` in float32.  The inputs are
+    seeded and the step is reproducible, so one build writes the same bits on every run with the same arguments, and
+    two builds can be compared array by array."""
+    import numpy as np
+    model.flush_lazy_rows()        # --grad-mode rowsparse: rows the lazily caught-up Adam has not brought current yet
+    arrays = {"loss": loss.detach().float().reshape(-1)}
+    arrays.update(("param." + k, p.detach().float()) for k, p in model.named_parameters())
+    nbytes = sum(v.numel() * 4 for v in arrays.values())
+    assert nbytes <= 64 << 20, "outputs of %d bytes: sample them below 64 MB" % nbytes    # TEM workload: ~26 MB
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v.cpu().numpy())
 
 
 def bandwidth_regime(peaks, rows=16_000_000, d=128):
@@ -967,6 +983,9 @@ def run_b200_arm(a):
             transport = "nccl-all-to-all"
     else:
         model = ItemTransformerRanker(args, "cuda", V, P, None, word_dists=synth.word_dists(V), grad_mode=a.grad_mode)
+    # the step's negatives by inverse CDF on the device generator: the literal torch.multinomial calls are not
+    # reproducible on CUDA, and with them a run's results would not be a function of its arguments (--dump-outputs)
+    model.reproducible_draws = True
     optim = build_optim(args, model)
     model.train()
     torch.manual_seed(666 + 7919 * rank)      # per-rank negatives / dropout masks from here on
@@ -1027,7 +1046,7 @@ def run_b200_arm(a):
     for it in range(a.steps):
         flush.zero_()
         starts[it].record()
-        step(devb[a.warmup + it])
+        loss = step(devb[a.warmup + it])
         ends[it].record()
     host_enqueue_ms = (time.perf_counter() - t_host) / a.steps * 1e3     # host time to enqueue one step
     barrier()
@@ -1052,6 +1071,8 @@ def run_b200_arm(a):
     if graphed is not None:       # replays do not pass through the library's host counter
         launches = graphed.launches_per_replay * a.steps
     dev_sec = sum(s.elapsed_time(e) for s, e in zip(starts, ends)) * 1e-3
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, loss, model)
     # ---- timed region 2: end to end from pinned host batches (H2D + step + loss.item()).  The host batches are collated
     #      into the graph's input layout beforehand (GraphedTrainStep.pack: one pinned buffer per batch, like pinning --
     #      not timed), so a step's inputs cross PCIe in one copy
@@ -1082,7 +1103,7 @@ def run_b200_arm(a):
     #      all ranks take part because the sharded step contains cross-GPU barriers
     n_prof = min(a.steps, 10)
     for it in range(2):
-        eager_step(devb[a.warmup + it])
+        eager_step(devb[it])      # warm-up batches: there are at least 3 of them, and --steps may be 1
     barrier()
     _lib.profile_enable(True)
     for it in range(n_prof):
@@ -1303,7 +1324,14 @@ def main():
                     help="N=1: dense = the reference's dense table gradients + dense Adam sweep; rowsparse = compact row "
                          "gradients + row-sparse lazily caught-up Adam (dense-equivalent results, O(rows touched))")
     ap.add_argument("--eager", action="store_true", help="launch the step kernel by kernel instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", dest="dump_outputs",
+                    help="b200 arm: after the timed steps, write the loss of the last one and the parameters it left as "
+                         "DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 arm's timed step computed; --impl %s has none" % a.impl)
     a.warmup = max(a.warmup, 3)
     if a.impl == "reference":
         run_reference_arm(a)

@@ -30,6 +30,13 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
     # with it).  "randint": torch.randint(0, P) -- the same uniform distribution, O(1), a different random stream;
     # for catalogs where the literal call is the bottleneck.
     item_negative_sampler = "multinomial"
+    # Opt-in for runs that must repeat bit for bit.  The literal torch.multinomial calls (item and word negatives) are
+    # not reproducible on CUDA: every call rebuilds the distribution's CDF with a float32 scan whose rounding varies from
+    # run to run (torch lists CUDA cumsum as nondeterministic), and a draw next to a bucket boundary then takes the
+    # neighbouring id (profiles/multinomial_repro.py).  With reproducible_draws the same distributions are sampled by
+    # inverse CDF instead: each constant distribution's CDF is summed once in float64 on the host, and a draw is one
+    # torch.rand on the device generator plus a search -- a different random stream from the reference's.
+    reproducible_draws = False
 
     def __init__(self, args, device, vocab_size, product_size, vocab_words, word_dists=None,
                  grad_mode="dense"):
@@ -158,9 +165,23 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         if self.item_negative_sampler == "randint":
             neg_items = torch.randint(0, self.prod_pad_idx, (B, K), device=self.prod_dists.device)
         else:
-            neg_items = torch.multinomial(self.prod_dists, B * K, replacement=True).view(B, K)
-        neg_words = torch.multinomial(self.word_dists, B * W * K, replacement=True).view(B, W, K)
+            neg_items = self._multinomial("prod_dists", B * K).view(B, K)
+        neg_words = self._multinomial("word_dists", B * W * K).view(B, W, K)
         return neg_items, neg_words
+
+    def _multinomial(self, name, n):
+        """n draws with replacement from the constant distribution ``self.<name>`` (see reproducible_draws)."""
+        dist = getattr(self, name)
+        if not self.reproducible_draws:
+            return torch.multinomial(dist, n, replacement=True)
+        cache = self.__dict__.setdefault("_cdfs", {})
+        if name not in cache or cache[name][0] is not dist:
+            cdf = torch.cumsum(dist.detach().to("cpu", torch.float64), 0)
+            cache[name] = (dist, (cdf / cdf[-1]).to(dist.device))
+        cdf = cache[name][1]
+        # u in [0, 1) and cdf[-1] == 1: the id is the number of CDF entries <= u, so zero-probability ids (the pad
+        # word) are never drawn
+        return torch.searchsorted(cdf, torch.rand(n, dtype=torch.float64, device=cdf.device), right=True)
 
     def forward_dotproduct(self, batch_data, train_pv=False):
         query_word_idxs = batch_data.query_word_idxs
@@ -267,7 +288,7 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         and joins before reading the per-item losses that are then returned un-averaged."""
         B, W = target_word_idxs.shape
         if neg_sample_idxs is None:
-            neg_sample_idxs = torch.multinomial(self.word_dists, B * W * n_negs, replacement=True)
+            neg_sample_idxs = self._multinomial("word_dists", B * W * n_negs)
         if item_w is None:
             item_w, item_sink = self.product_emb.weight, self.item_sink
         anchor = F_.gather_rows(item_w, target_prod_idxs, item_sink, stream=stream)

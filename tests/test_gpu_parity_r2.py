@@ -227,6 +227,43 @@ def test_sampled_negatives_equal_reference_draws():
     assert torch.equal(after_model, torch.cuda.get_rng_state())
 
 
+def test_reproducible_draws_are_the_inverse_cdf_of_the_device_uniforms():
+    """reproducible_draws: every id is the inverse CDF (float64, summed on the host) of one torch.rand draw of the device
+    generator, items first, then words -- a pure function of the generator state, so one seed gives the same ids on
+    every run; the ids follow the reference's distributions (uniform items; word_dists, the pad word never); inside a
+    captured step they change from replay to replay."""
+    from prodsearch_b200 import synth
+    from prodsearch_b200.item_transformer import ItemTransformerRanker
+    cfg = _cfg(model_name="item_transformer")
+    P, V, W, K, n = 18000, 32000, 1, 5, 200_000
+    wd = np.asarray(synth.word_dists(V), dtype=np.float64)
+    model = ItemTransformerRanker(cfg, "cuda", V, P, None, word_dists=wd)
+    model.reproducible_draws = True
+    torch.manual_seed(1234)
+    neg_items, neg_words = model._draw_negatives(n // K, W, K)
+    torch.manual_seed(1234)
+    u_items = torch.rand(n, dtype=torch.float64, device="cuda").cpu()
+    u_words = torch.rand(n, dtype=torch.float64, device="cuda").cpu()
+    for got, u, p in ((neg_items, u_items, np.ones(P)), (neg_words, u_words, np.float32(wd).astype(np.float64))):
+        cdf = np.cumsum(p)
+        want = np.searchsorted(cdf / cdf[-1], u.numpy(), side="right")
+        assert np.array_equal(got.reshape(-1).cpu().numpy(), want)
+    items, words = neg_items.reshape(-1).cpu().numpy(), neg_words.reshape(-1).cpu().numpy()
+    assert items.min() >= 0 and items.max() < P and words.min() >= 0 and words.max() < V - 1
+    # frequencies against the distributions: every id's count within 6 sigma of its expectation
+    for ids, p in ((items, np.full(P, 1.0 / P)), (words, wd / wd.sum())):
+        cnt = np.bincount(ids, minlength=len(p)).astype(np.float64)
+        assert np.all(np.abs(cnt - n * p) <= 6 * np.sqrt(n * p * (1 - p)) + 1)
+    g = torch.cuda.CUDAGraph()
+    torch.manual_seed(5)
+    with torch.cuda.graph(g):
+        ni, nw = model._draw_negatives(64, W, K)
+    g.replay()
+    first = (ni.clone(), nw.clone())
+    g.replay()
+    assert not torch.equal(first[0], ni) and not torch.equal(first[1], nw)
+
+
 def test_pv_pvc_draws_equal_reference_draws(monkeypatch):
     from prodsearch_b200 import synth
     from prodsearch_b200.pv import ParagraphVector

@@ -261,24 +261,18 @@ int psb_catalog_topk_f16(const float* queries, int64_t m, const float* table, co
                          int64_t id_base, int64_t id_stride, void* workspace, int64_t workspace_bytes,
                          int64_t* out_ids, float* out_scores, psb_stream_t stream);
 
-/* Debug aid for the fp16 shortlist kernel's v2 epilogue (environment PSB_TC16_EPI=2 and PSB_TC16_STATS=1, both read
- * once per process): sums over CTAs and launches of clock64 counters -- host_out[0] MMA-issuer total, [1] issuer
- * waiting for a free accumulator set (epilogue-bound), [2] issuer waiting for item tiles (TMA-bound), [3] epilogue
- * warp total, [4] epilogue warp waiting for scores (MMA-bound), [5] TMA producer waiting for a free stage, [6] item
- * tiles, [7] CTA launches.  Synchronises the device; all zeros when the knobs are unset.  host_out: 8 words (host). */
-int psb_debug_tc16_stats(uint64_t* host_out, int32_t reset);
-
 /* Debug aid: TMEM read rate of tcgen05.ld.32x32b.x32 issued back to back by `warps` (1..16) warps of one CTA,
  * in bytes per SM clock -- bytes_per_clk[0] with one CTA on the GPU, [1] with one CTA per SM.  The catalog
  * contraction (K = 128) reads every accumulator element back after 8 MMAs, so this rate bounds its tensor-pipe
  * utilisation.  Synchronises the device, allocates and frees 20 KB.  bytes_per_clk: 2 doubles (host). */
 int psb_debug_tmem_read_bw(int32_t warps, int32_t iters, double* bytes_per_clk);
 
-/* Debug aid / building block under validation: out[m, j] = a[m, k] . bt[j, k]^T (+ bias[j]) on tcgen05 with the
- * 3xTF32 split (csrc/gemm3_tf32.cu) -- the tensor-core form of the encoder's linear layers (models/neural.py:118-120
- * linear_keys / linear_values / linear_query; models/transformer.py:37-88), which the FFMA kernels compute today.
+/* Debug aid: out[m, j] = a[m, k] . bt[j, k]^T (+ bias[j]) on tcgen05 with the 3xTF32 split (csrc/gemm3_tf32.cu) --
+ * the tensor-core form of the encoder's linear layers (models/neural.py:118-120 linear_keys / linear_values /
+ * linear_query; models/transformer.py:37-88), which the FFMA kernels compute on the FFMA path (PSB_ENC_TC=0).
  * k % 64 == 0, j % 64 == 0, lda % 4 == 0, ldo % 4 == 0, 16-byte aligned pointers; PSB_E_UNSUPPORTED otherwise.  The
- * encoder forward uses it for the q and K|V projections when PSB_ENC_TC=1 (off by default: no GPU run yet). */
+ * encoder uses it for the q and K|V projections and the backward's grad-xn product on the tensor-core path (the
+ * default). */
 int psb_debug_gemm3_tf32(const float* a, int64_t lda, int64_t m, int64_t k, const float* bt, int64_t j,
                          const float* bias, float* out, int64_t ldo, psb_stream_t stream);
 /* Debug aid: with PSB_FT_TRACE=1 in the environment the fused tensor-core encoder tail (tail_fused_tc_kernel,

@@ -110,7 +110,6 @@ SIGNATURES = {
     "psb_catalog_topk_workspace_bytes": (c_i64, [c_i64, c_i64, c_i64, c_i64, c_i32]),
     "psb_catalog_topk": (c_i32, [c_vp, c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, c_i32, c_vp, c_vp,
                                  c_i64, c_vp, c_vp, c_vp]),
-    "psb_debug_tc16_stats": (c_i32, [c_vp, c_i32]),
     "psb_debug_tmem_read_bw": (c_i32, [c_i32, c_i32, c_vp]),
     "psb_debug_gemm3_tf32": (c_i32, [c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp]),
     "psb_debug_tail_trace": (c_i32, [c_vp]),

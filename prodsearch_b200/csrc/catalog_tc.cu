@@ -19,9 +19,6 @@
 // swizzle), 2-stage ring of item tiles, TMEM: 2 accumulators x 128 columns (double buffered).
 #include <cuda.h>
 #include <cuda_fp16.h>
-#include <stdlib.h>
-
-#include <string.h>
 
 #include "catalog_common.cuh"
 #include "tc_ptx.cuh"
@@ -53,7 +50,6 @@ struct TcParams {
   int32_t* cand_i;
   int32_t* cand_n;                  // [m_pad * n_slices]
   int cap;
-  int debug;                        // experiment switches (PSB_TC_DEBUG): 1 = skip epilogue scan, 2 = skip MMA
 };
 
 template <bool DUMP>
@@ -244,14 +240,6 @@ tc_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
 constexpr int kKB16 = 64;                       // halves per k-block = one 128-byte swizzle row
 constexpr uint32_t kQBlock16 = kTM * 128;       // bytes of one 128-row k-block (16 KB)
 
-__device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 // Issue from a warp whose 32 lanes all execute the instruction stream (uniform control flow), with the instruction
 // itself predicated on the elected lane: the descriptors stay in uniform registers and ptxas has no reason to wrap
 // every tcgen05.mma in the per-lane "waterfall" loop it emits when the issue sits inside `if (lane == 0)`.
@@ -289,254 +277,20 @@ struct Tc16Params {
   int32_t* cand_i;
   int32_t* cand_n;
   int cap;
-  unsigned long long* stat;            // v2 + PSB_TC16_STATS only: 8 cycle counters per CTA (see tc16_score_v2_kernel)
 };
 
-// MT query tiles per CTA; item tile TN = 128 (MT <= 2) or 64 (MT = 3, 4): two accumulator sets of MT * TN
-// TMEM columns.  grid (item slices, query groups of MT tiles), 64 + 512 threads as tc_score_kernel.
-template <bool DUMP, int MT>
-__global__ void __launch_bounds__(kTcThreads, 1)
-tc16_score_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_e,
-                  const Tc16Params P) {
-  constexpr int TN = MT <= 2 ? 128 : 64;
-  constexpr int kAccCols = MT * TN;
-  constexpr int kTmemCols = 2 * kAccCols <= 256 ? 256 : 512;
-  constexpr uint32_t kIdesc16 = (1u << 4) | (static_cast<uint32_t>(TN >> 3) << 17) | (static_cast<uint32_t>(kTM >> 4) << 24);
-  constexpr int kMaxStages = 8;
-  extern __shared__ unsigned char smem_dyn[];
-  unsigned char* smem = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t q_bytes = static_cast<uint32_t>(MT * P.kblocks) * kQBlock16;
-  const uint32_t e_block = static_cast<uint32_t>(TN) * 128u;                 // bytes of one item k-block
-  const uint32_t stage_bytes = static_cast<uint32_t>(P.kblocks) * e_block;
-  const int S = P.stages;
-  unsigned char* sA = smem;
-  unsigned char* sB = smem + q_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sB + static_cast<size_t>(S) * stage_bytes);
-  uint64_t* a_full = bars;
-  uint64_t* b_full = bars + 1;
-  uint64_t* b_empty = bars + 1 + kMaxStages;
-  uint64_t* t_full = bars + 1 + 2 * kMaxStages;
-  uint64_t* t_empty = bars + 3 + 2 * kMaxStages;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 5 + 2 * kMaxStages);
-
-  const int n_slices = gridDim.x, slice = blockIdx.x, mtile0 = blockIdx.y * MT;
-  const int per = (P.n_tiles + n_slices - 1) / n_slices;
-  const int p_lo = slice * per;
-  const int p_hi = min(P.n_tiles, p_lo + per);
-  const int my_tiles = max(0, p_hi - p_lo);
-
-  if (threadIdx.x == 0) {
-    mbar_init(a_full, 1);
-    for (int st = 0; st < S; ++st) {
-      mbar_init(b_full + st, 1);
-      mbar_init(b_empty + st, 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(t_full + a, 1);
-      mbar_init(t_empty + a, 4 * kParts);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(kTmemCols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ===== TMA producer =====
-    if (lane == 0) {
-      mbar_expect_tx(a_full, q_bytes);
-      for (int mt = 0; mt < MT; ++mt)
-        for (int kb = 0; kb < P.kblocks; ++kb)
-          tma_load_2d(sA + (mt * P.kblocks + kb) * kQBlock16, &map_q, kb * kKB16, (mtile0 + mt) * kTM, a_full);
-      for (int it = 0; it < my_tiles; ++it) {
-        const int st = it % S;
-        const uint32_t ph = (it / S) & 1;
-        mbar_wait(b_empty + st, ph ^ 1);
-        mbar_expect_tx(b_full + st, stage_bytes);
-        const int tile = P.tile_begin + (p_lo + it) * P.tile_step;
-        for (int kb = 0; kb < P.kblocks; ++kb)
-          tma_load_2d(sB + static_cast<size_t>(st) * stage_bytes + kb * e_block, &map_e, kb * kKB16, tile * TN, b_full + st);
-      }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer =====
-    if (lane == 0) {
-      mbar_wait(a_full, 0);
-      // one thread issues every MMA of the CTA, so its instruction stream is on the critical path: descriptors
-      // are the base descriptor plus an address offset (>> 4, low 14 bits), never rebuilt per MMA
-      const uint64_t a_base = umma_desc(smem_u32(sA));
-      const uint64_t b_base = umma_desc(smem_u32(sB));
-      const uint32_t kb_a = kQBlock16 >> 4, kb_b = e_block >> 4, st_b = stage_bytes >> 4;
-      for (int it = 0; it < my_tiles; ++it) {
-        const int st = it % S;
-        const uint32_t ph = (it / S) & 1;
-        const int acc = it & 1;
-        const uint32_t aph = (it >> 1) & 1;
-        mbar_wait(t_empty + acc, aph ^ 1);
-        mbar_wait(b_full + st, ph);
-        tc_fence_after();
-        const uint64_t b_tile = b_base + static_cast<uint64_t>(st) * st_b;
-#pragma unroll
-        for (int mt = 0; mt < MT; ++mt) {
-          const uint32_t d_addr = tmem_base + static_cast<uint32_t>(acc * kAccCols + mt * TN);
-          const uint64_t a_tile = a_base + static_cast<uint64_t>(mt * P.kblocks) * kb_a;
-#pragma unroll 2
-          for (int kb = 0; kb < P.kblocks; ++kb) {
-#pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4)  // 4 x (K = 16 halves = 32 bytes) inside one 128-byte swizzle row
-              tc_mma_f16(d_addr, a_tile + static_cast<uint64_t>(kb) * kb_a + k4 * 2, b_tile + static_cast<uint64_t>(kb) * kb_b + k4 * 2,
-                         kIdesc16, (kb | k4) != 0 ? 1u : 0u);
-          }
-        }
-        tc_commit(b_empty + st);
-        tc_commit(t_full + acc);
-      }
-    }
-  } else {
-    // ===== epilogue: 16 warps; thread = (TMEM lane = query row inside a tile, part); 32-column chunks of the
-    // MT accumulators are dealt round-robin to the 4 parts
-    const int quarter = warp & 3;
-    const int part = (warp - 2) >> 2;
-    constexpr int kChunksPerTile = TN / 32;
-    float thr[MT];
-    int cnt[MT];
-    int64_t list[MT];
-    bool row_ok[MT];
-    const int n_lists = n_slices * kParts;
-#pragma unroll
-    for (int mt = 0; mt < MT; ++mt) {
-      const int row = (mtile0 + mt) * kTM + quarter * 32 + lane;
-      row_ok[mt] = row < P.m;
-      thr[mt] = INFINITY;
-      if (!DUMP && row_ok[mt]) thr[mt] = P.thr[row];
-      cnt[mt] = 0;
-      if (!DUMP && P.append && row_ok[mt]) cnt[mt] = P.cand_n[static_cast<int64_t>(row) * n_lists + slice * kParts + part];
-      list[mt] = (static_cast<int64_t>(row) * n_lists + slice * kParts + part) * P.cap;
-    }
-    const uint32_t lane_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
-    for (int it = 0; it < my_tiles; ++it) {
-      const int acc = it & 1;
-      const uint32_t aph = (it >> 1) & 1;
-      const int p = p_lo + it;
-      const int tile = P.tile_begin + p * P.tile_step;
-      const bool full_tile = (tile + 1) * TN <= P.n_items && P.bias == nullptr;
-      mbar_wait(t_full + acc, aph);
-      tc_fence_after();
-      // ONE loop body (no unrolling over chunks: 16 warps x unrolled bodies thrash the instruction cache);
-      // the per-query-tile state is selected into scalars and written back
-#pragma unroll 1
-      for (int w = part; w < MT * kChunksPerTile; w += kParts) {
-        const int mt = w / kChunksPerTile;
-        const int c0 = (w % kChunksPerTile) * 32;
-        float th = thr[0];
-        int cn = cnt[0];
-        int64_t li = list[0];
-        bool ok = row_ok[0];
-#pragma unroll
-        for (int j = 1; j < MT; ++j)
-          if (mt == j) {
-            th = thr[j];
-            cn = cnt[j];
-            li = list[j];
-            ok = row_ok[j];
-          }
-        uint32_t v[32];
-        __syncwarp();
-        tc_ld32(lane_addr + static_cast<uint32_t>(acc * kAccCols + mt * TN + c0), v);
-        const int id0 = tile * TN + c0;
-        if (DUMP) {
-          const int row = (mtile0 + mt) * kTM + quarter * 32 + lane;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            const int id = id0 + i;
-            float sc = __uint_as_float(v[i]);
-            if (P.bias != nullptr && id < P.n_items) sc += P.bias[id];
-            if (ok) P.dump[static_cast<int64_t>(row) * P.ld_dump + p * TN + c0 + i] = id < P.n_items ? sc : -INFINITY;
-          }
-        } else if (full_tile) {
-          // one branch per 32 scores (almost never taken once the threshold is refined), then one per 8
-          float mx8[4];
-#pragma unroll
-          for (int g = 0; g < 4; ++g) {
-            const int g8 = g * 8;
-            const float m0 = fmaxf(fmaxf(__uint_as_float(v[g8]), __uint_as_float(v[g8 + 1])),
-                                   fmaxf(__uint_as_float(v[g8 + 2]), __uint_as_float(v[g8 + 3])));
-            mx8[g] = fmaxf(m0, fmaxf(fmaxf(__uint_as_float(v[g8 + 4]), __uint_as_float(v[g8 + 5])),
-                                     fmaxf(__uint_as_float(v[g8 + 6]), __uint_as_float(v[g8 + 7]))));
-          }
-          if (!(fmaxf(fmaxf(mx8[0], mx8[1]), fmaxf(mx8[2], mx8[3])) < th)) {
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-              const int g8 = g * 8;
-              if (!(mx8[g] < th)) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                  const float sc = __uint_as_float(v[g8 + i]);
-                  if (!(sc < th)) {
-                    if (cn < P.cap) {
-                      P.cand_s[li + cn] = sc;
-                      P.cand_i[li + cn] = id0 + g8 + i;
-                    }
-                    ++cn;
-                  }
-                }
-              }
-            }
-          }
-        } else {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            const int id = id0 + i;
-            float sc = __uint_as_float(v[i]);
-            if (P.bias != nullptr && id < P.n_items) sc += P.bias[id];
-            if (!(sc < th) && id < P.n_items) {
-              if (cn < P.cap) {
-                P.cand_s[li + cn] = sc;
-                P.cand_i[li + cn] = id;
-              }
-              ++cn;
-            }
-          }
-        }
-#pragma unroll
-        for (int j = 0; j < MT; ++j)
-          if (mt == j) cnt[j] = cn;
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(t_empty + acc);
-    }
-    if (!DUMP) {
-#pragma unroll
-      for (int mt = 0; mt < MT; ++mt) {
-        const int row = (mtile0 + mt) * kTM + quarter * 32 + lane;
-        if (row_ok[mt]) P.cand_n[static_cast<int64_t>(row) * n_lists + slice * kParts + part] = cnt[mt];
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols));
-  }
-}
-
-// ------------------------------------------------------------------ fp16 shortlist, epilogue v2 (PSB_TC16_EPI=2)
-// Same TMA producer and MMA issuer as tc16_score_kernel; the hand-off and the epilogue differ:
+// ------------------------------------------------------------------ fp16 shortlist kernel
+// MT query tiles per CTA; item tile TN = 128 (MT <= 2) or 64 (MT = 3, 4): two accumulator sets of MT * TN TMEM
+// columns.  grid (item slices, query groups of MT tiles), 64 + 512 threads as tc_score_kernel.  Against the tf32
+// kernel's layout:
 //  (1) the accumulator set is handed over per QUERY TILE (one mbarrier per (set, tile), committed right after the
 //      tile's 8 MMAs): the epilogue of tile 0 runs while the MMAs of tiles 1.. are still in flight;
 //  (2) every epilogue warp owns a FIXED run of 32-column chunks of ONE query tile, so threshold, count and list
-//      base are scalars for the whole kernel (v1 deals chunks round-robin over the parts and re-selects the
-//      per-tile state for every chunk: ~35 of its ~80 instructions per chunk in the SASS);
-//  (3) a row therefore has AP candidate lists per item slice (the parts that own chunks of its tile), not kParts.
-// Written at the end of round 1 without GPU time left: compiled and SASS-checked only, OFF by default.
+//      base are scalars for the whole kernel (dealing chunks round-robin over the parts re-selects the per-tile
+//      state for every chunk: ~35 of ~80 instructions per chunk in the SASS of the round-1 kernel);
+//  (3) a row therefore has AP candidate lists per item slice (the parts that own chunks of its tile), not kParts;
+//  (4) the MMA issuer is the whole warp 1 with elected-lane predication (see tc_mma_f16_if): 11-19 % faster end to
+//      end than a lane-0 issuer (profiles/r01_summary.md).
 template <int MT>
 struct Tc16V2 {
   static constexpr int TN = MT <= 2 ? 128 : 64;
@@ -548,21 +302,11 @@ struct Tc16V2 {
   static_assert(kChunksPerTile % CPP == 0, "a part's run of chunks must stay inside one query tile");
 };
 
-// STATS: clock64 split of the three roles of one CTA, accumulated over launches into P.stat[cta * 8 + ...]:
-//   0 issuer total, 1 issuer waiting for a free accumulator set (epilogue-bound), 2 issuer waiting for item tiles
-//   (TMA / HBM / L2-bound), 3 epilogue warp 2 total, 4 epilogue warp 2 waiting for scores (MMA-bound),
-//   5 producer waiting for a free stage, 6 item tiles, 7 launches.  issuer total - 1 - 2 = MMA issue time.
-// VAR = PSB_TC16_EPI: 2 = the above; 3 = the MMA issuer is the whole warp 1 with elected-lane predication (see
-// tc_mma_f16_if); 4 = 3 + a part whose run is two chunks reads BOTH from TMEM under one wait (tc_ld32x2) and hands the
-// accumulator set back BEFORE it scans the 64 scores it now holds in registers, so the issuer's wait for a free set
-// (655 of 2554 cycles per tile in the v3 split at M = 4096) overlaps the scan instead of following it.
-template <bool DUMP, int MT, bool STATS, int VAR>
+template <bool DUMP, int MT>
 __global__ void __launch_bounds__(kTcThreads, 1)
 tc16_score_v2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_e,
                      const Tc16Params P) {
   using V = Tc16V2<MT>;
-  constexpr bool ELECT = VAR >= 3;
-  constexpr bool DUAL = VAR == 4 && !DUMP && V::CPP == 2;
   constexpr int TN = V::TN;
   constexpr int kAccCols = MT * TN;
   constexpr int kTmemCols = 2 * kAccCols <= 256 ? 256 : 512;
@@ -613,51 +357,39 @@ tc16_score_v2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
-    // ===== TMA producer (as v1) =====
+    // ===== TMA producer =====
     if (lane == 0) {
       mbar_expect_tx(a_full, q_bytes);
       for (int mt = 0; mt < MT; ++mt)
         for (int kb = 0; kb < P.kblocks; ++kb)
           tma_load_2d(sA + (mt * P.kblocks + kb) * kQBlock16, &map_q, kb * kKB16, (mtile0 + mt) * kTM, a_full);
-      long long w_prod = 0;
       for (int it = 0; it < my_tiles; ++it) {
         const int st = it % S;
         const uint32_t ph = (it / S) & 1;
-        long long w0 = 0;
-        if (STATS) w0 = clock64();
         mbar_wait(b_empty + st, ph ^ 1);
-        if (STATS) w_prod += clock64() - w0;
         mbar_expect_tx(b_full + st, stage_bytes);
         const int tile = P.tile_begin + (p_lo + it) * P.tile_step;
         for (int kb = 0; kb < P.kblocks; ++kb)
           tma_load_2d(sB + static_cast<size_t>(st) * stage_bytes + kb * e_block, &map_e, kb * kKB16, tile * TN, b_full + st);
       }
-      if (STATS && P.stat != nullptr) P.stat[(blockIdx.y * gridDim.x + blockIdx.x) * 8 + 5] += static_cast<unsigned long long>(w_prod);
     }
   } else if (warp == 1) {
-    // ===== MMA issuer: one commit per query tile =====
-    if (ELECT || lane == 0) {
-      const uint32_t leader = ELECT ? elect_one() : 1u;
+    // ===== MMA issuer: all 32 lanes run the loop, the instructions are predicated on the elected lane; one commit
+    //       per query tile =====
+    {
+      const uint32_t leader = elect_one();
       mbar_wait(a_full, 0);
+      // descriptors are the base descriptor plus an address offset (>> 4, low 14 bits), never rebuilt per MMA
       const uint64_t a_base = umma_desc(smem_u32(sA));
       const uint64_t b_base = umma_desc(smem_u32(sB));
       const uint32_t kb_a = kQBlock16 >> 4, kb_b = e_block >> 4, st_b = stage_bytes >> 4;
-      long long w_acc = 0, w_tile = 0, t_begin = 0;
-      if (STATS) t_begin = clock64();
       for (int it = 0; it < my_tiles; ++it) {
         const int st = it % S;
         const uint32_t ph = (it / S) & 1;
         const int acc = it & 1;
         const uint32_t aph = (it >> 1) & 1;
-        long long w0 = 0, w1 = 0;
-        if (STATS) w0 = clock64();
         mbar_wait(t_empty + acc, aph ^ 1);
-        if (STATS) w1 = clock64();
         mbar_wait(b_full + st, ph);
-        if (STATS) {
-          w_acc += w1 - w0;
-          w_tile += clock64() - w1;
-        }
         tc_fence_after();
         const uint64_t b_tile = b_base + static_cast<uint64_t>(st) * st_b;
 #pragma unroll
@@ -667,25 +399,13 @@ tc16_score_v2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
 #pragma unroll 2
           for (int kb = 0; kb < P.kblocks; ++kb) {
 #pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4)
-              if (ELECT)
-                tc_mma_f16_if(leader, d_addr, a_tile + static_cast<uint64_t>(kb) * kb_a + k4 * 2,
-                              b_tile + static_cast<uint64_t>(kb) * kb_b + k4 * 2, kIdesc16, (kb | k4) != 0 ? 1u : 0u);
-              else
-                tc_mma_f16(d_addr, a_tile + static_cast<uint64_t>(kb) * kb_a + k4 * 2, b_tile + static_cast<uint64_t>(kb) * kb_b + k4 * 2,
-                           kIdesc16, (kb | k4) != 0 ? 1u : 0u);
+            for (int k4 = 0; k4 < 4; ++k4)  // 4 x (K = 16 halves = 32 bytes) inside one 128-byte swizzle row
+              tc_mma_f16_if(leader, d_addr, a_tile + static_cast<uint64_t>(kb) * kb_a + k4 * 2,
+                            b_tile + static_cast<uint64_t>(kb) * kb_b + k4 * 2, kIdesc16, (kb | k4) != 0 ? 1u : 0u);
           }
-          if (ELECT) tc_commit_if(leader, t_full + acc * MT + mt); else tc_commit(t_full + acc * MT + mt);
+          tc_commit_if(leader, t_full + acc * MT + mt);
         }
-        if (ELECT) tc_commit_if(leader, b_empty + st); else tc_commit(b_empty + st);
-      }
-      if (STATS && P.stat != nullptr && lane == 0) {
-        unsigned long long* o = P.stat + (blockIdx.y * gridDim.x + blockIdx.x) * 8;
-        o[0] += static_cast<unsigned long long>(clock64() - t_begin);
-        o[1] += static_cast<unsigned long long>(w_acc);
-        o[2] += static_cast<unsigned long long>(w_tile);
-        o[6] += static_cast<unsigned long long>(my_tiles);
-        o[7] += 1ull;
+        tc_commit_if(leader, b_empty + st);
       }
     }
   } else if (((warp - 2) >> 2) < V::kActiveParts) {
@@ -707,75 +427,14 @@ tc16_score_v2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
       if (P.append) cn = P.cand_n[lidx];
     }
     const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(mt * TN + col0);
-    long long w_sc = 0, e_begin = 0;
-    if (STATS) e_begin = clock64();
     for (int it = 0; it < my_tiles; ++it) {
       const int acc = it & 1;
       const uint32_t aph = (it >> 1) & 1;
       const int p = p_lo + it;
       const int tile = P.tile_begin + p * P.tile_step;
       const bool full_tile = (tile + 1) * TN <= P.n_items && P.bias == nullptr;
-      long long w0 = 0;
-      if (STATS) w0 = clock64();
       mbar_wait(t_full + acc * MT + mt, aph);
-      if (STATS) w_sc += clock64() - w0;
       tc_fence_after();
-      if constexpr (DUAL) {
-        uint32_t v2[2][32];
-        __syncwarp();
-        tc_ld32x2(t_addr + static_cast<uint32_t>(acc * kAccCols), v2[0], v2[1]);
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(t_empty + acc);       // the scores are in registers: the set is free again
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int id0 = tile * TN + col0 + j * 32;
-          if (full_tile) {
-            float mx8[4];
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-              const int g8 = g * 8;
-              const float m0 = fmaxf(fmaxf(__uint_as_float(v2[j][g8]), __uint_as_float(v2[j][g8 + 1])),
-                                     fmaxf(__uint_as_float(v2[j][g8 + 2]), __uint_as_float(v2[j][g8 + 3])));
-              mx8[g] = fmaxf(m0, fmaxf(fmaxf(__uint_as_float(v2[j][g8 + 4]), __uint_as_float(v2[j][g8 + 5])),
-                                       fmaxf(__uint_as_float(v2[j][g8 + 6]), __uint_as_float(v2[j][g8 + 7]))));
-            }
-            if (!(fmaxf(fmaxf(mx8[0], mx8[1]), fmaxf(mx8[2], mx8[3])) < th)) {
-#pragma unroll
-              for (int g = 0; g < 4; ++g) {
-                const int g8 = g * 8;
-                if (!(mx8[g] < th)) {
-#pragma unroll
-                  for (int i = 0; i < 8; ++i) {
-                    const float sc = __uint_as_float(v2[j][g8 + i]);
-                    if (!(sc < th)) {
-                      if (cn < P.cap) {
-                        P.cand_s[li + cn] = sc;
-                        P.cand_i[li + cn] = id0 + g8 + i;
-                      }
-                      ++cn;
-                    }
-                  }
-                }
-              }
-            }
-          } else {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
-              const int id = id0 + i;
-              float sc = __uint_as_float(v2[j][i]);
-              if (P.bias != nullptr && id < P.n_items) sc += P.bias[id];
-              if (!(sc < th) && id < P.n_items) {
-                if (cn < P.cap) {
-                  P.cand_s[li + cn] = sc;
-                  P.cand_i[li + cn] = id;
-                }
-                ++cn;
-              }
-            }
-          }
-        }
-      } else {
 #pragma unroll 1
       for (int j = 0; j < V::CPP; ++j) {
         const int c0 = col0 + j * 32;
@@ -839,14 +498,8 @@ tc16_score_v2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(t_empty + acc);
-      }
     }
     if (!DUMP && ok) P.cand_n[lidx] = cn;
-    if (STATS && P.stat != nullptr && warp == 2 && lane == 0) {
-      unsigned long long* o = P.stat + (blockIdx.y * gridDim.x + blockIdx.x) * 8;
-      o[3] += static_cast<unsigned long long>(clock64() - e_begin);
-      o[4] += static_cast<unsigned long long>(w_sc);
-    }
   }
   tc_fence_before();
   __syncthreads();
@@ -1407,7 +1060,6 @@ int catalog_topk_tc(const float* queries, int64_t m, const float* table, int64_t
   P.cand_i = cand_i;
   P.cand_n = cand_n;
   P.cap = pl.cap;
-  { const char* e = getenv("PSB_TC_DEBUG"); P.debug = e ? atoi(e) : 0; }
   // 1. pilot
   P.tile_begin = 0;
   P.tile_step = pl.pilot_step;
@@ -1464,60 +1116,15 @@ static int make_map16(CUtensorMap* map, const void* base, int64_t rows, int64_t 
   return r == CUDA_SUCCESS ? PSB_OK : PSB_E_ARG;
 }
 
-// Epilogue variant of the fp16 shortlist kernel: 3 (default since round 2: the whole GPU suite incl. the 16M-row
-// full-size test passes with it, lists bit-identical to variant 1, 11-19 % faster end to end) = tc16_score_v2_kernel
-// with per-tile accumulator hand-off and MMAs issued from a converged warp; 1 = tc16_score_kernel (round-1 default);
-// 2 / 4 = the other tc16_score_v2_kernel<.., VAR> instantiations (PSB_TC16_EPI=1|2|4).  Read once per process.
-static int tc16_epilogue_variant() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSB_TC16_EPI");
-    const int x = e != nullptr ? atoi(e) : 3;
-    v = (x >= 1 && x <= 4) ? x : 3;
-  }
-  return v;
-}
-
-// PSB_TC16_STATS=1 (with PSB_TC16_EPI=2): a library-owned counter block the v2 kernel adds its cycle split to
-// (debug aid, the one allocation this library makes besides the peer buffers); read by psb_debug_tc16_stats.
-constexpr int kTc16StatCtas = 256;
-static unsigned long long* g_tc16_stat = nullptr;
-static unsigned long long* tc16_stat_buffer() {
-  static int wanted = -1;
-  if (wanted < 0) {
-    const char* e = getenv("PSB_TC16_STATS");
-    wanted = (e != nullptr && atoi(e) != 0 && tc16_epilogue_variant() != 1) ? 1 : 0;
-  }
-  if (wanted == 1 && g_tc16_stat == nullptr) {
-    if (cudaMalloc(reinterpret_cast<void**>(&g_tc16_stat), kTc16StatCtas * 8 * sizeof(unsigned long long)) != cudaSuccess ||
-        cudaMemset(g_tc16_stat, 0, kTc16StatCtas * 8 * sizeof(unsigned long long)) != cudaSuccess) {
-      g_tc16_stat = nullptr;
-      wanted = 0;
-    }
-  }
-  return g_tc16_stat;
-}
-
-// Query tiles resident per CTA: 4 (default) = 512 queries per pass over the table at 64 items per MMA; PSB_TC16_MT=2
-// = 256 queries per pass at 128 items per MMA -- half the tcgen05.mma instructions for the same flops (the issuing
-// thread, not the tensor pipe, paces the MT = 4 kernel: DESIGN.md section 8) against twice the table passes.
-// Tuning knob, read once per process.
-static int tc16_max_tiles_per_cta(int m_tiles) {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSB_TC16_MT");
-    const int x = e != nullptr ? atoi(e) : 0;
-    v = (x >= 1 && x <= 4) ? x : 0;
-  }
-  if (v > 0) return v;
-  // unset: measured on B200 (profiles/r02a_tc16_variants.jsonl, 1M items): 4 tiles per CTA win up to a few hundred
-  // queries (M = 384: 0.305 vs 0.314 ms), 2 tiles x 128 items per MMA from a few thousand on (M = 4096: 2.01 vs 2.06 ms)
-  return m_tiles >= 16 ? 2 : 4;
-}
+// Query tiles resident per CTA: 4 = 512 queries per pass over the table at 64 items per MMA; 2 = 256 queries per pass
+// at 128 items per MMA -- half the tcgen05.mma instructions for the same flops (the issuing thread, not the tensor pipe,
+// paces the MT = 4 kernel: DESIGN.md section 8) against twice the table passes.  Measured on B200
+// (profiles/r02a_tc16_variants.jsonl, 1M items): 4 tiles per CTA win up to a few hundred queries (M = 384: 0.305 vs
+// 0.314 ms), 2 tiles x 128 items per MMA from a few thousand on (M = 4096: 2.01 vs 2.06 ms).
+static int tc16_max_tiles_per_cta(int m_tiles) { return m_tiles >= 16 ? 2 : 4; }
 
 // candidate lists per (query row, item slice): one per epilogue part that scores columns of the row's query tile
 static int tc16_lists_per_slice(int MT) {
-  if (tc16_epilogue_variant() == 1) return kParts;
   switch (MT) {
     case 1: return Tc16V2<1>::AP;
     case 2: return Tc16V2<2>::AP;
@@ -1560,30 +1167,11 @@ static Tc16Plan plan16_for(int64_t m, int64_t n_items, int64_t d, int64_t k) {
   // Measured at 1M / 2M items (profiles/tc16_segs.py): dropping the middle segment (2150 instead of 1550 candidates
   // per row) costs +33 us at 384 queries and +0.32 ms at 4096, but saves 17 us at 24.  Hence: few queries -> one
   // refinement; a few hundred -> first segment 10x the pilot, then 5x steps; thousands -> 3x steps from the start.
-  // PSB_TC16_SCHED="r0:r" overrides (r = 0: no further refinement); read once.
-  // (profiles/r02D_tc16_sched.jsonl: 1M items, 4096 queries 2.02 -> 1.90 ms with 3x steps; 24 queries 0.163 -> 0.143 ms
+  // (r = 0: no further refinement; profiles/r02D_tc16_sched.jsonl: 1M items, 4096 queries 2.02 -> 1.90 ms with 3x steps; 24 queries 0.163 -> 0.143 ms
   // with one refinement -- but only on small tables: at 16M one refinement leaves 18k candidates per row, the lists
   // overflow and the exact fallback answers, 341 ms)
   const bool small_table = n_items <= 2500000;
-  int r0 = m <= 1024 ? 10 : 3, r = m <= 64 ? (small_table ? 0 : 5) : (m <= 1024 ? 5 : 3);
-  {
-    static int e_r0 = -1, e_r = -1;
-    if (e_r0 < 0) {
-      const char* e = getenv("PSB_TC16_SCHED");
-      e_r0 = 0;
-      e_r = 0;
-      if (e != nullptr) {
-        e_r0 = atoi(e);
-        const char* c = strchr(e, ':');
-        e_r = c != nullptr ? atoi(c + 1) : 0;
-        if (e_r0 < 2 || e_r0 > 64) e_r0 = 0;
-      }
-    }
-    if (e_r0 > 0) {
-      r0 = e_r0;
-      r = e_r;
-    }
-  }
+  const int r0 = m <= 1024 ? 10 : 3, r = m <= 64 ? (small_table ? 0 : 5) : (m <= 1024 ? 5 : 3);
   p.nseg = 0;
   {
     int64_t end = static_cast<int64_t>(r0) * 8192 / p.TN;
@@ -1656,61 +1244,19 @@ static int launch_tc16(int MT, dim3 grid, size_t smem, cudaStream_t s, const CUt
   static DeviceAttr attr_done;
   if (attr_done.need()) {
     const int lim = 227 * 1024;
-    cudaError_t e = cudaSuccess;
-#define PSB_TC16_ATTR(D, M) \
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_kernel<D, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim)
-    PSB_TC16_ATTR(true, 1); PSB_TC16_ATTR(true, 2); PSB_TC16_ATTR(true, 3); PSB_TC16_ATTR(true, 4);
-    PSB_TC16_ATTR(false, 1); PSB_TC16_ATTR(false, 2); PSB_TC16_ATTR(false, 3); PSB_TC16_ATTR(false, 4);
-#undef PSB_TC16_ATTR
+    cudaError_t e = cudaFuncSetAttribute(tc16_score_v2_kernel<DUMP, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_v2_kernel<DUMP, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_v2_kernel<DUMP, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_v2_kernel<DUMP, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
     if (e != cudaSuccess) return static_cast<int>(e);
     attr_done.done();
   }
-  if (tc16_epilogue_variant() != 1) {
-    // the pilot (DUMP) pass has no scan to overlap: variant 4 runs it as variant 3
-    const int var = (DUMP && tc16_epilogue_variant() == 4) ? 3 : tc16_epilogue_variant();
-    const bool stats = P.stat != nullptr && !DUMP && static_cast<int>(grid.x * grid.y) <= kTc16StatCtas;
-    static DeviceAttr attr2_done;
-    if (attr2_done.need()) {
-      const int lim = 227 * 1024;
-      cudaError_t e = cudaSuccess;
-#define PSB_TC16_ATTR2(D, M) \
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_v2_kernel<D, M, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim); \
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_v2_kernel<D, M, true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim); \
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_v2_kernel<D, M, false, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim); \
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(tc16_score_v2_kernel<D, M, true, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim); \
-  if (e == cudaSuccess && !D) e = cudaFuncSetAttribute(tc16_score_v2_kernel<false, M, false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim); \
-  if (e == cudaSuccess && !D) e = cudaFuncSetAttribute(tc16_score_v2_kernel<false, M, true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim)
-      PSB_TC16_ATTR2(true, 1); PSB_TC16_ATTR2(true, 2); PSB_TC16_ATTR2(true, 3); PSB_TC16_ATTR2(true, 4);
-      PSB_TC16_ATTR2(false, 1); PSB_TC16_ATTR2(false, 2); PSB_TC16_ATTR2(false, 3); PSB_TC16_ATTR2(false, 4);
-#undef PSB_TC16_ATTR2
-      if (e != cudaSuccess) return static_cast<int>(e);
-      attr2_done.done();
-    }
-    PSB_PROF(var == 4 ? "tc16_score_v4_kernel" : var == 3 ? "tc16_score_v3_kernel" : "tc16_score_v2_kernel", s);
-#define PSB_TC16_GO(M)                                                                                      \
-  do {                                                                                                      \
-    if (var == 4 && stats) tc16_score_v2_kernel<false, M, true, 4><<<grid, kTcThreads, smem, s>>>(mq, me, P);      \
-    else if (var == 4) tc16_score_v2_kernel<false, M, false, 4><<<grid, kTcThreads, smem, s>>>(mq, me, P);         \
-    else if (var == 3 && stats) tc16_score_v2_kernel<DUMP, M, true, 3><<<grid, kTcThreads, smem, s>>>(mq, me, P);  \
-    else if (var == 3) tc16_score_v2_kernel<DUMP, M, false, 3><<<grid, kTcThreads, smem, s>>>(mq, me, P);          \
-    else if (stats) tc16_score_v2_kernel<DUMP, M, true, 2><<<grid, kTcThreads, smem, s>>>(mq, me, P);              \
-    else tc16_score_v2_kernel<DUMP, M, false, 2><<<grid, kTcThreads, smem, s>>>(mq, me, P);                        \
-  } while (0)
-    switch (MT) {
-      case 1: PSB_TC16_GO(1); break;
-      case 2: PSB_TC16_GO(2); break;
-      case 3: PSB_TC16_GO(3); break;
-      default: PSB_TC16_GO(4); break;
-    }
-#undef PSB_TC16_GO
-    return launch_status();
-  }
-  PSB_PROF("tc16_score_kernel", s);
+  PSB_PROF("tc16_score_v3_kernel", s);   // the profiler label the benchmark output has always used for this kernel
   switch (MT) {
-    case 1: tc16_score_kernel<DUMP, 1><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
-    case 2: tc16_score_kernel<DUMP, 2><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
-    case 3: tc16_score_kernel<DUMP, 3><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
-    default: tc16_score_kernel<DUMP, 4><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
+    case 1: tc16_score_v2_kernel<DUMP, 1><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
+    case 2: tc16_score_v2_kernel<DUMP, 2><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
+    case 3: tc16_score_v2_kernel<DUMP, 3><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
+    default: tc16_score_v2_kernel<DUMP, 4><<<grid, kTcThreads, smem, s>>>(mq, me, P); break;
   }
   return launch_status();
 }
@@ -1767,7 +1313,6 @@ int catalog_topk_tc16(const float* queries, int64_t m, const float* table, const
   P.cand_n = cand_n;
   P.cap = pl.cap;
   P.append = 0;
-  P.stat = tc16_stat_buffer();
   // 1. pilot
   P.tile_begin = 0;
   P.tile_step = pl.pilot_step;
@@ -1821,20 +1366,6 @@ int catalog_topk_tc16(const float* queries, int64_t m, const float* table, const
 }
 
 }  // namespace psb
-
-extern "C" int psb_debug_tc16_stats(uint64_t* host_out, int32_t reset) {
-  if (host_out == nullptr) return PSB_E_ARG;
-  for (int i = 0; i < 8; ++i) host_out[i] = 0;
-  if (psb::g_tc16_stat == nullptr) return PSB_OK;                  // knobs not set: all zeros
-  static unsigned long long h[psb::kTc16StatCtas * 8];
-  cudaError_t e = cudaDeviceSynchronize();
-  if (e == cudaSuccess) e = cudaMemcpy(h, psb::g_tc16_stat, sizeof(h), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && reset != 0) e = cudaMemset(psb::g_tc16_stat, 0, sizeof(h));
-  if (e != cudaSuccess) return static_cast<int>(e);
-  for (int c = 0; c < psb::kTc16StatCtas; ++c)
-    for (int i = 0; i < 8; ++i) host_out[i] += h[c * 8 + i];
-  return PSB_OK;
-}
 
 // ------------------------------------------------------------------ TMEM read bandwidth probe (debug aid)
 // The catalog contraction has K = d = 128: every fp32 accumulator element is read back (tcgen05.ld) after only 8

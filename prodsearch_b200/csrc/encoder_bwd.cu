@@ -7,11 +7,9 @@
 //   embed_bwd  (+ pre-LN') + residual, masked -> grad of the token inputs
 //   wgrad      every dW = G^T A as split-M 128x128 FFMA tiles with per-chunk partials
 //   reduce     partials summed in chunk order (deterministic; no float atomics anywhere)
-// With PSB_ENC_TC = 4 (the default) tail_bwd becomes tail_bwd_fused_tc_kernel (gemm3_tf32.cu: the product chain on
+// On the tensor-core path (the default) tail_bwd becomes tail_bwd_fused_tc_kernel (gemm3_tf32.cu: the product chain on
 // tcgen05) + tail_attn_bwd_kernel (below), the grad-xn product runs on gemm3_tf32_kernel, and wgrad / reduce are
 // launched in two halves on streams of their own (see psb_encoder_bwd).
-#include <stdlib.h>
-
 #include "encoder_common.cuh"
 
 namespace psb {
@@ -302,7 +300,7 @@ static int launch_tail_bwd(const TailBwdArgs& a, cudaStream_t s) {
   return launch_status();
 }
 
-// ------------------------------------------------------------------ attention backward on its own (PSB_ENC_TC=4)
+// ------------------------------------------------------------------ attention backward on its own (tensor-core path)
 // Steps (7a-c) of tail_bwd_kernel + the residual sum for a tile of spt sequences (R = spt * C copy rows) when the product
 // chain ran on tcgen05 (gemm3_tf32.cu tail_bwd_fused_tc_kernel): gy and g_ctx come from global memory.  Everything the
 // tile reads more than once -- its K | V rows included -- is staged in shared memory with one wave of coalesced loads,
@@ -600,18 +598,9 @@ __global__ void __launch_bounds__(128) embed_bwd_kernel(const EmbedBwdArgs a) {
 }
 
 // ------------------------------------------------------------------ weight gradients dW = G^T A
-// rows of M per CTA (PSB_WG_CHUNK overrides, multiple of kSub; 96 / 128 / 160 / 192 measured within 1 % of each other on
-// the batch-384 step: profiles/r02_summary.md)
-static int wg_chunk() {
-  static int v = 0;
-  if (v == 0) {
-    const char* e = getenv("PSB_WG_CHUNK");
-    const int x = e != nullptr ? atoi(e) : 128;
-    v = (x >= 32 && x <= 4096 && x % 32 == 0) ? x : 128;
-  }
-  return v;
-}
-#define kChunk wg_chunk()
+// rows of M per CTA (a multiple of kSub; 96 / 128 / 160 / 192 measured within 1 % of each other on the batch-384 step:
+// profiles/r02_summary.md)
+constexpr int kChunk = 128;
 constexpr int kSub = 32;      // rows staged in shared memory at a time
 struct WgProb {
   const float* G;  // [M][ldg], columns n0.. of the gradient operand
@@ -627,7 +616,6 @@ struct WgProb {
 struct WgProbs {
   WgProb p[6];
   int n;
-  int chunk;   // rows of M per CTA (wg_chunk())
 };
 
 __global__ void __launch_bounds__(256) wgrad_kernel(const WgProbs probs) {
@@ -639,9 +627,9 @@ __global__ void __launch_bounds__(256) wgrad_kernel(const WgProbs probs) {
   const WgProb& P = probs.p[q];
   const int ch = b / (P.ntn * P.ntk), t2 = b - ch * (P.ntn * P.ntk), tn = t2 / P.ntk, tk = t2 - tn * P.ntk;
   const int M = P.m_dev != nullptr ? *P.m_dev : P.m_host;
-  const int m0 = ch * probs.chunk;
+  const int m0 = ch * kChunk;
   if (m0 >= M) return;
-  const int m1 = min(M, m0 + probs.chunk);
+  const int m1 = min(M, m0 + kChunk);
   const int n0 = tn * 128, k0 = tk * 128;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   float acc[8][8];
@@ -762,17 +750,6 @@ static BwdWs bwd_ws_layout(const Dims& D) {
 using namespace psb;
 using namespace psb::enc;
 
-// PSB_DEBUG_SKIP (timing experiments only, results are WRONG): bit 0 / 1 / 2 = do not launch the first / second
-// weight-gradient kernel / the partial-sum reduce -- is the side-stream chain on the step's critical path?
-static int debug_skip() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSB_DEBUG_SKIP");
-    v = e != nullptr ? atoi(e) : 0;
-  }
-  return v;
-}
-
 extern "C" int64_t psb_encoder_workspace_bytes(const psb_encoder_cfg_t* cfg, int32_t backward) {
   Dims D;
   const int st = dims_from_cfg(cfg, &D);
@@ -807,25 +784,13 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
   const TokSrc ts{cfg->first, cfg->table, cfg->table_rows, cfg->idx, cfg->pad_idx, cfg->dense, cfg->mask, cfg->pe, cfg->raw_input != 0 && cfg->first == nullptr};
   const int d = D.d, F = D.F, SC = D.S * D.C;
 
-  // [Wk ; Wv] stacked so grad xn is ONE product over the 2d-wide [gK | gV] rows.  Big token counts (RTM: 117k rows)
-  // run that product on tcgen05 (gemm3_tf32.cu), which wants the K-major operand [Wk^T | Wv^T] : [d][2d] instead
-  // With the tensor-core encoder (PSB_ENC_TC >= 1, the default) the forward pass left that operand in the saved state.
-  const bool tc_saved = rows_gemm_tc_enabled() &&
-                        rows_gemm_tc_supported(ws + W.gkv, 2 * d, 2 * d, sv + L.wkv_t, nullptr, 0, d, nullptr, ws + W.gxn, d);
-  const bool tc_gxn = tc_saved || (rows_gemm_tc_auto(static_cast<int64_t>(D.S) * D.T) &&
-                      rows_gemm_tc_supported(ws + W.gkv, 2 * d, 2 * d, ws + W.wkv, nullptr, 0, d, nullptr, ws + W.gxn, d));
-  const float* wkv_op = tc_saved ? sv + L.wkv_t : ws + W.wkv;
+  // [Wk ; Wv] stacked so grad xn is ONE product over the 2d-wide [gK | gV] rows.  On the tensor-core path that product
+  // runs on tcgen05 (gemm3_tf32.cu), which wants the K-major operand [Wk^T | Wv^T] : [d][2d] instead: the forward pass
+  // left it in the saved state.
+  const bool tc_gxn = enc_tc_enabled() &&
+                      rows_gemm_tc_supported(ws + W.gkv, 2 * d, 2 * d, sv + L.wkv_t, nullptr, 0, d, nullptr, ws + W.gxn, d);
   cudaError_t ce = cudaSuccess;
-  if (tc_saved) {
-    // nothing to prepare
-  } else if (tc_gxn) {
-    TrJobs jobs;
-    jobs.n = 0;
-    jobs.j[jobs.n++] = TrJob{p->wk, ws + W.wkv, d, d, 2 * d, 0, 0};
-    jobs.j[jobs.n++] = TrJob{p->wv, ws + W.wkv, d, d, 2 * d, d, 0};
-    int st0 = launch_transposes(jobs, s);
-    if (st0 != PSB_OK) return st0;
-  } else {
+  if (!tc_gxn) {
     ce = cudaMemcpyAsync(ws + W.wkv, p->wk, sizeof(float) * d * d, cudaMemcpyDeviceToDevice, s);
     if (ce == cudaSuccess)
       ce = cudaMemcpyAsync(ws + W.wkv + static_cast<size_t>(d) * d, p->wv, sizeof(float) * d * d, cudaMemcpyDeviceToDevice, s);
@@ -850,7 +815,6 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
   // weight gradients
   WgProbs probs;
   probs.n = 0;
-  probs.chunk = kChunk;
   int total_tiles = 0;
   auto add = [&](int i, const float* G, int ldg, const float* A, int lda, const int32_t* m_dev, int m_host, int m_max,
                  int N, int K) {
@@ -891,7 +855,7 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
   if (tail_bwd_fused_for(D)) {
     // (the forward pass took the same decision and saved what this path reads: no falling back from here)
     if (!tail_bwd_fused_supported(tb)) return PSB_E_ALIGN;
-    // PSB_ENC_TC=4: the product chain on tcgen05 (gemm3_tf32.cu), then the attention backward from gy / g_ctx
+    // tensor-core path: the product chain on tcgen05 (gemm3_tf32.cu), then the attention backward from gy / g_ctx
     if ((st = launch_tail_bwd_fused(tb, s)) != PSB_OK) return st;
     a.gy_in = tb.gy;
     a.gctx_in = tb.g_ctx;
@@ -907,14 +871,13 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
       if (e0 != cudaSuccess) return static_cast<int>(e0);
       WgProbs first;
       first.n = 3;
-      first.chunk = probs.chunk;
       int tiles = 0;
       for (int i = 0; i < 3; ++i) {
         first.p[i] = probs.p[i];
         tiles += probs.p[i].tiles;
       }
       PSB_PROF("wgrad_kernel", sw0);
-      if (!(debug_skip() & 1)) wgrad_kernel<<<tiles, 256, 0, sw0>>>(first);
+      wgrad_kernel<<<tiles, 256, 0, sw0>>>(first);
       if ((st = launch_status()) != PSB_OK) return st;
       // ... and their partial sums are reduced right behind them, on the same stream; the rest of the weight gradients
       // (dWk / dWv / dWq, which wait for the attention backward) get a stream of their own
@@ -928,7 +891,7 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
       }
       if (blocks_a > 0) {
         PSB_PROF("reduce_kernel", sw0);
-        if (!(debug_skip() & 4)) reduce_kernel<<<blocks_a, 256, 0, sw0>>>(ja);
+        reduce_kernel<<<blocks_a, 256, 0, sw0>>>(ja);
         if ((st = launch_status()) != PSB_OK) return st;
       }
       if ((e0 = cudaEventRecord(first_done, sw0)) != cudaSuccess) return static_cast<int>(e0);
@@ -959,8 +922,8 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
         },
         [&]() {
           if (tc_gxn)
-            return launch_rows_gemm_tc(ws + W.gkv, 2 * d, off + D.S, 0, D.S * D.T, 2 * d, wkv_op, nullptr, 0, d, nullptr,
-                                       ws + W.gxn, d, s);
+            return launch_rows_gemm_tc(ws + W.gkv, 2 * d, off + D.S, 0, D.S * D.T, 2 * d, sv + L.wkv_t, nullptr, 0, d,
+                                       nullptr, ws + W.gxn, d, s);
           return launch_rows_gemm(ws + W.gkv, 2 * d, off + D.S, 0, D.S * D.T, 2 * d, ws + W.wkv, d, nullptr,
                                   ws + W.gxn, d, s);
         });
@@ -984,14 +947,13 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
   {
     WgProbs rest;
     rest.n = 0;
-    rest.chunk = probs.chunk;
     int tiles = 0;
     for (int i = wgrad_from; i < 6; ++i) {
       rest.p[rest.n++] = probs.p[i];
       tiles += probs.p[i].tiles;
     }
     PSB_PROF("wgrad_kernel", sw);
-    if (!(debug_skip() & 2)) wgrad_kernel<<<tiles, 256, 0, sw>>>(rest);
+    wgrad_kernel<<<tiles, 256, 0, sw>>>(rest);
     if ((st = launch_status()) != PSB_OK) return st;
   }
 
@@ -1014,7 +976,7 @@ extern "C" int psb_encoder_bwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
   }
   if (total_blocks > 0) {
     PSB_PROF("reduce_kernel", sw);
-    if (!(debug_skip() & 4)) reduce_kernel<<<total_blocks, 256, 0, sw>>>(jobs);
+    reduce_kernel<<<total_blocks, 256, 0, sw>>>(jobs);
     if ((st = launch_status()) != PSB_OK) return st;
   }
   if (fork_wgrad) {

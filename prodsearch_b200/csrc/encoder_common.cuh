@@ -7,7 +7,7 @@
 // every product exist: fp32 FFMA CTA tiles of R = 16/24 rows (this header's tile_gemm; ~100-200
 // CTAs, weights streamed from L2 once per CTA, activations broadcast from shared memory) -- the
 // fallback for any d <= 128 / ff <= 1024 -- and, for d = 128 / ff = 512, 3xTF32 products on tcgen05
-// chained inside cluster kernels (gemm3_tf32.cu), the default since round 2 (PSB_ENC_TC).
+// chained inside cluster kernels (gemm3_tf32.cu), the default since round 2 (PSB_ENC_TC=0 selects the FFMA path).
 #pragma once
 #include "psb_common.cuh"
 
@@ -287,7 +287,7 @@ struct Saved {
   size_t ctx, y, n, z, pre1, h1;    // [S*C,d] x4, [S*C,F] x2
   // transposed tail weights for the tensor-core backward tail (gemm3_tf32.cu tail_bwd_fused_tc_kernel), split into tf32
   // hi part and exact remainder, hi rows stacked on lo rows: Wo^T [2][d][d], W1^T [2][d][F], W2^T [2][F][d].  Written by
-  // the forward pass's transpose launch (they are this step's weights) when PSB_ENC_TC >= 3.
+  // the forward pass's transpose launch (they are this step's weights) on the tensor-core path.
   size_t wot_hl, w1t_hl, w2t_hl;
   size_t wkv_t;                     // [Wk^T | Wv^T] : [d][2d], the K-major operand of the backward's grad-xn product on tcgen05
   size_t total;                     // floats
@@ -382,16 +382,16 @@ struct TrJobs {
 int launch_transposes(const TrJobs& jobs, cudaStream_t s);   // encoder_fwd.cu: weight transposes, one launch
 int launch_rows_gemm(const float* A, int lda, const int32_t* m_dev, int m_host, int m_max, int I, const float* B,
                      int J, const float* bias, float* out, int ldo, cudaStream_t s);
-// gemm3_tf32.cu: the same product on tcgen05 (3xTF32 split) from the K-major operand Bt [J][K] (rows [split, J) from
-// Bt1 when given); off unless PSB_ENC_TC=1
-bool rows_gemm_tc_enabled();
-bool rows_gemm_tc_auto(int64_t m_max);
+// gemm3_tf32.cu: true = the tensor-core path (default), false = the FFMA path for every encoder product (PSB_ENC_TC=0)
+bool enc_tc_enabled();
+// launch_rows_gemm's product on tcgen05 (3xTF32 split) from the K-major operand Bt [J][K] (rows [split, J) from Bt1 when
+// given)
 bool rows_gemm_tc_supported(const float* A, int lda, int K, const float* Bt0, const float* Bt1, int split, int J,
                             const float* bias, const float* out, int ldo);
 int launch_rows_gemm_tc(const float* A, int lda, const int32_t* m_dev, int m_host, int m_max, int K, const float* Bt0,
                         const float* Bt1, int split, int J, const float* bias, float* out, int ldo, cudaStream_t s);
-// PSB_ENC_TC=2: the forward tail (encoder_fwd.cu tail_fwd_kernel) as a ctx kernel + three of those GEMMs with fused
-// epilogues, on the original (K-major) weights; same saved tensors, same dropout streams
+// The forward tail (encoder_fwd.cu tail_fwd_kernel) on tcgen05: ctx kernel + ONE cluster kernel chaining the three
+// products (FFN hidden dimension split over 4 CTAs); same saved tensors, same dropout streams
 struct TailTcArgs {
   Dims D;
   const int32_t *nact, *off, *tok;
@@ -401,19 +401,13 @@ struct TailTcArgs {
   float *ctx, *y, *n, *z, *pre1, *h1;            // saved for the backward pass
   float* out;
   const uint64_t* seed_dev;
-  const float *wo_hl, *w1_hl, *w2_hl;            // fused tail only: pre-split weights (FwdWs), written by the transpose launch
-  float* ctx_hl;                                 // fused tail only: pre-split ctx rows
-  int save_dact;                                 // fused tail only: the pre1 slot receives dropout_3 . gelu'(pre1)
+  const float *wo_hl, *w1_hl, *w2_hl;            // pre-split weights (FwdWs), written by the transpose launch
+  float* ctx_hl;                                 // pre-split ctx rows
+  int save_dact;                                 // the pre1 slot receives dropout_3 . gelu'(pre1)
 };
-bool tail_tc_enabled();
-bool tail_tc3_enabled();
-bool tail_tc_supported(const TailTcArgs& a);
-int launch_tail_fwd_tc(const TailTcArgs& a, cudaStream_t s);
-// PSB_ENC_TC=3: ctx kernel + ONE cluster kernel chaining the three products (FFN hidden dimension split over 4 CTAs)
-bool tail_fused_enabled();
 bool tail_fused_supported(const TailTcArgs& a);
 int launch_tail_fwd_fused(const TailTcArgs& a, cudaStream_t s);
-// PSB_ENC_TC=4: the backward tail's product chain (LN_out' -> W2' -> gelu' -> W1' -> LN_ff' -> Wo') as ONE cluster kernel
+// The backward tail's product chain (LN_out' -> W2' -> gelu' -> W1' -> LN_ff' -> Wo') as ONE cluster kernel
 // in the transposed form (weights are the M operand, the 128 copy rows the N operand: every global access of the
 // epilogues runs along a row); the attention backward then reads gy / g_ctx from global memory (tail_bwd_kernel<R, true>)
 struct TailBwdTcArgs {
@@ -424,7 +418,6 @@ struct TailBwdTcArgs {
   float* lnp;                                    // [4 * tiles][4][d]
   const uint64_t* seed_dev;
 };
-bool tail_bwd_fused_enabled();
 unsigned long long* ft_trace_buffer();           // PSB_FT_TRACE=1: 64 %globaltimer slots (psb_debug_tail_trace), else NULL
 // Shared-memory floats of tail_attn_bwd_kernel (encoder_bwd.cu) for a tile of spt sequences, R = spt * C copy rows
 __host__ __device__ inline size_t attn_bwd_smem_floats(int R, int d, int H, int T, int spt) {
@@ -440,7 +433,7 @@ inline int attn_bwd_spt(const Dims& D) {
   return spt;
 }
 inline bool tail_bwd_fused_for(const Dims& D) {
-  return tail_bwd_fused_enabled() && tail_fused_enabled() && D.d == 128 && D.F == 512 && D.S * D.C > 0 && attn_bwd_spt(D) > 0;
+  return enc_tc_enabled() && D.d == 128 && D.F == 512 && D.S * D.C > 0 && attn_bwd_spt(D) > 0;
 }
 int tail_bwd_fused_parts(const Dims& D);         // LayerNorm partial rows the kernel writes (4 per 128-row tile)
 bool tail_bwd_fused_supported(const TailBwdTcArgs& a);

@@ -9,8 +9,9 @@
 //   attn       per sequence: scores of the ONE query position, softmax -> P
 //   tail       per tile of R copy-rows: dropout(P) V -> Wo -> +x[o] -> LN -> W1 -> gelu -> W2 ->
 //              +y -> LN, everything between the two HBM touches kept in shared memory
-// With PSB_ENC_TC >= 1 (default 4) the projections run on tcgen05 (gemm3_tf32_kernel) and the tail is
-// tail_ctx_kernel + tail_fused_tc_kernel (gemm3_tf32.cu); the FFMA kernels below stay the fallback.
+// On the tensor-core path (the default) the projections run on tcgen05 (gemm3_tf32_kernel) and the tail is
+// tail_ctx_kernel + tail_fused_tc_kernel (gemm3_tf32.cu); the FFMA kernels below are the FFMA path (PSB_ENC_TC=0) and
+// the fallback for the shapes the tensor-core kernels do not take.
 #include "encoder_common.cuh"
 
 namespace psb {
@@ -593,11 +594,12 @@ extern "C" int psb_encoder_fwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
   add(p->w2, ws + W.w2_t, d, F, d, 0);           // W2 [d][F] -> [F][d]
   add(p->bk, ws + W.bkv, d, 1, 2 * d, 0);        // bias concat as 1-column "transposes"
   add(p->bv, ws + W.bkv, d, 1, 2 * d, d);
-  if (rows_gemm_tc_enabled()) {                    // the backward's grad-xn product reads [Wk^T | Wv^T] from the saved state
+  const bool tc = enc_tc_enabled();
+  if (tc) {                                        // the backward's grad-xn product reads [Wk^T | Wv^T] from the saved state
     add(p->wk, sv + L.wkv_t, d, d, 2 * d, 0);
     add(p->wv, sv + L.wkv_t, d, d, 2 * d, d);
   }
-  const bool fused_tail = tail_fused_enabled() && d == 128 && F == 512;
+  const bool fused_tail = tc && d == 128 && F == 512;
   if (fused_tail) {                                // hi / lo parts of the tail's weights for tail_fused_tc_kernel
     add(p->wo, ws + W.wo_hl, d, d, -1, 0);
     add(p->w1, ws + W.w1_hl, F, d, -1, 0);
@@ -633,10 +635,9 @@ extern "C" int psb_encoder_fwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
 
   // [K | V] rows of the active tokens, q of the output position
   // (independent products: the small q projection runs on the library's side stream next to the K|V one)
-  // PSB_ENC_TC=1: both products on tcgen05 (gemm3_tf32.cu) straight from the K-major weights Wq / Wk / Wv
-  const bool tc_q = rows_gemm_tc_enabled() && rows_gemm_tc_supported(sv + L.xno, d, d, p->wq, nullptr, 0, d, p->bq, sv + L.qv, d);
-  const bool tc_kv = (rows_gemm_tc_enabled() || rows_gemm_tc_auto(static_cast<int64_t>(D.S) * D.T)) &&
-                     rows_gemm_tc_supported(sv + L.xn, d, d, p->wk, p->wv, d, 2 * d, ws + W.bkv, sv + L.kv, 2 * d);
+  // tensor-core path: both products on tcgen05 (gemm3_tf32.cu) straight from the K-major weights Wq / Wk / Wv
+  const bool tc_q = tc && rows_gemm_tc_supported(sv + L.xno, d, d, p->wq, nullptr, 0, d, p->bq, sv + L.qv, d);
+  const bool tc_kv = tc && rows_gemm_tc_supported(sv + L.xn, d, d, p->wk, p->wv, d, 2 * d, ws + W.bkv, sv + L.kv, 2 * d);
   st = fork_join(
       s, 1,
       [&](cudaStream_t s2) {
@@ -658,8 +659,8 @@ extern "C" int psb_encoder_fwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
                                                                                    sv + L.kv, sv + L.p);
   if ((st = launch_status()) != PSB_OK) return st;
 
-  if (tail_tc_enabled()) {
-    // PSB_ENC_TC=2: ctx kernel + three 3xTF32 tcgen05 GEMMs with fused epilogues (gemm3_tf32.cu) on the original weights
+  if (fused_tail) {
+    // tensor-core path: ctx kernel + one cluster kernel chaining the tail's three products (gemm3_tf32.cu)
     TailTcArgs t;
     t.D = D;
     t.nact = nact; t.off = off; t.tok = tok;
@@ -671,8 +672,7 @@ extern "C" int psb_encoder_fwd(const psb_encoder_cfg_t* cfg, const psb_encoder_p
     t.seed_dev = cfg->seed_dev;
     t.wo_hl = ws + W.wo_hl; t.w1_hl = ws + W.w1_hl; t.w2_hl = ws + W.w2_hl; t.ctx_hl = ws + W.ctx_hl;
     t.save_dact = tail_bwd_fused_for(D) ? 1 : 0;
-    if (fused_tail) return tail_fused_supported(t) ? launch_tail_fwd_fused(t, s) : PSB_E_ALIGN;
-    if (tail_tc3_enabled() && tail_tc_supported(t)) return launch_tail_fwd_tc(t, s);
+    return tail_fused_supported(t) ? launch_tail_fwd_fused(t, s) : PSB_E_ALIGN;
   }
   TailFwdArgs a;
   a.D = D;

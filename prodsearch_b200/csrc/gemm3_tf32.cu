@@ -19,19 +19,19 @@
 //   warp 1      MMA issuer (converged warp, elected-lane predicate: see catalog_tc.cu tc_mma_f16_if for why):
 //               per k-step of 8: main += hi.hi, corr += lo.hi, corr += hi.lo   (M 128, N, K 8)
 //   warps 2..5  epilogue: thread = output row (TMEM lane) holding its N sums (main + corr) in registers, handed to an
-//               epilogue functor: bias (projections), bias + gelu + dropout (FFN up), or bias + dropout + residual +
-//               LayerNorm over the whole d = 128 row (out-projection, FFN down) -- a row never leaves its thread
+//               epilogue functor (EpiBias: out = acc + bias) -- a row never leaves its thread
 // Rows >= M (M may live on the device: the number of active tokens) are computed on whatever the buffer holds and not
 // stored; a GEMM row depends on its own A row only.  CTAs whose first row is >= M exit at once.
 //
-// This file holds every tensor-core form of the encoder (levels of PSB_ENC_TC, see enc_tc_level below; 4 is the default):
+// This file holds the encoder's tensor-core path (the default; PSB_ENC_TC=0 selects the FFMA path, see enc_tc_enabled):
 //   gemm3_tf32_kernel          one product with a fused epilogue: the q / K|V projections, the backward's grad-xn product
 //   tail_ctx_kernel + tail_fused_tc_kernel      the forward tail as ONE cluster kernel (three chained products)
 //   tail_bwd_fused_tc_kernel   the backward tail's product chain as one cluster kernel, transposed form
 //                              (+ encoder_bwd.cu tail_attn_bwd_kernel for the attention backward)
 // All of them have run on B200s: profiles/r02a_gemm3.jsonl (accuracy against fp64), profiles/r02W_diff_enc_*.jsonl (stage by
-// stage against the FFMA kernels), tests/test_gpu_enc_tc_levels.py (every level, every round).
+// stage against the FFMA kernels), tests/test_gpu_enc_tc_levels.py (forward and backward, every round).
 #include <stdlib.h>
+#include <string.h>
 
 #include "encoder_common.cuh"
 #include "tc_ptx.cuh"
@@ -119,94 +119,6 @@ struct EpiBias {
       }
       *reinterpret_cast<float4*>(o + i) = r;
     }
-  }
-};
-
-// FFN first layer (encoder_fwd.cu tail_fwd_kernel step 5): pre1 = acc + b1 (saved), h1 = dropout_3(gelu(pre1)) (saved)
-template <int N>
-struct EpiFfnUp {
-  const float* b1;
-  float *pre1, *h1;
-  int F;
-  const uint64_t* seed_dev;
-  uint32_t thr;
-  float keep;
-  __device__ __forceinline__ void operator()(int row, int n0, float (&acc)[N]) const {
-    const Drop drop = make_drop(seed_dev, thr, keep);
-    const size_t base = static_cast<size_t>(row) * F + n0;
-#pragma unroll
-    for (int i = 0; i < N; i += 4) {
-      const float4 b = *reinterpret_cast<const float4*>(b1 + n0 + i);
-      const float4 v = make_float4(acc[i] + b.x, acc[i + 1] + b.y, acc[i + 2] + b.z, acc[i + 3] + b.w);
-      *reinterpret_cast<float4*>(pre1 + base + i) = v;
-      float4 h = make_float4(gelu_tanh(v.x), gelu_tanh(v.y), gelu_tanh(v.z), gelu_tanh(v.w));
-      if (drop.on()) {
-        const float4 m = drop.mul4(3u, base + i);
-        h.x *= m.x; h.y *= m.y; h.z *= m.z; h.w *= m.w;
-      }
-      *reinterpret_cast<float4*>(h1 + base + i) = h;
-    }
-  }
-};
-
-// Projection + dropout + residual + LayerNorm over the whole d = N = 128 row (tail_fwd_kernel steps 3 + 4 and 6 + 7):
-// pre = dropout_sid(acc + bias) + res[row / res_div] (saved), out = LN(pre).  The row sums are formed in the order the
-// warp-per-row kernels use (lane l holds columns 4l..4l+3, then the xor butterfly 16, 8, 4, 2, 1).
-template <int N>
-struct EpiResLn {
-  static_assert(N == 128, "the LayerNorm epilogue owns the whole d = 128 row");
-  const float *bias, *res, *ln_g, *ln_b;
-  float *pre, *out;
-  int res_div;
-  uint32_t sid;
-  float eps;
-  const uint64_t* seed_dev;
-  uint32_t thr;
-  float keep;
-  __device__ __forceinline__ static float butterfly(float (&s)[32]) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int l = 0; l < 32; ++l)
-        if ((l & o) == 0) {                 // both partners get s[l] + s[l ^ o] (addition commutes): keep one copy
-          const float t = s[l] + s[l ^ o];
-          s[l] = t;
-          s[l ^ o] = t;
-        }
-    }
-    return s[0];
-  }
-  __device__ __forceinline__ void operator()(int row, int /*n0*/, float (&acc)[N]) const {
-    const Drop drop = make_drop(seed_dev, thr, keep);
-    const size_t base = static_cast<size_t>(row) * N;
-    const float* r = res + static_cast<size_t>(row / res_div) * N;
-    float part[32];
-#pragma unroll
-    for (int i = 0; i < N; i += 4) {
-      const float4 b = *reinterpret_cast<const float4*>(bias + i);
-      float4 v = make_float4(acc[i] + b.x, acc[i + 1] + b.y, acc[i + 2] + b.z, acc[i + 3] + b.w);
-      if (drop.on()) {
-        const float4 m = drop.mul4(sid, base + i);
-        v.x *= m.x; v.y *= m.y; v.z *= m.z; v.w *= m.w;
-      }
-      const float4 x = *reinterpret_cast<const float4*>(r + i);
-      v.x += x.x; v.y += x.y; v.z += x.z; v.w += x.w;
-      *reinterpret_cast<float4*>(pre + base + i) = v;
-      acc[i] = v.x; acc[i + 1] = v.y; acc[i + 2] = v.z; acc[i + 3] = v.w;
-      part[i >> 2] = (v.x + v.y) + (v.z + v.w);
-    }
-    const float mean = butterfly(part) / static_cast<float>(N);
-#pragma unroll
-    for (int i = 0; i < N; i += 4) {
-      const float a0 = acc[i] - mean, a1 = acc[i + 1] - mean, a2 = acc[i + 2] - mean, a3 = acc[i + 3] - mean;
-      part[i >> 2] = (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3);
-    }
-    const RowStats st{mean, 1.f / sqrtf(butterfly(part) / static_cast<float>(N) + eps)};
-#pragma unroll
-    for (int i = 0; i < N; i += 4)
-      *reinterpret_cast<float4*>(out + base + i) =
-          ln_apply(make_float4(acc[i], acc[i + 1], acc[i + 2], acc[i + 3]), st, *reinterpret_cast<const float4*>(ln_g + i),
-                   *reinterpret_cast<const float4*>(ln_b + i));
   }
 };
 
@@ -368,38 +280,18 @@ static int g3_make_map(CUtensorMap* map, const float* base, int64_t rows, int64_
   return r == CUDA_SUCCESS ? PSB_OK : PSB_E_ARG;
 }
 
-// PSB_ENC_TC, read once per process.  Unset = 4: every encoder product that has a tensor-core form runs on tcgen05 --
-//   1  forward q and K|V projections (gemm3_tf32_kernel)
-//   2  1 + the forward tail as ctx kernel + three 3xTF32 GEMMs with fused epilogues (launch_tail_fwd_tc; measured slower
-//      than the FFMA tail at TEM's size, kept for comparison: only PSB_ENC_TC=2 exactly selects it)
-//   3  1 + the forward tail as ctx kernel + ONE cluster kernel (tail_fused_tc_kernel)
-//   4  3 + the backward tail's product chain as one cluster kernel (tail_bwd_fused_tc_kernel) + tail_attn_bwd_kernel
-//   0  the fp32 FFMA kernels everywhere (encoder_fwd.cu / encoder_bwd.cu), also the fallback for shapes the tensor-core
-//      kernels do not take (d != 128, ff != 512, misaligned operands)
-static int enc_tc_level() {
+// PSB_ENC_TC=0 selects the fp32 FFMA kernels everywhere (encoder_fwd.cu / encoder_bwd.cu): the reference the tests compare
+// the tensor-core path against.  Unset, or any other value: every encoder product that has a tensor-core form runs on
+// tcgen05 (the projections, the forward tail, the backward tail).  The FFMA kernels also remain the fallback for the shapes
+// the tensor-core kernels do not take (d != 128, ff != 512, misaligned operands).  Read once per process.
+bool enc_tc_enabled() {
   static int v = -1;
   if (v < 0) {
     const char* e = getenv("PSB_ENC_TC");
-    const int x = e != nullptr ? atoi(e) : 4;
-    v = (x >= 0 && x <= 4) ? x : 4;
+    v = (e != nullptr && strcmp(e, "0") == 0) ? 0 : 1;
   }
-  return v;
+  return v == 1;
 }
-bool rows_gemm_tc_enabled() { return enc_tc_level() >= 1; }
-// Unset PSB_ENC_TC: the K|V projection goes to tcgen05 by itself once it is big enough to be throughput- rather than
-// latency-bound: from 16 384 token rows on (RTM: 384 x 51 = 19.6k rows for the positives, 1920 x 51 = 98k for the
-// negatives: 0.31 ms on FFMA, 0.06 ms here); at TEM's 8k-row plan (~3.5k active rows) the FFMA kernel is as fast
-// (profiles/r02a_bench_enc_tc.json).  PSB_ENC_TC=0 switches the automatic choice off.
-bool rows_gemm_tc_auto(int64_t m_max) {
-  static int allowed = -1;
-  if (allowed < 0) {
-    const char* e = getenv("PSB_ENC_TC");
-    allowed = (e != nullptr && atoi(e) == 0 && e[0] == '0') ? 0 : 1;
-  }
-  return allowed == 1 && m_max >= 16384;
-}
-bool tail_tc_enabled() { return enc_tc_level() >= 2; }       // some tensor-core forward tail
-bool tail_tc3_enabled() { return enc_tc_level() == 2; }      // the three-GEMM form of it
 
 // One launch: out-tile epilogue `epi` over A [m rows, K] (row stride lda) and Bt rows [0, split) from Bt0, the rest from Bt1
 template <int N, int KC, class Epi>
@@ -457,7 +349,7 @@ int launch_rows_gemm_tc(const float* A, int lda, const int32_t* m_dev, int m_hos
   return g3_launch<64, 64>("gemm3_tf32_kernel", A, lda, m_dev, m_host, m_max, K, Bt0, Bt1, split, J, epi, s);
 }
 
-// ------------------------------------------------------------------ forward tail on tcgen05 (PSB_ENC_TC=2)
+// ------------------------------------------------------------------ forward tail: attention context
 // Steps 1 + 2 of tail_fwd_kernel on their own: ctx[row] = sum_al dropout_1(P)[h, al] * V[al], one warp per copy row,
 // lane = 4 columns (d = 128), the same sequential fmaf chain over the active tokens -> the same bits.
 __global__ void __launch_bounds__(256) tail_ctx_kernel(Dims D, const int32_t* __restrict__ nact, const int32_t* __restrict__ off,
@@ -531,44 +423,7 @@ __global__ void __launch_bounds__(256) tail_ctx_kernel(Dims D, const int32_t* __
   }
 }
 
-bool tail_tc_supported(const TailTcArgs& a) {
-  const Dims& D = a.D;
-  if (D.d != 128 || D.F % 64 != 0 || D.F <= 0) return false;
-  if (a.P == nullptr || a.nact == nullptr || a.off == nullptr || a.tok == nullptr) return false;
-  const float* ptrs[] = {a.kv, a.xo, a.wo, a.bo, a.w1, a.b1, a.w2, a.b2, a.ln_ff_g, a.ln_ff_b, a.ln_out_g,
-                         a.ln_out_b, a.ctx, a.y, a.n, a.z, a.pre1, a.h1, a.out};
-  for (const float* q : ptrs)
-    if (q == nullptr || misaligned16(q)) return false;
-  return true;
-}
-
-int launch_tail_fwd_tc(const TailTcArgs& a, cudaStream_t s) {
-  if (!tail_tc_supported(a)) return PSB_E_UNSUPPORTED;
-  const Dims& D = a.D;
-  const int SC = D.S * D.C, d = D.d, F = D.F;
-  int st;
-  PSB_PROF("tail_ctx_kernel", s);
-  tail_ctx_kernel<<<(SC + 7) / 8, 256, 0, s>>>(D, a.nact, a.off, a.tok, a.P, a.kv, a.ctx, a.seed_dev);
-  if ((st = launch_status()) != PSB_OK) return st;
-  // y = dropout_2(ctx . Wo^T + bo) + x[o];  n = LN_ff(y)
-  EpiResLn<128> e1;
-  e1.bias = a.bo; e1.res = a.xo; e1.ln_g = a.ln_ff_g; e1.ln_b = a.ln_ff_b; e1.pre = a.y; e1.out = a.n;
-  e1.res_div = D.C; e1.sid = 2u; e1.eps = D.eps; e1.seed_dev = a.seed_dev; e1.thr = D.thr; e1.keep = D.keep;
-  if ((st = g3_launch<128, 32>("gemm3_out_proj_ln_kernel", a.ctx, d, nullptr, SC, SC, d, a.wo, nullptr, 0, d, e1, s)) != PSB_OK)
-    return st;
-  // pre1 = n . W1^T + b1;  h1 = dropout_3(gelu(pre1))
-  EpiFfnUp<64> e2;
-  e2.b1 = a.b1; e2.pre1 = a.pre1; e2.h1 = a.h1; e2.F = F; e2.seed_dev = a.seed_dev; e2.thr = D.thr; e2.keep = D.keep;
-  if ((st = g3_launch<64, 64>("gemm3_ffn_up_kernel", a.n, d, nullptr, SC, SC, d, a.w1, nullptr, 0, F, e2, s)) != PSB_OK) return st;
-  // z = dropout_4(h1 . W2^T + b2) + y;  out = LN_out(z)
-  EpiResLn<128> e3;
-  e3.bias = a.b2; e3.res = a.y; e3.ln_g = a.ln_out_g; e3.ln_b = a.ln_out_b; e3.pre = a.z; e3.out = a.out;
-  e3.res_div = 1; e3.sid = 4u; e3.eps = D.eps; e3.seed_dev = a.seed_dev; e3.thr = D.thr; e3.keep = D.keep;
-  return g3_launch<128, 32>("gemm3_ffn_down_ln_kernel", a.h1, F, nullptr, SC, SC, F, a.w2, nullptr, 0, d, e3, s);
-}
-
-
-// ------------------------------------------------------------------ forward tail as ONE cluster kernel (PSB_ENC_TC=3)
+// ------------------------------------------------------------------ forward tail as ONE cluster kernel
 // tail_ctx_kernel, then tail_fused_tc_kernel: the three products of the tail (out-projection, FFN up, FFN down) chained
 // inside one launch, the FFN's hidden dimension split over a cluster of 4 CTAs.
 //
@@ -599,7 +454,6 @@ struct FtParams {
   const float *xo, *bo, *b1, *b2, *ln_ff_g, *ln_ff_b, *ln_out_g, *ln_out_b;
   float *y, *n, *z, *pre1, *h1, *out;
   const uint64_t* seed_dev;
-  int exp;                     // PSB_FT_EXP (timing experiments only): 1 = no pre1 / h1 stores, 2 = no gelu
   int save_dact;               // the pre1 slot receives dropout_3 . gelu'(pre1) (what the tensor-core backward multiplies by)
   unsigned long long* trace;   // PSB_FT_TRACE=1: %globaltimer at the phase boundaries of CTA 0 (psb_debug_tail_trace)
 };
@@ -950,7 +804,7 @@ tail_fused_tc_kernel(const __grid_constant__ CUtensorMap map_ctx, const __grid_c
       __syncwarp();
       if (lane == 0) mbar_arrive(a_ready + 2);
       // off the critical path, next to the phase-3 MMAs: h1 = hi + lo row-contiguous (pre1 follows at the very end)
-      if (!(P.exp & 1)) ft_store_block<true>(a_hi, a_lo, quarter, cg, P.h1, F, r0, q * 128 + c0, P.SC, 0, 8);
+      ft_store_block<true>(a_hi, a_lo, quarter, cg, P.h1, F, r0, q * 128 + c0, P.SC, 0, 8);
     }
     // ---- epilogue 3: this CTA's partial sums of the FFN's second product -> shared memory, [chunk][row] float4
     mbar_wait(acc_full + 2, 0);
@@ -1023,7 +877,7 @@ tail_fused_tc_kernel(const __grid_constant__ CUtensorMap map_ctx, const __grid_c
   // ---- pre1 = acc2 + b1, the last saved tensor: the phase-2 accumulators are still in TMEM; staged through the (dead) lo
   //      tile in the A layout so that the stores are row-contiguous like h1's.  With the tensor-core backward
   //      (save_dact) the slot holds dropout_3 . gelu'(pre1) instead: all the backward pass ever forms from pre1.
-  if (warp >= 2 && !(P.exp & 1)) {
+  if (warp >= 2) {
     const int e = warp - 2, quarter = warp & 3, cg = e >> 2, c0 = cg * 32;
     const int rl = quarter * 32 + lane;
     float v[32];
@@ -1054,8 +908,6 @@ tail_fused_tc_kernel(const __grid_constant__ CUtensorMap map_ctx, const __grid_c
   }
 }
 
-bool tail_fused_enabled() { return enc_tc_level() >= 3; }
-
 // PSB_FT_TRACE=1: a 64-slot device buffer CTA 0 of the fused tail kernels stamps with %globaltimer (forward: slots 0..31,
 // backward: 32..63; read back by psb_debug_tail_trace)
 unsigned long long* ft_trace_buffer() {
@@ -1073,9 +925,14 @@ unsigned long long* ft_trace_buffer() {
 }
 
 bool tail_fused_supported(const TailTcArgs& a) {
-  return tail_tc_supported(a) && a.D.F == 128 * kFtCluster && a.D.S * a.D.C > 0 && a.wo_hl != nullptr && a.w1_hl != nullptr &&
-         a.w2_hl != nullptr && a.ctx_hl != nullptr && !misaligned16(a.wo_hl) && !misaligned16(a.w1_hl) &&
-         !misaligned16(a.w2_hl) && !misaligned16(a.ctx_hl);
+  const Dims& D = a.D;
+  if (D.d != 128 || D.F != 128 * kFtCluster || D.S * D.C <= 0) return false;
+  if (a.P == nullptr || a.nact == nullptr || a.off == nullptr || a.tok == nullptr) return false;
+  const float* ptrs[] = {a.kv, a.xo, a.wo, a.bo, a.w1, a.b1, a.w2, a.b2, a.ln_ff_g, a.ln_ff_b, a.ln_out_g, a.ln_out_b,
+                         a.ctx, a.y, a.n, a.z, a.pre1, a.h1, a.out, a.wo_hl, a.w1_hl, a.w2_hl, a.ctx_hl};
+  for (const float* q : ptrs)
+    if (q == nullptr || misaligned16(q)) return false;
+  return true;
 }
 
 int launch_tail_fwd_fused(const TailTcArgs& a, cudaStream_t s) {
@@ -1112,10 +969,6 @@ int launch_tail_fwd_fused(const TailTcArgs& a, cudaStream_t s) {
   P.seed_dev = a.seed_dev;
   P.trace = ft_trace_buffer();
   P.save_dact = a.save_dact;
-  {
-    const char* e = getenv("PSB_FT_EXP");
-    P.exp = e != nullptr ? atoi(e) : 0;
-  }
   const unsigned tiles = static_cast<unsigned>((SC + 127) / 128);
   PSB_PROF("tail_fused_tc_kernel", s);
   {
@@ -1127,7 +980,7 @@ int launch_tail_fwd_fused(const TailTcArgs& a, cudaStream_t s) {
 }
 
 
-// ------------------------------------------------------------------ backward tail as ONE cluster kernel (PSB_ENC_TC=4)
+// ------------------------------------------------------------------ backward tail as ONE cluster kernel
 // encoder_bwd.cu tail_bwd_kernel steps (1)..(6) on tcgen05, TRANSPOSED: the weights are the M operand (128 output
 // features = TMEM lanes) and the tile's 128 copy rows the N operand (TMEM columns), so a thread of the epilogue owns one
 // feature for 32 rows and every global load / store of the epilogues runs along a row (coalesced), and the activation
@@ -1475,7 +1328,6 @@ tail_bwd_fused_tc_kernel(const __grid_constant__ CUtensorMap map_w2t, const __gr
   }
 }
 
-bool tail_bwd_fused_enabled() { return enc_tc_level() >= 4; }
 int tail_bwd_fused_parts(const Dims& D) { return ((D.S * D.C + 127) / 128) * kFtCluster; }
 
 bool tail_bwd_fused_supported(const TailBwdTcArgs& a) {

@@ -1,10 +1,10 @@
-"""Backward of the encoder with the tensor-core tail (PSB_ENC_TC=4, csrc/gemm3_tf32.cu tail_bwd_fused_tc_kernel) against
+"""Backward of the encoder on the tensor-core path (the default, csrc/gemm3_tf32.cu tail_bwd_fused_tc_kernel) against
 the FFMA kernels (PSB_ENC_TC=0): the same seeded TEM-layout call (batch 384, 21 positions, d 128, ff 512, 8 heads, 1 + 5
-copies, dropout 0.1 on a fixed Philox seed) and the same upstream gradient run once per level in their own subprocesses;
+copies, dropout 0.1 on a fixed Philox seed) and the same upstream gradient run once per path in their own subprocesses;
 every gradient the backward returns (grad_first, grad_rest, all 18 parameter gradients) and the backward workspace's
 intermediate regions (g_h2, g_pre, g_o1, gxo, g_qlin, gkv) are compared, largest difference over the tensor's maximum.
 
-    timeout 300 python profiles/diff_enc_bwd_tc.py [levels]       # one JSON line per (level, tensor)"""
+    timeout 300 python profiles/diff_enc_bwd_tc.py       # one JSON line per tensor"""
 import json
 import os
 import subprocess
@@ -54,28 +54,28 @@ np.savez(sys.argv[1], **{k: v.detach().cpu().numpy() for k, v in res.items()})
 ''' % (ROOT, S, T, D, FF, H, C)
 
 
-def run(level, path):
-    env = dict(os.environ, PSB_ENC_TC=str(level))
+def run(path_name, path):
+    """path_name "ffma": PSB_ENC_TC=0; "tc": the default tensor-core path."""
+    env = {k: v for k, v in os.environ.items() if k != "PSB_ENC_TC"}
+    if path_name == "ffma":
+        env["PSB_ENC_TC"] = "0"
     try:
         r = subprocess.run([sys.executable, "-c", CHILD, path], env=env, capture_output=True, text=True, timeout=120)
     except subprocess.TimeoutExpired:
-        print(json.dumps({"level": level, "error": "timeout (hang?)"}))
+        print(json.dumps({"path": path_name, "error": "timeout (hang?)"}))
         return None
     if r.returncode != 0:
-        print(json.dumps({"level": level, "error": r.stderr[-800:]}))
+        print(json.dumps({"path": path_name, "error": r.stderr[-800:]}))
         return None
     return np.load(path)
 
 
 if __name__ == "__main__":
     tmp = tempfile.mkdtemp()
-    base = run(0, os.path.join(tmp, "l0.npz"))
-    ok = base is not None
-    for level in [int(x) for x in sys.argv[1:]] or [3, 4]:
-        got = run(level, os.path.join(tmp, "l%d.npz" % level)) if base is not None else None
-        if got is None:
-            ok = False
-            continue
+    base = run("ffma", os.path.join(tmp, "ffma.npz"))
+    got = run("tc", os.path.join(tmp, "tc.npz")) if base is not None else None
+    ok = got is not None
+    if ok:
         for name in base.files:
             a, b = base[name].astype(np.float64), got[name].astype(np.float64)
             # d_bk is zero in exact arithmetic (a key bias shifts every score of a softmax row alike): measured against d_bv
@@ -83,6 +83,6 @@ if __name__ == "__main__":
             err = float(np.abs(a - b).max() / max(scale, 1e-30))
             good = err < 3e-5 and bool(np.isfinite(b).all())
             ok = ok and good
-            print(json.dumps({"level": level, "tensor": name, "max_abs_diff_over_max": err, "ok": good}))
+            print(json.dumps({"path": "tc", "tensor": name, "max_abs_diff_over_max": err, "ok": good}))
     print("VERDICT:", "tensor-core backward agrees with the FFMA kernels" if ok else "MISMATCH or failure")
     sys.exit(0 if ok else 1)

@@ -1,7 +1,7 @@
-"""Timeline of the fused tensor-core encoder tail (PSB_ENC_TC=3, PSB_FT_TRACE=1): %globaltimer stamps of CTA 0 at its
+"""Timeline of the fused tensor-core encoder tail (the default path, PSB_FT_TRACE=1): %globaltimer stamps of CTA 0 at its
 phase boundaries, relative to the kernel's first instruction, for a few launches of the TEM-shaped forward call.
 
-    PSB_ENC_TC=3 PSB_FT_TRACE=1 timeout 200 python profiles/tail_trace.py"""
+    PSB_FT_TRACE=1 timeout 200 python profiles/tail_trace.py"""
 import ctypes
 import json
 import os

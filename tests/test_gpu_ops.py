@@ -458,10 +458,11 @@ def test_catalog_topk_tc_scaled_rows(ops):
 @pytest.mark.parametrize("m,n,k,with_bias", [(24, 100_000, 100, False), (130, 70_001, 100, True),
                                              (384, 1_000_000, 100, False), (5, 40_000, 10, True),
                                              (300, 250_000, 100, True), (513, 120_000, 50, False),
-                                             (1100, 90_000, 100, False)])
+                                             (1100, 90_000, 100, False), (2100, 150_000, 100, True)])
 def test_catalog_topk_f16_equals_exact(ops, m, n, k, with_bias):
-    """fp16 shortlist (1..4 query tiles per CTA, 1..3 query groups) + exact fp32 rescoring == the fp32 mode,
-    bit for bit, incl. ragged last item tile / last query tile and the bias path."""
+    """fp16 shortlist (1..4 query tiles per CTA, 1..9 query groups; from 16 query tiles on, 2 tiles per CTA at 128 items
+    per MMA) + exact fp32 rescoring == the fp32 mode, bit for bit, incl. ragged last item tile / last query tile and the
+    bias path."""
     from prodsearch_b200 import _lib
     g = torch.Generator(device="cuda").manual_seed(m + n)
     E = torch.randn(n + 1, 128, generator=g, device="cuda")

@@ -7,8 +7,6 @@
 // read from HBM exactly once per use and no [n, w, 1+k, d] tensor is ever materialised.
 // HBM-bound: algorithmic bytes per anchor = w * (1 + k) * d * 4 (rows) + d * 4 (anchor)
 // + d * 4 (grad_anchor) (+ k * d * 8 when per-negative anchors are used).
-#include <stdlib.h>
-
 #include "psb_common.cuh"
 
 namespace psb {
@@ -289,12 +287,11 @@ ns_loss_fast_kernel(const float4* __restrict__ anchor_a, const float4* __restric
 // w == 1 (one target position per anchor: the TEM score/loss tail, item_to_words and PV with pv_window_size 1):
 // every position is its own anchor, the masked-mean denominator is 1, and the kernel is a pure stream of
 // (anchor row, 1 + k table rows) reads.  NR = rows handled per anchor (1 + k <= NR; 6 for the reference's 5
-// negatives); row ids travel through the shuffles as int32.  DB: the rows of the NEXT anchor are requested
-// before the current anchor is evaluated (two row buffers).  Measured on the 16M-row table (profiles/r01f_ab.jsonl):
-// generic fast kernel 0.66 of HBM peak, this kernel with one row buffer 0.85, with two buffers 0.69 (103 registers
-// -> 2 CTAs/SM), so DB is kept only as a tuning variant.
-template <bool HAS_B, int NR, bool DB>
-__global__ void __launch_bounds__(256, (DB || HAS_B) ? 2 : 3)
+// negatives); row ids travel through the shuffles as int32.  One row buffer: requesting the next anchor's rows
+// into a second buffer before evaluating the current one measured 0.69 of HBM peak against 0.85 for this form on
+// the 16M-row table (profiles/r01i_ab.jsonl), because its 103 registers drop it to 2 CTAs/SM.
+template <bool HAS_B, int NR>
+__global__ void __launch_bounds__(256, HAS_B ? 2 : 3)
 ns_loss_w1_kernel(const float4* __restrict__ anchor_a, const float4* __restrict__ anchor_b,
                   const float4* __restrict__ table, int64_t table_rows, int d4,
                   const float* __restrict__ bias, const int64_t* __restrict__ pos_idx,
@@ -409,41 +406,15 @@ ns_loss_w1_kernel(const float4* __restrict__ anchor_a, const float4* __restrict_
     if (col_ok) grad_a[a_i * a_stride * d4 + lane] = ga;
   };
 
-  if (!DB) {
-    Meta mn;
-    fetch(i, mn);
-    for (; i < n; i += nw) {
-      const Meta m = mn;
-      float4 row[NR], a;
-      float bv;
-      issue(m, i, row, a, bv);
-      if (i + nw < n) fetch(i + nw, mn);
-      compute(m, i, row, a, bv);
-    }
-  } else {
-    Meta mA, mB;
-    float4 rowA[NR], rowB[NR], aA, aB;
-    float bA, bB = 0.f;
-    fetch(i, mA);
-    issue(mA, i, rowA, aA, bA);
-    mB = mA;
-    if (i + nw < n) fetch(i + nw, mB);
-    // one half-step: request the next anchor's rows into the idle buffer, evaluate the current one
-    auto half = [&](float4 (&rc)[NR], float4& ac, float& bc, Meta& mc, float4 (&rn)[NR], float4& an, float& bn,
-                    Meta& mnx) -> bool {
-      const bool has_next = i + nw < n;
-      Meta mnn = mc;
-      if (has_next) {
-        issue(mnx, i + nw, rn, an, bn);
-        if (i + 2 * nw < n) fetch(i + 2 * nw, mnn);
-      }
-      compute(mc, i, rc, ac, bc);
-      mc = mnn;   // meta of the anchor after next: its rows go into this (now idle) buffer
-      i += nw;
-      return has_next;
-    };
-    while (half(rowA, aA, bA, mA, rowB, aB, bB, mB) && half(rowB, aB, bB, mB, rowA, aA, bA, mA)) {
-    }
+  Meta mn;
+  fetch(i, mn);
+  for (; i < n; i += nw) {
+    const Meta m = mn;
+    float4 row[NR], a;
+    float bv;
+    issue(m, i, row, a, bv);
+    if (i + nw < n) fetch(i + nw, mn);
+    compute(m, i, row, a, bv);
   }
 }
 
@@ -559,7 +530,7 @@ extern "C" int psb_tem_loss_fwd(const float* enc_out, const float* table, int64_
   PSB_PROF("ns_loss_w1_kernel", s);
 #define PSB_TEM_LAUNCH(NR)                                                                                          \
   {                                                                                                                 \
-    const cudaError_t le = launch_pdl(ns_loss_w1_kernel<true, NR, false>, dim3(gridf), dim3(256), 0, s, a4, a4 + d4,  \
+    const cudaError_t le = launch_pdl(ns_loss_w1_kernel<true, NR>, dim3(gridf), dim3(256), 0, s, a4, a4 + d4,         \
                                       reinterpret_cast<const float4*>(table), table_rows, d4, bias, pos_idx, neg_idx, \
                                       nullptr, -1, nullptr, pos_weight, n, static_cast<int>(k), loss_rows, coef_pos,  \
                                       coef_neg, g4, g4 + d4, C, C, grad_scale);                                       \
@@ -583,16 +554,6 @@ extern "C" int psb_tem_loss_finish(const float* ps_rows, const float* il_rows, i
     if (le != cudaSuccess) return static_cast<int>(le);
   }
   return launch_status();
-}
-
-// Tuning knob read once: PSB_NS_W1 selects the w == 1 kernel variant (see psb_ns_loss_fwd).
-static int ns_w1_variant() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSB_NS_W1");
-    v = (e != nullptr && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1;
-  }
-  return v;
 }
 
 extern "C" int psb_score_rows(const float* anchor, const float* table, int64_t table_rows, int64_t d,
@@ -645,24 +606,19 @@ extern "C" int psb_ns_loss_fwd(const float* anchor_a, const float* anchor_b, con
       reinterpret_cast<const float4*>(table), table_rows, d4, bias, pos_idx, neg_idx, mask, pad_idx,       \
       neg_weight, pos_weight, n, static_cast<int>(w), static_cast<int>(k), loss, coef_pos, coef_neg,       \
       reinterpret_cast<float4*>(grad_anchor_a), reinterpret_cast<float4*>(grad_anchor_b))
-  if (w == 1 && d4 <= 32 && k <= 7 && table_rows < (1ll << 31) && ns_w1_variant() != 0) {
-    // variants (PSB_NS_W1 = 0 | 1 | 2, default 1): 0 generic fast kernel, 1 single row buffer at 3 CTAs/SM
-    // (measured 0.85 of HBM peak), 2 double-buffered rows at 2 CTAs/SM (0.69: the lost occupancy costs more)
-    const bool db = ns_w1_variant() == 2 && anchor_b == nullptr;
-    const int gridf = grid_for(n, 8, db ? 8 : 32);
+  if (w == 1 && d4 <= 32 && k <= 7 && table_rows < (1ll << 31)) {
+    const int gridf = grid_for(n, 8, 32);
     PSB_PROF("ns_loss_w1_kernel", s);
-#define PSB_W1_LAUNCH(HASB, NR, DB)                                                                          \
-  ns_loss_w1_kernel<HASB, NR, DB><<<gridf, 256, 0, s>>>(                                                      \
+#define PSB_W1_LAUNCH(HASB, NR)                                                                              \
+  ns_loss_w1_kernel<HASB, NR><<<gridf, 256, 0, s>>>(                                                          \
       reinterpret_cast<const float4*>(anchor_a), reinterpret_cast<const float4*>(anchor_b),                  \
       reinterpret_cast<const float4*>(table), table_rows, d4, bias, pos_idx, neg_idx, mask, pad_idx, neg_weight, \
       pos_weight, n, static_cast<int>(k), loss, coef_pos, coef_neg, reinterpret_cast<float4*>(grad_anchor_a),  \
       reinterpret_cast<float4*>(grad_anchor_b))
     if (anchor_b != nullptr) {
-      if (k <= 5) PSB_W1_LAUNCH(true, 6, false); else PSB_W1_LAUNCH(true, 8, false);
-    } else if (db) {
-      if (k <= 5) PSB_W1_LAUNCH(false, 6, true); else PSB_W1_LAUNCH(false, 8, true);
+      if (k <= 5) PSB_W1_LAUNCH(true, 6); else PSB_W1_LAUNCH(true, 8);
     } else {
-      if (k <= 5) PSB_W1_LAUNCH(false, 6, false); else PSB_W1_LAUNCH(false, 8, false);
+      if (k <= 5) PSB_W1_LAUNCH(false, 6); else PSB_W1_LAUNCH(false, 8);
     }
 #undef PSB_W1_LAUNCH
   } else if (d4 <= 32 && k <= 7) {

@@ -10,7 +10,6 @@
 //                      adds them in rank order (bit-identical result on every rank)
 //   peer_barrier       cross-GPU barrier on flag words in peer memory (release/acquire at system scope),
 //                      with a clock64 time-out that raises a device error flag instead of hanging
-#include <stdlib.h>
 #include <string.h>
 
 #include "psb_common.cuh"
@@ -69,24 +68,9 @@ __global__ void __launch_bounds__(32) peer_barrier_kernel(PeerPtrs flags, int ra
   }
 }
 
-// How a row that lives in a PEER's memory is loaded (PSB_PEER_LD, read once; profiles/peer_bw.py measures them):
-//   0  ld.global.nc.L1::no_allocate.v4   (the local-gather path: non-coherent / texture path)
-//   1  ld.global.v4                      (plain coherent load)
-//   2  ld.global.relaxed.sys.v4          (system-scope load)
-template <int MODE>
-__device__ __forceinline__ float4 ld_peer4(const float4* p) {
-  float4 v;
-  if (MODE == 0) {
-    v = ldg_row4(p);
-  } else if (MODE == 1) {
-    asm volatile("ld.global.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-  } else {
-    asm volatile("ld.global.relaxed.sys.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-  }
-  return v;
-}
-
-template <int R, int MODE>
+// Peer rows are loaded like local gathers (ldg_row4, the non-coherent path): the plain coherent and the system-scope
+// loads measured within 5 % of it on an isolated remote fetch (profiles/r02j_peer_bw_n2.jsonl, r02m_peer_bw_n2.jsonl).
+template <int R>
 __global__ void __launch_bounds__(256)
 peer_gather_rows_kernel(PeerPtrs shards, int G, int64_t rows_total, int d4, const int64_t* __restrict__ idx, int64_t n,
                         float4* __restrict__ out, int64_t* __restrict__ remap, int64_t pad_id, int64_t pad_pos,
@@ -119,7 +103,7 @@ peer_gather_rows_kernel(PeerPtrs shards, int G, int64_t rows_total, int d4, cons
     for (int c = lane; c < d4; c += 32) {
       float4 v[R];
 #pragma unroll
-      for (int i = 0; i < R; ++i) v[i] = src[i] != nullptr ? ld_peer4<MODE>(src[i] + c) : zero4();
+      for (int i = 0; i < R; ++i) v[i] = src[i] != nullptr ? ldg_row4(src[i] + c) : zero4();
 #pragma unroll
       for (int i = 0; i < R; ++i)
         if (base + i < n) stg4(out + (base + i) * d4 + c, v[i]);
@@ -180,12 +164,12 @@ peer_gather_rows_lazy_kernel(LazyShards S, int G, int64_t rows_total, int d4, co
       float4 v[R];
 #pragma unroll
       for (int i = 0; i < R; ++i)
-        v[i] = owner[i] >= 0 ? ld_peer4<0>(static_cast<const float4*>(S.p[owner[i]]) + local[i] * d4 + c) : zero4();
+        v[i] = owner[i] >= 0 ? ldg_row4(static_cast<const float4*>(S.p[owner[i]]) + local[i] * d4 + c) : zero4();
 #pragma unroll
       for (int i = 0; i < R; ++i) {
         if (owner[i] >= 0 && last[i] > 0 && last[i] < cur) {   // warp-uniform: every lane holds the same owner / last
-          const float4 m = ld_peer4<0>(static_cast<const float4*>(S.m[owner[i]]) + local[i] * d4 + c);
-          const float4 vv = ld_peer4<0>(static_cast<const float4*>(S.v[owner[i]]) + local[i] * d4 + c);
+          const float4 m = ldg_row4(static_cast<const float4*>(S.m[owner[i]]) + local[i] * d4 + c);
+          const float4 vv = ldg_row4(static_cast<const float4*>(S.v[owner[i]]) + local[i] * d4 + c);
           const int64_t gap = cur - last[i];
           const float4 dl = catchup_series4(m, vv, last[i], static_cast<int>(gap < catchup_max ? gap : catchup_max), h, hist,
                                             hist_cap);
@@ -520,25 +504,11 @@ extern "C" int psb_peer_gather_rows(const void* const* shards, int32_t G, int64_
   if (n == 0) return PSB_OK;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (rows_total >= (1ll << 31)) return PSB_E_DIM;
-  static int mode = -1, rows_in_flight = -1;
-  if (mode < 0) {
-    const char* e = getenv("PSB_PEER_LD");
-    const int x = e != nullptr ? atoi(e) : 0;
-    mode = (x >= 0 && x <= 2) ? x : 0;
-    e = getenv("PSB_PEER_ROWS");
-    rows_in_flight = (e != nullptr && atoi(e) == 16) ? 16 : 8;
-  }
+  constexpr int R = 8;
   PSB_PROF("peer_gather_rows_kernel", s);
-#define PSB_PG_LAUNCH(R, M)                                                                                      \
-  peer_gather_rows_kernel<R, M><<<grid_for(n, 8 * R), 256, 0, s>>>(S, G, rows_total, static_cast<int>(d / 4), idx, n, \
-                                                                   reinterpret_cast<float4*>(out), remap_out, pad_id,  \
-                                                                   pad_pos, err_flag)
-  if (rows_in_flight == 16) {
-    if (mode == 0) PSB_PG_LAUNCH(16, 0); else if (mode == 1) PSB_PG_LAUNCH(16, 1); else PSB_PG_LAUNCH(16, 2);
-  } else {
-    if (mode == 0) PSB_PG_LAUNCH(8, 0); else if (mode == 1) PSB_PG_LAUNCH(8, 1); else PSB_PG_LAUNCH(8, 2);
-  }
-#undef PSB_PG_LAUNCH
+  peer_gather_rows_kernel<R><<<grid_for(n, 8 * R), 256, 0, s>>>(S, G, rows_total, static_cast<int>(d / 4), idx, n,
+                                                                reinterpret_cast<float4*>(out), remap_out, pad_id, pad_pos,
+                                                                err_flag);
   return launch_status();
 }
 
@@ -624,18 +594,11 @@ extern "C" int psb_peer_fold_lists(const psb_fold_table_t* tables, int32_t n_tab
     peer_fold_kernel<false><<<grid, 256, 0, s>>>(a);
     if ((st = launch_status()) != PSB_OK) return st;
   }
-  {   // entries per warp and iteration (~1 / G of them are folded here, one after the other): PSB_PEER_FOLD_E overrides
-    static int e_env = -1;
-    if (e_env < 0) {
-      const char* e = getenv("PSB_PEER_FOLD_E");
-      e_env = e != nullptr ? atoi(e) : 0;
-    }
-    // measured at N = 8 (profiles/r02C_bench_n8_E*.json): 32 entries 55 us / 0.502 ms per step, 16 entries 45 us /
-    // 0.484 ms, 8 entries 50 us / 0.489 ms -> about two leaders per warp and iteration
-    int e_auto = 2 * G < 32 ? 2 * G : 32;
-    if (e_auto < 8) e_auto = 8;
-    a.entries_per_warp = (e_env >= 2 && e_env <= 32) ? e_env : e_auto;
-  }
+  // entries per warp and iteration (~1 / G of them are folded here, one after the other), measured at N = 8
+  // (profiles/r02C_bench_n8_E*.json): 32 entries 55 us / 0.502 ms per step, 16 entries 45 us / 0.484 ms, 8 entries
+  // 50 us / 0.489 ms -> about two leaders per warp and iteration
+  a.entries_per_warp = 2 * G < 32 ? 2 * G : 32;
+  if (a.entries_per_warp < 8) a.entries_per_warp = 8;
   dim3 grid(grid_for(cap_max, 8 * a.entries_per_warp, 2), n_tables, G);
   PSB_PROF("peer_fold_sum_kernel", s);
   peer_fold_kernel<true><<<grid, 256, 0, s>>>(a);

@@ -10,8 +10,6 @@
 // The reduction kernel (one warp per destination row, 128-bit row loads, 4 source rows in
 // flight) is the HBM-bound part: algorithmic bytes = n_slots * d * 4 read (when sources
 // are materialised rows) + n_unique * d * 4 written + metadata; sort traffic is overhead.
-#include <stdlib.h>
-
 #include "psb_common.cuh"
 
 namespace psb {
@@ -422,7 +420,7 @@ radix_scan_kernel(int* __restrict__ hist, int nblocks, int* __restrict__ totals)
   if (threadIdx.x == 0) totals[blockIdx.x] = carry;
 }
 
-template <bool BALLOT, bool FIRST>
+template <bool FIRST>
 __global__ void __launch_bounds__(kNT, 3)
 radix_scatter_kernel(const uint32_t* __restrict__ keys_in, const uint32_t* __restrict__ vals_in, int64_t n,
                      int shift, int nblocks, const int* __restrict__ hist, const int* __restrict__ totals,
@@ -452,7 +450,7 @@ radix_scatter_kernel(const uint32_t* __restrict__ keys_in, const uint32_t* __res
     if (FIRST) val[r] = static_cast<uint32_t>(base + p);   // pass 0: the payload is the slot position
     else val[r] = valid[r] ? vals_in[base + p] : 0u;
   }
-  tile_rank<kNT, kIPT, BALLOT>(key, valid, shift, pos, whist, dstart, scan_sm);
+  tile_rank<kNT, kIPT, true>(key, valid, shift, pos, whist, dstart, scan_sm);
 #pragma unroll
   for (int r = 0; r < kIPT; ++r)
     if (valid[r]) {
@@ -913,17 +911,6 @@ static WorkspaceLayout layout_for(int64_t n_total, int64_t d = 512) {
 
 using namespace psb;
 
-// Tuning knob read once: PSB_RADIX_MATCH=match selects the MATCH.ANY ranking in the multi-CTA radix scatter
-// (default: ballot-based peer masks).
-static bool radix_use_ballot() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PSB_RADIX_MATCH");
-    v = (e != nullptr && e[0] == 'm') ? 0 : 1;
-  }
-  return v != 0;
-}
-
 extern "C" int64_t psb_scatter_reduce_workspace_bytes(int64_t n_total, int64_t table_rows) {
   (void)table_rows;
   if (n_total < 0) return PSB_E_ARG;
@@ -1026,7 +1013,6 @@ static int scatter_run(int phase, const psb_contrib_t* contribs, int32_t n_contr
   } else {
     const int nblocks = static_cast<int>((n_total + kTile - 1) / kTile);
     uint32_t *ki = keys_a, *vi = vals_a, *ko = keys_b, *vo = vals_b;
-    const bool ballot = radix_use_ballot();
     for (int pass = 0; pass < passes; ++pass) {
       PSB_PROF("radix_hist_kernel", s);
       if (pass == 0) radix_hist_kernel<true><<<nblocks, kNT, 0, s>>>(T, table_rows, drop_idx, ki, n_total, 0, nblocks, hist);
@@ -1036,11 +1022,8 @@ static int scatter_run(int phase, const psb_contrib_t* contribs, int32_t n_contr
       radix_scan_kernel<<<256, 256, 0, s>>>(hist, nblocks, totals);
       if ((st = launch_status()) != PSB_OK) return st;
       PSB_PROF("radix_scatter_kernel", s);
-#define PSB_RS_LAUNCH(B, F)                                                                                      \
-  radix_scatter_kernel<B, F><<<nblocks, kNT, 0, s>>>(ki, vi, n_total, pass * 8, nblocks, hist, totals, ko, vo)
-      if (pass == 0) { if (ballot) PSB_RS_LAUNCH(true, true); else PSB_RS_LAUNCH(false, true); }
-      else { if (ballot) PSB_RS_LAUNCH(true, false); else PSB_RS_LAUNCH(false, false); }
-#undef PSB_RS_LAUNCH
+      if (pass == 0) radix_scatter_kernel<true><<<nblocks, kNT, 0, s>>>(ki, vi, n_total, 0, nblocks, hist, totals, ko, vo);
+      else radix_scatter_kernel<false><<<nblocks, kNT, 0, s>>>(ki, vi, n_total, pass * 8, nblocks, hist, totals, ko, vo);
       if ((st = launch_status()) != PSB_OK) return st;
       uint32_t* t = ki; ki = ko; ko = t;
       t = vi; vi = vo; vo = t;

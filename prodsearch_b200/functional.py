@@ -42,12 +42,10 @@ class RowGradSink(object):
     """Gradient collector for one embedding table (and the bias vector indexed like it).
 
     The sort + segmented reduce of different tables are independent, and at batch 384 each is a chain of short,
-    narrow launches (one CTA of counting sort, then the reduce): with ``concurrent`` set, every dense-mode sink runs
-    its chain on its own side stream, forked from and joined back into the stream ``backward()`` ran on, so the
-    chains of the item and the word table overlap (inside a captured CUDA graph they become parallel branches)."""
+    narrow launches (one CTA of counting sort, then the reduce): every sink of a CUDA table runs its chain on its own
+    side stream, forked from and joined back into the stream ``backward()`` ran on, so the chains of the item and the
+    word table overlap (inside a captured CUDA graph they become parallel branches)."""
 
-    concurrent = True
-    presort = True                    # sort the step's index lists next to the backward pass (see expect())
     _forked = []                      # sinks whose chain is in flight on a side stream (not yet joined)
     _seq = 0                          # global order of expect() / mark_forward_end() calls
     _fwd_mark = {}                    # device -> (event recorded when a model's forward pass ended, its sequence number)
@@ -95,7 +93,7 @@ class RowGradSink(object):
         NEXT TO the backward kernels -- and finalize() is left with the segmented reduce.  If what backward delivers
         does not match what forward announced (a branch without gradient, a second forward), finalize() falls back to
         the one-call sort + reduce; the result is the same."""
-        if not (RowGradSink.presort and self.weight.is_cuda and self.weight.requires_grad):
+        if not (self.weight.is_cuda and self.weight.requires_grad):
             return
         if len(self._expected) >= 2 * ops._lib.MAX_CONTRIBS:
             return
@@ -162,7 +160,7 @@ class RowGradSink(object):
                 self._launch_presort()
 
     def _finalize_callback(self):
-        if not (RowGradSink.concurrent and self.weight.is_cuda):
+        if not self.weight.is_cuda:
             return self.finalize()
         run_forked(self)
 
@@ -574,7 +572,6 @@ class SeqEncoderFn(Function):
     # gradient yet and no earlier node of the same pass has gradients of the same weights in flight: AccumulateGrad
     # then merely adopts the new tensors -- an in-place accumulation would touch them on the calling stream too
     # early, so in that case whatever is in flight is joined first and this node runs on the calling stream.
-    overlap_wgrad = True
     _events = {}
     _pending = {}          # device -> [event, [(workspace, forward call, grad_out) kept alive], {id(weight) in flight}]
 
@@ -592,8 +589,7 @@ class SeqEncoderFn(Function):
         pend = SeqEncoderFn._pending.get(dev)
         ids = set(id(w) for w in ctx.weights)
         clash = pend is not None and not ids.isdisjoint(pend[2])
-        fork = (SeqEncoderFn.overlap_wgrad and not ctx.pre_ln and not clash and
-                all(w.grad is None for w in ctx.weights))
+        fork = not ctx.pre_ln and not clash and all(w.grad is None for w in ctx.weights)
         if clash or (pend is not None and not fork):
             SeqEncoderFn._join(dev)
             pend = None

@@ -20,9 +20,6 @@ from .transformer import TransformerEncoder
 
 
 class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
-    overlap_query_pooling = True     # query pooling on a side stream under the encoder's plan / transpose kernels
-    overlap_item_to_words = True     # item -> word loss kernels on a side stream next to the encoder
-    fused_loss_tail = True           # training under dropout: ranking loss on the encoder's output block in place
     # Item negatives (item_transformer.py:447: torch.multinomial(ones(P), B * K, replacement=True)).  "multinomial" is
     # that literal call -- bit-identical ids on the same device generator (tests/test_gpu_parity_r2.py).  Its cost is
     # O(P) per draw: ATen renormalises the distribution with ONE thread block and rebuilds the CDF every call --
@@ -131,7 +128,7 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         # the query pooling runs on a side stream; the encoder call enqueues its token plan and weight transposes
         # (which do not read the pooled queries) and waits for the event only before the kernel that does
         side = ready = None
-        if self.overlap_query_pooling and self.word_embeddings.weight.is_cuda:
+        if self.word_embeddings.weight.is_cuda:
             if getattr(self, "_q_stream", None) is None:
                 self._q_stream = torch.cuda.Stream(device=self.word_embeddings.weight.device)
                 self._q_ready = torch.cuda.Event()
@@ -199,7 +196,7 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         dev_t = self.product_emb.weight
         cur = torch.cuda.current_stream(dev_t.device) if dev_t.is_cuda else None
         side = None
-        if cur is not None and self.overlap_item_to_words:
+        if cur is not None:
             if getattr(self, "_iw_stream", None) is None:
                 self._iw_stream = torch.cuda.Stream(device=dev_t.device)
             side = self._iw_stream
@@ -237,7 +234,7 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
             # dropout makes the positive and the K negative encodes differ (transformer.py:56, neural.py:226):
             # 1 + K dropout draws of the SAME sequence, K/V projections shared between them
             out = self.encode_queries(query_word_idxs, u_item_idxs, copies=1 + K, hist=hist).view(B, 1 + K, -1)
-            if self.fused_loss_tail and K <= 7 and self.embedding_size <= 128 and out.is_cuda:
+            if K <= 7 and self.embedding_size <= 128 and out.is_cuda:
                 # ranking loss on the encoder's output block in place + loss combination and running sums: two launches
                 if side is not None:
                     cur.wait_stream(side)        # sampled item negatives and the item -> word losses are ready
@@ -534,7 +531,7 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
                                                        pad_idx=item_pad, use_pos=self.args.use_pos_emb,
                                                        out_pos=out_pos, copies=copies, first_ready=self._q_ready)
         pos_weight = float(K) if self.args.pos_weight else 1.0
-        if stochastic and self.fused_loss_tail and K <= 7 and self.embedding_size <= 128:
+        if stochastic and K <= 7 and self.embedding_size <= 128:
             # ranking loss on the encoder's output block in place + loss combination: two launches (see the base class)
             cur.wait_stream(self._iw_stream)
             if self._ps_acc is None:
@@ -573,10 +570,8 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
     # distributions are constant: the draws for step t + 1 are made on a side stream DURING step t (fetch + encoder take
     # longer) into a second pair of buffers and copied into the live pair at the start of step t + 1.  Same generator,
     # same draw order (items, words, items, words, ...); each draw is merely issued one step early.
-    prefetch_negatives = True
-
     def _negatives_for_step(self, B, W, K):
-        if self.injected_negatives is not None or not self.prefetch_negatives or not self.training:
+        if self.injected_negatives is not None or not self.training:
             self._neg_fork = None
             ni, nw = self._draw_negatives(B, W, K)
             return ni, nw
@@ -625,15 +620,14 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
                 it.lazy_optim = opt
         self.sync_stage()
         self.peer.barrier(1)       # every rank's compact lists and dense bucket are complete
+        # real multi-process groups: shard norm, barrier and global norm in one tail launch (psb_peer_norm_exchange)
         fused = (optim is not None and hasattr(getattr(optim, "optimizer", optim), "global_norm_slots")
-                 and self.peer.world > 1 and self.peer._sim is None and self.fused_norm_exchange)
+                 and self.peer.world > 1 and self.peer._sim is None)
         self.sync_fold(norm_exchange=optim if fused else None)
         if fused or optim is None or not hasattr(getattr(optim, "optimizer", optim), "set_global_sqnorm"):
             return
         self.peer.barrier(2)       # every rank's shard norm is published
         self.sync_norm(optim)
-
-    fused_norm_exchange = True     # shard norm, barrier and global norm in one tail launch (psb_peer_norm_exchange)
 
     def sync_stage(self):
         self._bucket.stage()

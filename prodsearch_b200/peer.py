@@ -374,7 +374,7 @@ class PeerGradSink(object):
     # ---- sort next to the backward pass (the same scheme as functional.RowGradSink.expect) ----------------------
     def expect(self, idx):
         from . import functional as F_
-        if not (F_.RowGradSink.presort and self.weight.requires_grad) or self._expected is None:
+        if not self.weight.requires_grad or self._expected is None:
             return
         g = self._origin.get(idx.data_ptr())
         if g is None or g.numel() != idx.numel() or len(self._expected) >= _lib.MAX_CONTRIBS:
@@ -416,10 +416,7 @@ class PeerGradSink(object):
 
     def _finalize_callback(self):
         from . import functional as F_
-        if F_.RowGradSink.concurrent:
-            F_.run_forked(self)       # the item and the word table's sort + reduce chains overlap
-        else:
-            self.finalize()
+        F_.run_forked(self)           # the item and the word table's sort + reduce chains overlap
 
     def begin(self, ids, origin):
         self._ids, self._origin = ids, origin

@@ -4,15 +4,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 from test_gpu_sparse_adam import _tem, _cuda
 from prodsearch_b200 import synth, _lib
-from prodsearch_b200 import functional as F_
 from prodsearch_b200.graph_step import GraphedTrainStep
-from prodsearch_b200.item_transformer import ItemTransformerRanker
 from prodsearch_b200.optimizers import Optimizer
 mode = sys.argv[1] if len(sys.argv) > 1 else "default"
-if "noconc" in mode: F_.RowGradSink.concurrent = False
-if "nooverlap" in mode:
-    ItemTransformerRanker.overlap_query_pooling = False
-    ItemTransformerRanker.overlap_item_to_words = False
 a, b = _tem("rowsparse"), _tem("rowsparse")
 b.load_state_dict(a.state_dict())
 oa, ob = Optimizer("adam", 5e-3, 5.0), Optimizer("adam", 5e-3, 5.0)

@@ -5,8 +5,7 @@
 Brackets psb_peer_gather_rows (random rows of a row-sharded 16M x 128 table, 1M rows per rank) with what the same
 box does for the same bytes: (a) cudaMemcpyAsync from the peer mapping (copy engine), (b) NCCL all_to_all_single,
 (c) the gather kernel on SEQUENTIAL remote rows (pure P2P load stream), (d) on random rows, local rows only / remote
-rows only / the mix.  PSB_PEER_LD / PSB_PEER_ROWS select the load instruction and the rows in flight per warp (read once
-per process: the driver script runs this file once per setting)."""
+rows only / the mix."""
 import ctypes
 import json
 import os
@@ -51,7 +50,7 @@ def main():
     dist.barrier()
     out = torch.empty(n, d, device="cuda")
     g = torch.Generator(device="cuda").manual_seed(1 + rank)
-    res = {"world": world, "ld": os.environ.get("PSB_PEER_LD", "0"), "rows_in_flight": os.environ.get("PSB_PEER_ROWS", "8")}
+    res = {"world": world}
     nxt = (rank + 1) % world
 
     def gather(ids):

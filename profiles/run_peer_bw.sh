@@ -2,9 +2,6 @@
 # gpurun --gpus 2 --timeout 600 -- 'bash profiles/run_peer_bw.sh r02j 2'
 R=${1:-r02j}; N=${2:-2}
 mkdir -p gpurun_out
-for cfg in "0 8" "1 8" "2 8" "1 16"; do
-  set -- $cfg
-  PSB_PEER_LD=$1 PSB_PEER_ROWS=$2 timeout 200 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 \
+timeout 200 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 \
       --master-port 29511 profiles/peer_bw.py 2>/dev/null | grep '^{' >> gpurun_out/${R}_peer_bw_n$N.jsonl
-done
 cat gpurun_out/${R}_peer_bw_n$N.jsonl

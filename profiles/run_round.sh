@@ -1,12 +1,11 @@
 #!/bin/bash
-# One gpurun call: GPU parity tests, variant A/B timings, the default bench line, and ncu captures of the
+# One run: GPU parity tests, the default bench line, and ncu captures of the
 # bandwidth-regime kernels.
 #   gpurun --timeout 1500 -- 'bash profiles/run_round.sh r01f'
 R=${1:-r01f}
 mkdir -p gpurun_out
 timeout 900 python -m pytest tests -m gpu -q > gpurun_out/${R}_pytest.log 2>&1; echo "pytest exit $?" >> gpurun_out/${R}_pytest.log
 tail -5 gpurun_out/${R}_pytest.log
-timeout 400 python profiles/ab_variants.py > gpurun_out/${R}_ab.jsonl 2>&1; cat gpurun_out/${R}_ab.jsonl
 timeout 600 python bench.py > gpurun_out/${R}_bench.json 2> gpurun_out/${R}_bench.err; echo "bench exit $?"
 tail -c 400 gpurun_out/${R}_bench.err
 timeout 300 ncu --set full --clock-control none --import-source on \

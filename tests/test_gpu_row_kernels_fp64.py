@@ -24,9 +24,6 @@ The mean-pool is checked bit for bit instead.  The kernel adds each scaled row, 
 order reproduces it exactly.
 """
 import math
-import os
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -35,8 +32,6 @@ import oracle
 
 pytestmark = pytest.mark.gpu
 
-THIS_FILE = os.path.abspath(__file__)
-ROOT = os.path.dirname(os.path.dirname(THIS_FILE))
 U = 2.0 ** -24                      # unit roundoff of float32
 RATIOS = {}                         # group -> worst err / bound seen in this run
 
@@ -209,15 +204,40 @@ def _dev(t):
 K_NS = dict(loss=4.0, coef=6.0, ga=6.0, gb=4.0)
 
 
-def _run_ns(ops, group, label, case, n, w, k, d, V=1000):
+def _ns_loss_at_rows(inp, table_rows):
+    """psb_ns_loss_fwd with table_rows passed in place of the table's row count."""
+    from prodsearch_b200 import _lib
+    a, b, table, bias, pos, neg, mask, nw = (_dev(inp[x]) for x in ("anchor_a", "anchor_b", "table", "bias", "pos", "neg",
+                                                                    "mask", "neg_weight"))
+    n, w = pos.shape
+    k, d = neg.shape[-1], table.shape[1]
+    f = dict(dtype=torch.float32, device="cuda")
+    loss, cp, cn, ga = torch.empty(n, **f), torch.empty(n, w, **f), torch.empty(n, w, k, **f), torch.empty(n, d, **f)
+    gb = torch.empty(n * k, d, **f) if b is not None else None
+    P = _lib.ptr
+    _lib.check(_lib.load().psb_ns_loss_fwd(P(a), P(b), P(table), table_rows, d, P(bias), P(pos), P(neg), P(mask),
+                                           inp["pad_idx"], P(nw), inp["pos_weight"], n, w, k, P(loss), P(cp), P(cn),
+                                           P(ga), P(gb), _lib.stream_ptr()), "psb_ns_loss_fwd")
+    return loss, cp, cn, ga, gb
+
+
+def _run_ns(ops, group, label, case, n, w, k, d, V=1000, table_rows=None):
+    """table_rows: passed to the library in place of V.  Ids >= V then become table_rows + 3, so every id is either a
+    real row or out of range for the kernel as well: the kernel reads only rows whose id is in [0, table_rows)."""
     use_mask, use_bias, use_nw, pw, with_b = case
     inp = _ns_inputs(n * 131 + w * 17 + k * 5 + d, n, w, k, d, V, use_mask, use_bias, use_nw, pw, with_b)
+    if table_rows is not None:
+        for t in (inp["pos"], inp["neg"]):
+            t[t >= V] = table_rows + 3
     ref = _ns_ref(**inp)
     with _Kernels() as kern:
-        loss, cp, cn, ga, gb = ops.ns_loss(_dev(inp["anchor_a"]), _dev(inp["table"]), _dev(inp["pos"]),
-                                           _dev(inp["neg"]), anchor_b=_dev(inp["anchor_b"]), bias=_dev(inp["bias"]),
-                                           mask=_dev(inp["mask"]), pad_idx=inp["pad_idx"],
-                                           neg_weight=_dev(inp["neg_weight"]), pos_weight=pw)
+        if table_rows is not None:
+            loss, cp, cn, ga, gb = _ns_loss_at_rows(inp, table_rows)
+        else:
+            loss, cp, cn, ga, gb = ops.ns_loss(_dev(inp["anchor_a"]), _dev(inp["table"]), _dev(inp["pos"]),
+                                               _dev(inp["neg"]), anchor_b=_dev(inp["anchor_b"]), bias=_dev(inp["bias"]),
+                                               mask=_dev(inp["mask"]), pad_idx=inp["pad_idx"],
+                                               neg_weight=_dev(inp["neg_weight"]), pos_weight=pw)
     assert label in kern.names, (label, kern.names)
     _check(group + "/loss", loss, ref["loss"], ref["m_loss"], K_NS["loss"])
     _check(group + "/coef_pos", cp, ref["coef"][..., 0], ref["m_coef"][..., 0], K_NS["coef"])
@@ -241,13 +261,6 @@ def _fid(f):
                          "_pw" if f[3] != 1.0 else "")
 
 
-def _w1_variant():
-    """PSB_NS_W1 as the library reads it (once per process): 0 sends w == 1 to ns_loss_fast_kernel, 1 (default) to
-    ns_loss_w1_kernel, 2 to its double-buffered form when there is no anchor_b."""
-    e = os.environ.get("PSB_NS_W1", "")
-    return int(e[0]) if e[:1] in ("0", "1", "2") else 1
-
-
 def _w1_cases():
     out, i = [], 0
     for with_b in (False, True):
@@ -267,9 +280,7 @@ def _w1_cases():
 
 @pytest.mark.parametrize("case,k,d,n", _w1_cases())
 def test_ns_loss_w1_kernel(ops, case, k, d, n):
-    v = _w1_variant()
-    group = ("ns_w1_as_fast", "ns_w1", "ns_w1_db")[v]
-    _run_ns(ops, group, "ns_loss_fast_kernel" if v == 0 else "ns_loss_w1_kernel", case, n, 1, k, d)
+    _run_ns(ops, "ns_w1", "ns_loss_w1_kernel", case, n, 1, k, d)
 
 
 def _fast_cases():
@@ -287,6 +298,25 @@ def _fast_cases():
 @pytest.mark.parametrize("case,w,k,d,n", _fast_cases())
 def test_ns_loss_fast_kernel(ops, case, w, k, d, n):
     _run_ns(ops, "ns_fast", "ns_loss_fast_kernel", case, n, w, k, d)
+
+
+def _fast_w1_cases():
+    out, i = [], 3
+    for with_b in (False, True):
+        for k in (1, 5, 7):
+            for d in (64, 128):
+                f = _features(i, 1, k)
+                out.append(pytest.param(f + (with_b,), k, d, id="fast_kernel<%s>-w1-k%d-d%d-rows2^31-%s" % (
+                    "B" if with_b else "noB", k, d, _fid(f))))
+                i += 1
+    return out
+
+
+@pytest.mark.parametrize("case,k,d", _fast_w1_cases())
+def test_ns_loss_fast_kernel_w1_large_table(ops, case, k, d):
+    """w == 1 on a table of 2^31 rows or more: ns_loss_w1_kernel carries row ids as int32, so the fast kernel takes
+    these calls (the only way to reach ns_loss_fast_kernel<true>).  The small real table stands in for the large one."""
+    _run_ns(ops, "ns_fast_w1", "ns_loss_fast_kernel", case, 67, 1, k, d, table_rows=2 ** 31)
 
 
 def _generic_cases():
@@ -310,21 +340,6 @@ def _generic_cases():
 @pytest.mark.parametrize("case,w,k,d,n", _generic_cases())
 def test_ns_loss_generic_kernel(ops, case, w, k, d, n):
     _run_ns(ops, "ns_generic", "ns_loss_kernel", case, n, w, k, d)
-
-
-@pytest.mark.parametrize("variant", ["0", "2"])
-def test_ns_loss_w1_cases_under_psb_ns_w1(variant):
-    """PSB_NS_W1 is read once per process: the w == 1 cases run again in a subprocess per variant (0: the fast
-    kernel, ns_loss_fast_kernel<true / false>; 2: the double-buffered ns_loss_w1_kernel<false, NR, true>)."""
-    if "PSB_NS_W1" in os.environ:
-        pytest.skip("already running under a PSB_NS_W1 variant")
-    env = dict(os.environ, PSB_NS_W1=variant)
-    r = subprocess.run([sys.executable, "-m", "pytest", THIS_FILE, "-q", "-s", "-m", "gpu", "-p",
-                        "no:cacheprovider", "-k", "test_ns_loss_w1_kernel"], cwd=ROOT, env=env, capture_output=True,
-                       text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-4000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout and " failed" not in r.stdout, r.stdout[-2000:]
-    sys.stdout.write(r.stdout[r.stdout.rfind("worst err / bound"):] if "worst err / bound" in r.stdout else "")
 
 
 # ------------------------------------------------------------------------------------------------ tem_loss
@@ -363,7 +378,7 @@ K_TEM = dict(loss=4.0, coef=6.0, grad=4.0)
 @pytest.mark.parametrize("d", [32, 128])
 @pytest.mark.parametrize("k", [1, 5, 6, 7])
 def test_tem_loss_vs_fp64_tail(ops, k, d, with_bias, pos_weight, grad_scale):
-    """ns_loss_w1_kernel<true, 6, false> for k <= 5, <true, 8, false> for k = 6, 7, on the [n, 1 + k, d] block."""
+    """ns_loss_w1_kernel<true, 6> for k <= 5, <true, 8> for k = 6, 7, on the [n, 1 + k, d] block."""
     g = torch.Generator().manual_seed(k * 100 + d + int(with_bias))
     P, n = 3000, 77
     table = torch.randn(P, d, generator=g)

@@ -6,7 +6,8 @@ reference's embedding_dense_backward, SURVEY.md 0.6).  Each op *registers a cont
 (indices + source rows + per-slot scales) with the table's ``RowGradSink``; when the backward
 pass finishes, one deterministic sort + segmented-reduce per table (psb_scatter_reduce_rows)
 produces the gradient, either scattered into a persistent dense ``.grad`` (drop-in for the
-reference's dense Adam) or kept row-sparse as ``param.row_grad = (rows, values, n_rows)``.
+reference's dense Adam), kept row-sparse as ``param.row_grad = (rows, values, n_rows)``, or written into the
+caller-owned staging list a peer-sharded table's owners fold (peer.py).
 """
 import torch
 from torch.autograd import Function, Variable
@@ -41,6 +42,11 @@ def run_forked(sink):
 class RowGradSink(object):
     """Gradient collector for one embedding table (and the bias vector indexed like it).
 
+    ``rows``: the id space the sort runs over (and ``drop_idx`` is in), ``weight.shape[0]`` unless the table holds a
+    share of the rows (peer-sharded: global ids).  ``mode``: the reduced rows go into a persistent ``weight.grad``
+    ("dense"), ``weight.row_grad`` ("rowsparse") or the owner's staging list ``stage = (rows int32 [cap], count int32
+    [1], values fp32 [cap, d])``, set before the first step ("stage"; the bias gradient is a dense vector).
+
     The sort + segmented reduce of different tables are independent, and at batch 384 each is a chain of short,
     narrow launches (one CTA of counting sort, then the reduce): every sink of a CUDA table runs its chain on its own
     side stream, forked from and joined back into the stream ``backward()`` ran on, so the chains of the item and the
@@ -63,11 +69,15 @@ class RowGradSink(object):
         RowGradSink._seq += 1
         RowGradSink._fwd_mark[dev] = (ev, RowGradSink._seq)
 
-    def __init__(self, weight, drop_idx=-1, bias=None, mode="dense"):
+    def __init__(self, weight, drop_idx=-1, bias=None, mode="dense", rows=None):
         self.weight = weight
         self.bias = bias
         self.drop_idx = drop_idx
-        self.mode = mode              # "dense" | "rowsparse"
+        self.mode = mode              # "dense" | "rowsparse" | "stage"
+        self.rows = weight.shape[0] if rows is None else int(rows)
+        self.stage = None
+        self.ids = None               # begin(): the row id of every position of the fetched mini table
+        self._origin = None
         self._pending = []
         self._queued = False
         self._dense = None
@@ -85,6 +95,16 @@ class RowGradSink(object):
         self._sort_bufs = None
         self._last_seq = 0
 
+    def begin(self, ids, origin):
+        """A fetch handed out a mini table: contributions now index its positions, and position p is row ``ids[p]``.
+        ``origin`` maps each index tensor the fetch returned (by data pointer) to the row ids it was remapped from."""
+        self.ids, self._origin = ids, origin
+        self._expected = []
+
+    def _origin_of(self, idx):
+        g = self._origin.get(idx.data_ptr())
+        return g if g is not None and g.numel() == idx.numel() else None
+
     # -- called from Function.forward ---------------------------------------------------
     def expect(self, idx):
         """Announce an index list that backward will contribute with.  The sort of a step's contributions only needs
@@ -92,13 +112,20 @@ class RowGradSink(object):
         pass the sink sorts the announced lists on its own stream -- ordered behind the forward pass only, so it runs
         NEXT TO the backward kernels -- and finalize() is left with the segmented reduce.  If what backward delivers
         does not match what forward announced (a branch without gradient, a second forward), finalize() falls back to
-        the one-call sort + reduce; the result is the same."""
-        if not (self.weight.is_cuda and self.weight.requires_grad):
+        the one-call sort + reduce; the result is the same.  So does a step with more lists than one sort takes, or
+        with an index list the fetch (begin) did not hand out."""
+        if not (self.weight.is_cuda and self.weight.requires_grad) or self._expected is None:
             return
-        if len(self._expected) >= 2 * ops._lib.MAX_CONTRIBS:
-            return
+        if self._origin is not None:
+            idx = self._origin_of(idx)
+            if idx is None:
+                self._expected = None
+                return
         t = ops._idx(idx).reshape(-1)
         if t.numel() == 0:
+            return
+        if len(self._expected) >= ops._lib.MAX_CONTRIBS:
+            self._expected = None
             return
         self._expected.append(t)
         RowGradSink._seq += 1
@@ -106,23 +133,27 @@ class RowGradSink(object):
 
     def _launch_presort(self):
         exp, w = self._expected, self.weight
-        if not exp or len(exp) > ops._lib.MAX_CONTRIBS:
-            return
         if self.mode == "dense" and w.grad is not None and w.grad is self._dense:
             return                                   # gradient accumulation: finalize() takes its own path
         dev = w.device
         n_total = sum(t.numel() for t in exp)
+        if self.mode == "stage" and (self.stage is None or n_total > self.stage[0].numel()):
+            return                                   # finalize() raises
         if self._sort_stream is None:
             self._sort_stream = torch.cuda.Stream(device=dev)
             self._sort_done = torch.cuda.Event()
         bufs = self._sort_bufs
-        wb = ops.scatter_workspace_bytes(n_total, w.shape[0])
+        wb = ops.scatter_workspace_bytes(n_total, self.rows)
         if bufs is None or bufs[0].numel() < wb or bufs[1].numel() < n_total:
             if self._prev is not None and self._prev != "all" and bufs is not None and self._prev[0] is bufs[1]:
                 self._prev = "all"               # the old row list goes away with its buffer: next clear is a memset
-            bufs = self._sort_bufs = (torch.empty(wb, dtype=torch.uint8, device=dev),
-                                      torch.empty(max(n_total, 1), dtype=torch.int32, device=dev),
-                                      torch.zeros(1, dtype=torch.int32, device=dev))
+            ws = torch.empty(wb, dtype=torch.uint8, device=dev)
+            if self.mode == "stage":             # the sort writes the staging list's rows and count (sized once)
+                bufs = (ws,) + tuple(self.stage[:2])
+            else:
+                bufs = (ws, torch.empty(max(n_total, 1), dtype=torch.int32, device=dev),
+                        torch.zeros(1, dtype=torch.int32, device=dev))
+            self._sort_bufs = bufs
         ws, uniq, nu = bufs
         st = self._sort_stream
         # behind the end of the forward pass when the model marked it after this sink's last announcement, else
@@ -143,7 +174,7 @@ class RowGradSink(object):
                 self._prepare_dense(self.bias is not None and self._dense_bias is not None, clear=True)
                 cleared = True
             nu.zero_()
-            ops.scatter_sort(exp, w.shape[0], self.drop_idx, ws, uniq, nu)
+            ops.scatter_sort(exp, self.rows, self.drop_idx, ws, uniq, nu)
             self._sort_done.record(st)
         self._presort = dict(exp=exp, ws=ws, uniq=uniq, nu=nu, cleared=cleared)
 
@@ -151,6 +182,9 @@ class RowGradSink(object):
     def add(self, idx, src, src_row=None, src_div=1, scale=None, scale2=None, scale2_div=1, to_bias=False):
         if not self.weight.requires_grad and not (to_bias and self.bias is not None and self.bias.requires_grad):
             return
+        if self._origin is not None:
+            g = self._origin_of(idx)
+            idx = g if g is not None else self.ids[idx.reshape(-1)]
         self._pending.append(ops.make_contrib(idx, src, src_row, src_div, scale, scale2, scale2_div,
                                               to_bias and self.bias is not None))
         if not self._queued:
@@ -181,8 +215,10 @@ class RowGradSink(object):
         if not pending:
             return
         w = self.weight
-        rows, d = w.shape
+        rows, d = self.rows, w.shape[1]
         want_bias = self.bias is not None and any(c.to_bias for c, _ in pending)
+        if self.mode == "stage":
+            self._prepare_stage(pending, want_bias)
         if ps is not None and self._finalize_presorted(ps, pending, rows, d, want_bias):
             return
         if ps is not None and ps["cleared"]:
@@ -214,6 +250,10 @@ class RowGradSink(object):
                 self._attach(w, self._dense)
                 if want_bias:
                     self._attach(self.bias, self._dense_bias)
+            elif self.mode == "stage":
+                ops.scatter_reduce(chunk, rows, d, self.drop_idx, dense_bias_grad=self._dense_bias if want_bias else None,
+                                   want_rows=True, device=w.device, out_uniq=self.stage[0], out_nu=self.stage[1],
+                                   out_red=self.stage[2])
             else:
                 uniq, red, redb, nu = ops.scatter_reduce(chunk, rows, d, self.drop_idx, want_rows=True,
                                                          want_bias=want_bias, device=w.device)
@@ -254,6 +294,10 @@ class RowGradSink(object):
             self._attach(w, self._dense)
             if want_bias:
                 self._attach(self.bias, self._dense_bias)
+        elif self.mode == "stage":
+            ops.scatter_reduce_sorted(ordered, rows, d, self.drop_idx, ps["ws"], ps["uniq"], ps["nu"],
+                                      dense_bias_grad=self._dense_bias if want_bias else None, want_rows=True,
+                                      out_red=self.stage[2])
         else:
             red, redb = ops.scatter_reduce_sorted(ordered, rows, d, self.drop_idx, ps["ws"], ps["uniq"], ps["nu"],
                                                   want_rows=True, want_bias=want_bias)
@@ -307,6 +351,19 @@ class RowGradSink(object):
             else:
                 ops.zero_rows(uniq, nu, w.shape[1], self._dense, self._dense_bias)
             self._prev = None
+
+    def _prepare_stage(self, pending, want_bias):
+        if len(pending) > ops._lib.MAX_CONTRIBS:
+            raise RuntimeError("more than %d contributions to one table in a step" % ops._lib.MAX_CONTRIBS)
+        n_total, cap = sum(int(c.n) for c, _ in pending), self.stage[0].numel() if self.stage is not None else 0
+        if n_total > cap:
+            raise RuntimeError("gradient staging list too small (%d slots, %d needed): call reserve_stage with the "
+                               "largest step first" % (cap, n_total))
+        if want_bias:
+            if self._dense_bias is None:
+                self._dense_bias = torch.empty_like(self.bias)
+            self._dense_bias.zero_()
+            self.bias.grad = self._dense_bias     # replaced: this mode has no gradient accumulation
 
     @staticmethod
     def _attach(param, buf):
@@ -387,9 +444,10 @@ class MeanPoolFn(Function):
     @staticmethod
     def forward(ctx, weight, idx, fs_weight, fs_bias, sink, pad_idx, mask, tok_scale, keep_scale, stream=None):
         # validity by pad id with the pad row dropped by the sink anyway: the backward weights valid / count reduce to
-        # 1 / count per pool, which the forward kernel hands out for free (no token-weights launch in backward)
-        ctx.by_count = (mask is None and pad_idx >= 0 and sink is not None and
-                        getattr(sink, "drop_idx", None) == pad_idx and ctx.needs_input_grad[0])
+        # 1 / count per pool, which the forward kernel hands out for free (no token-weights launch in backward).  A sink
+        # that translates mini-table positions (begin) drops a row id, which pad_idx is not.
+        ctx.by_count = (mask is None and pad_idx >= 0 and sink is not None and sink.ids is None and
+                        sink.drop_idx == pad_idx and ctx.needs_input_grad[0])
         out, mean, inv = ops.gather_meanpool(weight, idx, pad_idx=pad_idx, mask=mask, tok_scale=tok_scale,
                                              keep_scale=keep_scale, fs_weight=fs_weight, fs_bias=fs_bias,
                                              want_inv_count=ctx.by_count, stream=stream)

@@ -517,7 +517,7 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
         wb = self.word_bias
         bias_mini = None
         if wb is not None:     # bias values at the mini positions (the bias vector itself is replicated)
-            bias_mini = _BiasAtFn.apply(wb, self.word_table.sink._ids)
+            bias_mini = _BiasAtFn.apply(wb, self.word_table.sink.ids)
         cur.wait_stream(self._fetch_stream)      # join: the item rows are needed by both branches below
         # the item -> word objective shares nothing with the encoder: a parallel branch, joined before the sum
         self._iw_stream.wait_stream(cur)

@@ -8,8 +8,8 @@ other rank.  From then on the exchange steps are loads inside hand-written kerne
 
   fetch   ``PeerShardedTable.fetch``: out[i] = shard[id % G][id / G]  (psb_peer_gather_rows) into a small
           local *mini table*; the unchanged single-GPU fused kernels then run on it with remapped indices
-  push    the table's ``PeerGradSink`` runs the usual deterministic sort + segmented reduce over GLOBAL row
-          ids into a peer-visible compact list (rows, values, count)
+  push    the table's sink (a ``functional.RowGradSink`` in "stage" mode) runs the usual deterministic sort +
+          segmented reduce over GLOBAL row ids into a peer-visible compact list (rows, values, count)
   fold    after a barrier every owner folds the slots it owns of each peer's list, peer by peer in rank order,
           into its dense shard gradient (psb_peer_fold_lists: two launches whatever G is): reproducible, no
           float atomics, no second sort
@@ -24,6 +24,7 @@ import ctypes
 import torch
 
 from . import _lib
+from . import functional as F_
 from ._lib import c_vp, check, load, stream_ptr
 
 
@@ -225,13 +226,14 @@ class PeerShardedTable(object):
         self.weight = torch.nn.Parameter(w)
         self.grad = torch.zeros_like(w)                    # dense shard gradient (what Adam reads)
         self.bias = bias                                   # replicated bias vector indexed like the table
-        self.bias_grad = torch.zeros_like(bias) if bias is not None else None
+        # contributions arrive as mini-table positions (fetch hands the sink their global ids); the reduced rows go
+        # into the staging list the owners fold
+        self.sink = F_.RowGradSink(self.weight, self.pad_idx, bias, "stage", rows=self.rows)
         self._stage = None
         self._cap = 0
         self._posmap = None
         if stage_cap:
             self._ensure_stage(stage_cap)
-        self.sink = PeerGradSink(self)
 
     # staging layout (peer-visible): [n_rows int32 | pad to 256][rows int32 cap][vals fp32 cap x d]
     def _ensure_stage(self, cap):
@@ -245,6 +247,7 @@ class PeerShardedTable(object):
         self.stage_n = self._stage.view(torch.int32, (1,), 0)
         self.stage_rows = self._stage.view(torch.int32, (cap,), self._off_rows)
         self.stage_vals = self._stage.view(torch.float32, (cap, self.d), self._off_vals)
+        self.sink.stage = (self.stage_rows, self.stage_n, self.stage_vals)
 
     def reserve_stage(self, cap):
         """Size the peer-visible gradient list for ``cap`` contribution slots per step.  Collective (and
@@ -348,132 +351,6 @@ def fold_tables(tables, scale):
             t.weight._psb_drop_idx = t.pad_idx // peer.world if t.pad_idx % peer.world == peer.rank else -1
         else:
             t.weight.grad = t.grad
-
-
-class PeerGradSink(object):
-    """RowGradSink counterpart of a peer-sharded table: contributions arrive with mini-table positions, are
-    translated back to GLOBAL row ids, and one sort + segmented reduce writes the compact list the owners fold."""
-
-    def __init__(self, table):
-        self.table = table
-        self._pending = []
-        self._queued = False
-        self._ids = None
-        self._origin = {}
-        self.weight = table.weight
-        self._stream = None
-        self._hold = None
-        self._expected = []           # GLOBAL-id tensors the forward pass announced (see RowGradSink.expect)
-        self._last_seq = 0
-        self._presort = None
-        self._sort_stream = None
-        self._sort_done = None
-        self._sort_ws = None
-        self._exp_event = None
-
-    # ---- sort next to the backward pass (the same scheme as functional.RowGradSink.expect) ----------------------
-    def expect(self, idx):
-        from . import functional as F_
-        if not self.weight.requires_grad or self._expected is None:
-            return
-        g = self._origin.get(idx.data_ptr())
-        if g is None or g.numel() != idx.numel() or len(self._expected) >= _lib.MAX_CONTRIBS:
-            self._expected = None         # an index list the fetch did not hand out: this step sorts in finalize()
-            return
-        self._expected.append(g.reshape(-1))
-        F_.RowGradSink._seq += 1
-        self._last_seq = F_.RowGradSink._seq
-
-    def _launch_presort(self):
-        from . import functional as F_
-        from . import ops
-        exp, t = self._expected, self.table
-        if not exp:
-            return
-        n_total = sum(x.numel() for x in exp)
-        if n_total > t._cap:
-            return
-        dev = self.weight.device
-        if self._sort_stream is None:
-            self._sort_stream = torch.cuda.Stream(device=dev)
-            self._sort_done = torch.cuda.Event()
-            self._exp_event = torch.cuda.Event()
-        wb = ops.scatter_workspace_bytes(n_total, t.rows)
-        if self._sort_ws is None or self._sort_ws.numel() < wb:
-            self._sort_ws = torch.empty(wb, dtype=torch.uint8, device=dev)
-        st = self._sort_stream
-        mark = F_.RowGradSink._fwd_mark.get(dev)
-        if mark is not None and mark[1] >= self._last_seq:
-            st.wait_event(mark[0])
-        else:
-            self._exp_event.record(torch.cuda.current_stream(dev))
-            st.wait_event(self._exp_event)
-        with torch.cuda.stream(st):
-            t.stage_n.zero_()
-            ops.scatter_sort(exp, t.rows, t.pad_idx, self._sort_ws, t.stage_rows, t.stage_n)
-            self._sort_done.record(st)
-        self._presort = dict(exp=exp, ws=self._sort_ws)
-
-    def _finalize_callback(self):
-        from . import functional as F_
-        F_.run_forked(self)           # the item and the word table's sort + reduce chains overlap
-
-    def begin(self, ids, origin):
-        self._ids, self._origin = ids, origin
-        self._expected = []
-
-    def add(self, idx, src, src_row=None, src_div=1, scale=None, scale2=None, scale2_div=1, to_bias=False):
-        from . import ops
-        from torch.autograd import Variable
-        g = self._origin.get(idx.data_ptr())
-        if g is None or g.numel() != idx.numel():
-            g = self._ids[idx.reshape(-1)]
-        self._pending.append(ops.make_contrib(g, src, src_row, src_div, scale, scale2, scale2_div,
-                                              to_bias and self.table.bias is not None))
-        if not self._queued:
-            self._queued = True
-            Variable._execution_engine.queue_callback(self._finalize_callback)
-            if self._expected and self._presort is None:
-                self._launch_presort()
-
-    def finalize(self):
-        from . import ops
-        self._queued = False
-        pending, self._pending = self._pending, []
-        ps, self._presort, self._expected = self._presort, None, []
-        if ps is not None:            # join the sort stream whatever happens next
-            torch.cuda.current_stream(self.weight.device).wait_event(self._sort_done)
-        if not pending:
-            return
-        t = self.table
-        if len(pending) > _lib.MAX_CONTRIBS:
-            raise RuntimeError("more than %d contributions to one table in a step" % _lib.MAX_CONTRIBS)
-        n_total = sum(int(c.n) for c, _ in pending)
-        if n_total > t._cap:
-            raise RuntimeError("gradient staging list too small (%d slots, %d needed): call reserve_stage with the "
-                               "largest step first" % (t._cap, n_total))
-        want_bias = t.bias is not None and any(c.to_bias for c, _ in pending)
-        if want_bias:
-            t.bias_grad.zero_()
-        ordered = None
-        if ps is not None and len(pending) == len(ps["exp"]):      # contributions in the order forward announced them
-            left, ordered = list(pending), []
-            for x in ps["exp"]:
-                hit = next((j for j, (c, _) in enumerate(left) if c.idx == x.data_ptr() and int(c.n) == x.numel()), None)
-                if hit is None:
-                    ordered = None
-                    break
-                ordered.append(left.pop(hit))
-        if ordered is not None:
-            ops.scatter_reduce_sorted(ordered, t.rows, t.d, t.pad_idx, ps["ws"], t.stage_rows, t.stage_n,
-                                      dense_bias_grad=t.bias_grad if want_bias else None, want_rows=True,
-                                      out_red=t.stage_vals)
-        else:
-            ops.scatter_reduce(pending, t.rows, t.d, t.pad_idx, dense_bias_grad=t.bias_grad if want_bias else None,
-                               want_rows=True, device=t.weight.device, out_uniq=t.stage_rows, out_nu=t.stage_n,
-                               out_red=t.stage_vals)
-        if want_bias:
-            t.bias.grad = t.bias_grad
 
 
 class DenseBucket(object):

@@ -62,14 +62,12 @@ def test_no_oracle_or_reference_in_product():
                 assert "/root/reference" not in src, f
 
 
-def test_forked_sink_plumbing_present():
-    """The gradient sinks fork their sort + reduce chains onto side streams and join them in one engine callback;
-    both ends must exist on every sink class (a missing join only shows up on a GPU box)."""
+def test_row_grad_sink_fork_plumbing_present():
+    """The gradient sink forks its sort + reduce chain onto a side stream and joins it in one engine callback;
+    both ends must exist (a missing join only shows up on a GPU box)."""
     from prodsearch_b200 import functional as F_
-    from prodsearch_b200 import peer
     assert callable(F_.run_forked) and callable(F_.RowGradSink._join_forked)
-    for cls in (F_.RowGradSink, peer.PeerGradSink):
-        assert callable(getattr(cls, "_finalize_callback")) and callable(getattr(cls, "finalize"))
+    assert callable(getattr(F_.RowGradSink, "_finalize_callback")) and callable(getattr(F_.RowGradSink, "finalize"))
 
 
 def _prototypes():

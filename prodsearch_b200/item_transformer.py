@@ -9,6 +9,8 @@ negatives: item_transformer.py:447,:268).  Implemented paths: ``forward_dotprodu
 (SURVEY.md 2.1 C1).  New, additive: ``rank_catalog`` (full-catalog top-k without the
 [M, N] matrix) and ``encode_queries``.
 """
+from types import SimpleNamespace
+
 import torch
 import torch.nn as nn
 
@@ -119,36 +121,86 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         self.query_encoder.initialize_parameters(logger)
         self.transformer_encoder.initialize_parameters(logger)
 
+    # ---- where a step or an evaluation reads its rows -----------------------------------
+    def _rows(self, **kw):
+        """Tables, gradient sinks and pad positions the step's kernels read, plus its index lists (``kw``): the model's
+        own tables unless ``kw`` names others (a fetched mini table).  ``fetch``: a side stream the item rows arrive
+        on -- the current stream joins it after query pooling, and the item -> word branch forks behind that join;
+        without one, the hook has already ordered the item -> word stream behind everything it reads.  ``join``: a
+        stream the current stream joins before the ranking loss."""
+        r = dict(item_w=self.product_emb.weight, item_sink=self.item_sink, item_pad=self.prod_pad_idx,
+                 word_w=self.word_embeddings.weight, word_sink=self.word_sink, word_pad=self.word_pad_idx,
+                 fetch=None, join=None)
+        r.update(kw)
+        return SimpleNamespace(**r)
+
+    def _side_stream(self, name):
+        s = getattr(self, name, None)
+        if s is None:
+            s = torch.cuda.Stream(device=self.product_emb.weight.device)
+            setattr(self, name, s)
+        return s
+
+    def _step_rows(self, batch, B, W, K):
+        """Rows and negatives of one training step: the full local tables.  The negatives are drawn on the item -> word
+        stream (see forward_dotproduct)."""
+        tgt, hist = batch.target_prod_idxs, batch.u_item_idxs
+        qw, pw = batch.query_word_idxs, batch.pos_iword_idxs
+        cur = torch.cuda.current_stream(self.product_emb.weight.device)
+        side = self._side_stream("_iw_stream")
+        side.wait_stream(cur)
+        # row-sparse optimizer: the rows this step reads are brought up to date in as few launches as possible
+        # (no-ops for ordinary tables) -- history + target rows and query + target words now, the sampled
+        # negatives on the side branch as soon as they exist; the gather wrappers then find nothing left to do
+        F_.ensure_current(self.hist_product_emb.weight if self.args.sep_prod_emb else self.product_emb.weight, (hist,))
+        F_.ensure_current(self.product_emb.weight, (tgt,))
+        F_.ensure_current(self.word_embeddings.weight, (qw, pw))
+        if self.injected_negatives is None:
+            with torch.cuda.stream(side):
+                neg, nw = self._draw_negatives(B, W, K)
+                F_.ensure_current(self.product_emb.weight, (neg,))
+                F_.ensure_current(self.word_embeddings.weight, (nw,))
+            # (allocated on the side stream and alive until backward has run; the side stream's next allocation
+            # happens after its next wait on the current stream, so the allocator cannot recycle them early)
+        else:
+            neg, nw = self._draw_negatives(B, W, K)
+            side.wait_stream(cur)
+        return self._rows(tgt=tgt, neg=neg, hist=hist, qw=qw, pw=pw, nw=nw)
+
+    def _eval_rows(self, query_word_idxs, item_idxs):
+        """(rows, item_idxs as the rows index them) of an evaluation: the full local tables, every resting row of the
+        row-sparse optimizer replayed first."""
+        self.flush_lazy_rows()
+        return self._rows(qw=query_word_idxs), item_idxs
+
+    def _product_bias(self):
+        return self.product_bias if self.args.sim_func == "bias_product" else None
+
     # ---- shared front half -----------------------------------------------------------
-    def encode_queries(self, query_word_idxs, u_item_idxs, copies=1, hist=None):
-        """Query encoder + [query, purchased items] sequence through the transformer, read at ``out_pos``
-        (item_transformer.py:449-484 / :118-140) -> [B*copies, d], copy-minor.  The history rows are
-        gathered inside the fused encoder kernels.  ``hist`` = (weight, sink, remapped idx, pad idx) when
-        the item table is sharded and the rows live in a fetched mini table."""
-        # the query pooling runs on a side stream; the encoder call enqueues its token plan and weight transposes
-        # (which do not read the pooled queries) and waits for the event only before the kernel that does
-        side = ready = None
-        if self.word_embeddings.weight.is_cuda:
-            if getattr(self, "_q_stream", None) is None:
-                self._q_stream = torch.cuda.Stream(device=self.word_embeddings.weight.device)
-                self._q_ready = torch.cuda.Event()
-            side, ready = self._q_stream, self._q_ready
-        q_emb = self.query_encoder.encode_indices(self.word_embeddings.weight, query_word_idxs, self.word_sink,
-                                                  pad_idx=self.word_pad_idx, stream=side)
-        if ready is not None:
-            ready.record(side)
-        if hist is None:
-            hist_w = self.hist_product_emb.weight if self.args.sep_prod_emb else self.product_emb.weight
-            hist = (hist_w, self.hist_sink, u_item_idxs, self.prod_pad_idx)
+    def _pool_queries(self, r):
+        """Query encoder on a side stream: the encoder call enqueues its token plan and weight transposes (which do not
+        read the pooled queries) and waits for ``_q_ready`` only before the kernel that does."""
+        side = self._side_stream("_q_stream")
+        if getattr(self, "_q_ready", None) is None:
+            self._q_ready = torch.cuda.Event()
+        q_emb = self.query_encoder.encode_indices(r.word_w, r.qw, r.word_sink, pad_idx=r.word_pad, stream=side)
+        self._q_ready.record(side)
+        return q_emb
+
+    def _encode(self, r, q_emb, hist, copies):
+        """[query, purchased items] sequence through the transformer, read at ``out_pos`` (item_transformer.py:449-484
+        / :118-140) -> [B*copies, d], copy-minor.  The history rows are gathered inside the fused encoder kernels."""
+        hist_w, hist_sink = ((self.hist_product_emb.weight, self.hist_sink) if self.args.sep_prod_emb
+                             else (r.item_w, r.item_sink))
         out_pos = -1 if self.args.use_item_pos else 0
         return self.transformer_encoder.encode_position(
-            first=q_emb.contiguous(), table=hist[0], idx=hist[2], sink=hist[1], pad_idx=hist[3],
-            use_pos=self.args.use_pos_emb, out_pos=out_pos, copies=copies, first_ready=ready)
+            first=q_emb.contiguous(), table=hist_w, idx=hist, sink=hist_sink, pad_idx=r.item_pad,
+            use_pos=self.args.use_pos_emb, out_pos=out_pos, copies=copies, first_ready=self._q_ready)
 
-    def _resolve_item_rows(self, target_prod_idxs, neg_item_idxs, u_item_idxs):
-        """(item weight, item sink, target idx, negative idx, hist triple or None) of this step.
-        Single GPU: the full local table.  The sharded subclass fetches a mini table instead."""
-        return self.product_emb.weight, self.item_sink, target_prod_idxs, neg_item_idxs, None
+    def encode_queries(self, query_word_idxs, u_item_idxs, copies=1):
+        """Query encoder + [query, purchased items] sequence through the transformer -> [B*copies, d], copy-minor."""
+        r, (hist,) = self._eval_rows(query_word_idxs, [u_item_idxs])
+        return self._encode(r, self._pool_queries(r), hist, copies)
 
     # ---- training -----------------------------------------------------------------------
     def forward(self, batch_data, train_pv=False):
@@ -180,92 +232,73 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         # word) are never drawn
         return torch.searchsorted(cdf, torch.rand(n, dtype=torch.float64, device=cdf.device), right=True)
 
+    def _loss_sums(self, device):
+        """Lazily synchronised running sums of the two losses (the reference calls .item() here); updated in place, so
+        a CUDA-graph replay keeps accumulating into the same buffers."""
+        if self._ps_acc is None:
+            self._ps_acc = torch.zeros((), device=device)
+            self._item_acc = torch.zeros((), device=device)
+        return self._ps_acc, self._item_acc
+
     def forward_dotproduct(self, batch_data, train_pv=False):
-        query_word_idxs = batch_data.query_word_idxs
-        target_prod_idxs = batch_data.target_prod_idxs
-        u_item_idxs = batch_data.u_item_idxs
-        pos_iword_idxs = batch_data.pos_iword_idxs
-        B, _ = u_item_idxs.shape
+        B, W = batch_data.pos_iword_idxs.shape
         K = self.args.neg_per_pos
-        W = pos_iword_idxs.shape[1]
-        # Neither the negatives nor the item -> word objective are needed by the encoder: the two torch.multinomial
-        # chains (renorm + scan + sample, ~70 us of serialised kernels for two constant distributions) and the item ->
-        # word kernels run on a side stream -- a parallel branch of the captured graph -- and are joined right before
-        # the ranking loss, the first reader of the sampled items.  The draw ORDER on the device generator is the
-        # reference's (items, then words: item_transformer.py:447, :268); only where the kernels are enqueued moves.
-        dev_t = self.product_emb.weight
-        cur = torch.cuda.current_stream(dev_t.device) if dev_t.is_cuda else None
-        side = None
-        if cur is not None:
-            if getattr(self, "_iw_stream", None) is None:
-                self._iw_stream = torch.cuda.Stream(device=dev_t.device)
-            side = self._iw_stream
+        # Where the rows and negatives come from is the model's (_step_rows); the step itself is the same for every
+        # model.  Neither the negatives nor the item -> word objective are needed by the encoder: the negative draws
+        # (two torch.multinomial chains, ~70 us of serialised kernels for two constant distributions) and the
+        # item -> word kernels run on side streams -- parallel branches of the captured graph -- and are joined right
+        # before the ranking loss, the first reader of the sampled items.  The draw ORDER on the device generator is
+        # the reference's (items, then words: item_transformer.py:447, :268), then the query-pooling dropout mask,
+        # then the encoder's dropout key; only where the kernels are enqueued moves.
+        r = self._step_rows(batch_data, B, W, K)
+        cur = torch.cuda.current_stream(r.item_w.device)
+        side = self._side_stream("_iw_stream")
+        # The item -> word branch is launched ahead of query pooling whenever its rows are ready: the order in which
+        # the two create their autograd nodes is the order of their backward kernels and of the word table's gradient
+        # sums.  Rows that arrive on a fetch stream are joined after pooling, which reads only word rows and must not
+        # queue behind the item fetch.
+        if r.fetch is None:
+            item_loss_rows = self._item_word_losses(r, self._word_bias(r), side)
+        q_emb = self._pool_queries(r)
+        if r.fetch is not None:
+            word_bias = self._word_bias(r)
+            cur.wait_stream(r.fetch)        # the item rows are needed by both branches below
             side.wait_stream(cur)
-        sharded = type(self)._resolve_item_rows is not ItemTransformerRanker._resolve_item_rows
-        if not sharded:
-            # row-sparse optimizer: the rows this step reads are brought up to date in as few launches as possible
-            # (no-ops for ordinary tables) -- history + target rows and query + target words now, the sampled
-            # negatives on the side branch as soon as they exist; the gather wrappers then find nothing left to do
-            F_.ensure_current(self.hist_product_emb.weight if self.args.sep_prod_emb else self.product_emb.weight,
-                              (u_item_idxs,))
-            F_.ensure_current(self.product_emb.weight, (target_prod_idxs,))
-            F_.ensure_current(self.word_embeddings.weight, (query_word_idxs, pos_iword_idxs))
-        if side is not None and not sharded and self.injected_negatives is None:
-            with torch.cuda.stream(side):
-                neg_item_idxs, neg_word_idxs = self._draw_negatives(B, W, K)
-                F_.ensure_current(self.product_emb.weight, (neg_item_idxs,))
-                F_.ensure_current(self.word_embeddings.weight, (neg_word_idxs,))
-            # (allocated on the side stream and alive until backward has run; the side stream's next allocation
-            # happens after its next wait on the current stream, so the allocator cannot recycle them early)
-        else:
-            neg_item_idxs, neg_word_idxs = self._draw_negatives(B, W, K)
-            if side is not None:
-                side.wait_stream(cur)
-        item_w, item_sink, tgt_idx, neg_idx, hist = self._resolve_item_rows(target_prod_idxs, neg_item_idxs,
-                                                                            u_item_idxs)
-        if side is not None and sharded:
-            side.wait_stream(cur)                # the fetched mini table is produced on the current stream
-        item_loss_rows = self.item_to_words(tgt_idx, pos_iword_idxs, K, neg_word_idxs, item_w, item_sink, stream=side,
-                                            reduce=False)
+            item_loss_rows = self._item_word_losses(r, word_bias, side)
         stochastic = self.training and self.args.dropout > 0
-        bias = self.product_bias if self.args.sim_func == "bias_product" else None
+        # dropout makes the positive and the K negative encodes differ (transformer.py:56, neural.py:226): 1 + K
+        # dropout draws of the SAME sequence, K/V projections shared between them
+        out = self._encode(r, q_emb, r.hist, 1 + K if stochastic else 1)
+        bias = self._product_bias()
         pos_weight = float(K) if self.args.pos_weight else 1.0
+        cur.wait_stream(side)                # the sampled item negatives and the item -> word losses are ready
+        if r.join is not None:
+            cur.wait_stream(r.join)
+        if stochastic and K <= 7 and self.embedding_size <= 128:
+            # ranking loss on the encoder's output block in place + loss combination and running sums: two launches
+            acc_ps, acc_il = self._loss_sums(out.device)
+            loss = F_.tem_tail(out.view(B, 1 + K, -1), item_loss_rows, r.item_w, r.tgt, r.neg, r.item_sink, bias=bias,
+                               pos_weight=pos_weight, acc_ps=acc_ps, acc_il=acc_il,
+                               src_rows=self._tail_src_rows(B, K, out.device))
+            F_.RowGradSink.mark_forward_end(out.device)     # every index list of the step exists: sorts may start
+            return loss
         if stochastic:
-            # dropout makes the positive and the K negative encodes differ (transformer.py:56, neural.py:226):
-            # 1 + K dropout draws of the SAME sequence, K/V projections shared between them
-            out = self.encode_queries(query_word_idxs, u_item_idxs, copies=1 + K, hist=hist).view(B, 1 + K, -1)
-            if K <= 7 and self.embedding_size <= 128 and out.is_cuda:
-                # ranking loss on the encoder's output block in place + loss combination and running sums: two launches
-                if side is not None:
-                    cur.wait_stream(side)        # sampled item negatives and the item -> word losses are ready
-                if self._ps_acc is None:
-                    self._ps_acc = torch.zeros((), device=out.device)
-                    self._item_acc = torch.zeros((), device=out.device)
-                loss = F_.tem_tail(out, item_loss_rows, item_w, tgt_idx, neg_idx, item_sink, bias=bias,
-                                   pos_weight=pos_weight, acc_ps=self._ps_acc, acc_il=self._item_acc,
-                                   src_rows=self._tail_src_rows(B, K, out.device))
-                F_.RowGradSink.mark_forward_end(out.device)     # every index list of the step exists: sorts may start
-                return loss
+            out = out.view(B, 1 + K, -1)
             pos_out = out[:, 0].contiguous()
             neg_out = out[:, 1:].reshape(B * K, -1)
         else:
             # deterministic encoder: the K copies the reference re-encodes (:473-476) are identical
-            pos_out = self.encode_queries(query_word_idxs, u_item_idxs, hist=hist)
+            pos_out = out
             neg_out = pos_out.unsqueeze(1).expand(-1, K, -1).reshape(B * K, -1)
-        if side is not None:
-            cur.wait_stream(side)                # the sampled item negatives (and the item -> word losses) are ready
-        ps = F_.ns_loss(pos_out.contiguous(), item_w, tgt_idx.view(B, 1), neg_idx.view(B, 1, K), item_sink,
+        ps = F_.ns_loss(pos_out.contiguous(), r.item_w, r.tgt.view(B, 1), r.neg.view(B, 1, K), r.item_sink,
                         anchor_b=neg_out.contiguous(), bias=bias, pos_weight=pos_weight)
         ps_loss = ps.mean()
         item_loss = item_loss_rows.mean()
-        with torch.no_grad():   # lazily synchronised running sums (the reference calls .item() here); in place,
-            if self._ps_acc is None:   # so a CUDA-graph replay keeps accumulating into the same buffers
-                self._ps_acc = torch.zeros((), device=ps_loss.device)
-                self._item_acc = torch.zeros((), device=ps_loss.device)
-            self._ps_acc.add_(ps_loss.detach())
-            self._item_acc.add_(item_loss.detach())
-        if ps_loss.is_cuda:
-            F_.RowGradSink.mark_forward_end(ps_loss.device)
+        with torch.no_grad():
+            acc_ps, acc_il = self._loss_sums(ps_loss.device)
+            acc_ps.add_(ps_loss.detach())
+            acc_il.add_(item_loss.detach())
+        F_.RowGradSink.mark_forward_end(ps_loss.device)
         return ps_loss + item_loss
 
     def _tail_src_rows(self, B, K, device):
@@ -279,20 +312,23 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
             cache = self._tail_rows_cache = (key, (base.contiguous(), neg.contiguous()))
         return cache[1]
 
-    def item_to_words(self, target_prod_idxs, target_word_idxs, n_negs, neg_sample_idxs=None, item_w=None,
-                      item_sink=None, stream=None, reduce=True):
-        """item_transformer.py:260-283.  stream / reduce=False: forward kernels on a side stream the caller forked
-        and joins before reading the per-item losses that are then returned un-averaged."""
+    def item_to_words(self, target_prod_idxs, target_word_idxs, n_negs, neg_sample_idxs=None):
+        """item_transformer.py:260-283 on the local tables."""
         B, W = target_word_idxs.shape
         if neg_sample_idxs is None:
             neg_sample_idxs = self._multinomial("word_dists", B * W * n_negs)
-        if item_w is None:
-            item_w, item_sink = self.product_emb.weight, self.item_sink
-        anchor = F_.gather_rows(item_w, target_prod_idxs, item_sink, stream=stream)
-        loss = F_.ns_loss(anchor, self.word_embeddings.weight, target_word_idxs,
-                          neg_sample_idxs.view(B, W, n_negs), self.word_sink, bias=self.word_bias,
-                          pad_idx=self.word_pad_idx, stream=stream)
-        return loss.mean() if reduce else loss
+        r = self._rows(tgt=target_prod_idxs, pw=target_word_idxs, nw=neg_sample_idxs.view(B, W, n_negs))
+        return self._item_word_losses(r, self.word_bias).mean()
+
+    def _item_word_losses(self, r, word_bias, stream=None):
+        """Per-item losses of the item -> word objective on ``r``'s rows.  stream: the forward kernels run on a side
+        stream the caller forked and joins before reading the losses."""
+        anchor = F_.gather_rows(r.item_w, r.tgt, r.item_sink, stream=stream)
+        return F_.ns_loss(anchor, r.word_w, r.pw, r.nw, r.word_sink, bias=word_bias, pad_idx=r.word_pad, stream=stream)
+
+    def _word_bias(self, r):
+        """The word bias as ``r``'s word rows index it: the bias values at a fetched mini table's positions."""
+        return self.word_bias if r.word_sink.ids is None else _BiasAtFn.apply(self.word_bias, r.word_sink.ids)
 
     # ---- evaluation ---------------------------------------------------------------------
     def test(self, batch_data):
@@ -302,11 +338,11 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         """Scores of an explicit candidate list [B, candi_k] (item_transformer.py:111-146).  The
         encoder output does not depend on the candidate (SURVEY.md 0.4), so it is computed once
         per query instead of candi_k times."""
-        self.flush_lazy_rows()
         with torch.no_grad():
-            q = self.encode_queries(batch_data.query_word_idxs, batch_data.u_item_idxs).contiguous()
-            bias = self.product_bias if self.args.sim_func == "bias_product" else None
-            return ops.score_rows(q, self.product_emb.weight, batch_data.candi_prod_idxs, bias)
+            r, (hist, cand) = self._eval_rows(batch_data.query_word_idxs,
+                                              [batch_data.u_item_idxs, batch_data.candi_prod_idxs])
+            q = self._encode(r, self._pool_queries(r), hist, 1).contiguous()
+            return ops.score_rows(q, r.item_w, cand, self._product_bias())
 
     def _max_row_sqnorm(self):
         """|e|^2 bound of the tensor-core shortlist, cached while the item table is unchanged."""
@@ -316,12 +352,13 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
             self._norm_cache = (key, ops.table_max_row_sqnorm(w, self.prod_pad_idx))
         return self._norm_cache[1]
 
-    def _prepared_catalog(self):
-        """fp16 shortlist copy of the item table, rebuilt when the table changes (evaluation: once)."""
+    def _prepared_catalog(self, n_items):
+        """fp16 shortlist copy of the first ``n_items`` rows of the item table (the whole catalog, or the catalog rows
+        of a shard), rebuilt when the table changes (evaluation: once)."""
         w = self.product_emb.weight
-        key = (w.data_ptr(), w._version, _lib.PARAM_EPOCH[0])      # FusedAdam / graph replays bump the epoch
+        key = (w.data_ptr(), w._version, n_items, _lib.PARAM_EPOCH[0])  # FusedAdam / graph replays bump the epoch
         if getattr(self, "_prep_cache", (None, None))[0] != key:
-            self._prep_cache = (key, ops.catalog_prepare_f16(w.detach(), self.prod_pad_idx))
+            self._prep_cache = (key, ops.catalog_prepare_f16(w.detach(), n_items))
         return self._prep_cache[1]
 
     def rank_catalog(self, batch_or_queries, k=100, mode=_lib.TOPK_TC16):
@@ -330,21 +367,40 @@ class ItemTransformerRanker(F_.LazyFlushMixin, nn.Module):
         mode TOPK_TC16 (default): tcgen05 fp16 shortlist on a cached half-precision copy of the table + exact fp32
         rescoring; TOPK_TC: tf32 shortlist straight from the fp32 table.  Both return exactly what TOPK_EXACT
         returns; shapes they do not cover (and tables that overflow fp16) run the next mode down."""
-        self.flush_lazy_rows()             # row-sparse optimizer: every resting row is replayed before a full scan
         with torch.no_grad():
             if torch.is_tensor(batch_or_queries):
+                self.flush_lazy_rows()     # row-sparse optimizer: every resting row is replayed before a full scan
                 q = batch_or_queries
-            else:
+            else:                          # (encode_queries reads its rows after the same replay)
                 q = self.encode_queries(batch_or_queries.query_word_idxs, batch_or_queries.u_item_idxs)
-            bias = self.product_bias if self.args.sim_func == "bias_product" else None
             prepared = None
             if mode == _lib.TOPK_TC16:
-                prepared = self._prepared_catalog()
+                prepared = self._prepared_catalog(self.prod_pad_idx)
                 if not prepared.fits:
                     mode, prepared = _lib.TOPK_TC, None
             norm = self._max_row_sqnorm() if mode == _lib.TOPK_TC else None
             return ops.catalog_topk(q.contiguous(), self.product_emb.weight, k, n_items=self.prod_pad_idx,
-                                    bias=bias, mode=mode, max_row_sqnorm=norm, prepared=prepared)
+                                    bias=self._product_bias(), mode=mode, max_row_sqnorm=norm, prepared=prepared)
+
+    def _rank_shards(self, batch_or_queries, k, mode, group):
+        """Full-catalog top-k of a row-sharded model (sharded.sharded_rank_catalog): every rank ranks the gathered
+        queries against its shard (global id = rank + G * local row).  Every mode returns the exact mode's lists (the
+        shortlists are rescored in fp32)."""
+        from . import sharded
+
+        def shard_topk(q, kk, id_base, id_stride):
+            n_local = max(0, (self.prod_pad_idx - id_base + id_stride - 1) // id_stride)
+            m, prepared = mode, None
+            if m == _lib.TOPK_TC16:
+                prepared = self._prepared_catalog(n_local)
+                if not prepared.fits:
+                    m, prepared = _lib.TOPK_TC, None
+            return ops.catalog_topk(q, self.product_emb.weight.detach(), kk, n_items=n_local, id_base=id_base,
+                                    id_stride=id_stride, mode=m, prepared=prepared)
+        with torch.no_grad():
+            q = batch_or_queries if torch.is_tensor(batch_or_queries) else self.encode_queries(
+                batch_or_queries.query_word_idxs, batch_or_queries.u_item_idxs)
+            return sharded.sharded_rank_catalog(q.contiguous(), k, shard_topk, ops.topk_merge, group)
 
 
 # the north star names the class ProdSearchModel; the reference's real name is kept as primary
@@ -389,11 +445,21 @@ class ShardedItemTransformerRanker(ItemTransformerRanker):
         self._mini = None
         self._dense = sharded.DenseGradAllReduce(self, skip=("product_emb.weight",), group=group)
 
-    def _resolve_item_rows(self, target_prod_idxs, neg_item_idxs, u_item_idxs):
-        mini, (tgt, neg, hist), pad = self.item_table.fetch([target_prod_idxs, neg_item_idxs, u_item_idxs])
+    def _step_rows(self, batch, B, W, K):
+        """The step's item rows, fetched from their owners into a mini table; the word table is local."""
+        neg, nw = self._draw_negatives(B, W, K)
+        mini, (tgt, neg, hist), pad = self.item_table.fetch([batch.target_prod_idxs, neg, batch.u_item_idxs])
         sink = F_.RowGradSink(mini, pad, None, "dense")
         self._mini = mini
-        return mini, sink, tgt, neg, (mini, sink, hist, pad)
+        # the mini table is produced on the current stream
+        self._side_stream("_iw_stream").wait_stream(torch.cuda.current_stream(mini.device))
+        return self._rows(item_w=mini, item_sink=sink, item_pad=pad, tgt=tgt, neg=neg, hist=hist,
+                          qw=batch.query_word_idxs, pw=batch.pos_iword_idxs, nw=nw)
+
+    def _eval_rows(self, query_word_idxs, item_idxs):
+        with torch.no_grad():
+            mini, idx, pad = self.item_table.fetch(item_idxs)
+        return self._rows(item_w=mini, item_sink=None, item_pad=pad, qw=query_word_idxs), idx
 
     def sync_grads(self):
         if self._mini is not None:
@@ -403,24 +469,8 @@ class ShardedItemTransformerRanker(ItemTransformerRanker):
             self._mini = None
         self._dense.reduce()
 
-    def test_dotproduct(self, batch_data):
-        with torch.no_grad():
-            mini, (cand, hist), pad = self.item_table.fetch([batch_data.candi_prod_idxs, batch_data.u_item_idxs])
-            q = self.encode_queries(batch_data.query_word_idxs, batch_data.u_item_idxs, hist=(mini, None, hist, pad))
-            return ops.score_rows(q.contiguous(), mini, cand, None)
-
     def rank_catalog(self, batch_or_queries, k=100, mode=_lib.TOPK_TC):
-        from . import sharded
-        with torch.no_grad():
-            if torch.is_tensor(batch_or_queries):
-                q = batch_or_queries
-            else:
-                raise NotImplementedError("sharded rank_catalog takes encoded query vectors")
-
-            def topk(qa, w, kk, n_local, base, stride, bias):
-                return ops.catalog_topk(qa, w, kk, n_items=n_local, bias=bias, id_base=base, id_stride=stride, mode=mode)
-            return sharded.sharded_rank_catalog(q.contiguous(), self.item_table, self.prod_pad_idx, k, topk,
-                                                ops.topk_merge)
+        return self._rank_shards(batch_or_queries, k, mode, self._group)
 
 
 class PeerShardedItemTransformerRanker(ItemTransformerRanker):
@@ -485,85 +535,22 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
         return super()._apply(fn, *a, **k)
 
     # ---- training ----------------------------------------------------------------------------------------
-    def forward_dotproduct(self, batch_data, train_pv=False):
-        query_word_idxs = batch_data.query_word_idxs
-        target_prod_idxs = batch_data.target_prod_idxs
-        u_item_idxs = batch_data.u_item_idxs
-        pos_iword_idxs = batch_data.pos_iword_idxs
-        B, _ = u_item_idxs.shape
-        K = self.args.neg_per_pos
-        W = pos_iword_idxs.shape[1]
-        neg_item_idxs, neg_word_idxs = self._negatives_for_step(B, W, K)
-        L = u_item_idxs.shape[1]
+    def _step_rows(self, batch, B, W, K):
+        """The step's item and word rows, gathered from their owners with P2P loads into two mini tables; the item rows
+        travel on a side stream while the word rows are fetched and the queries pooled."""
+        qw, pw = batch.query_word_idxs, batch.pos_iword_idxs
+        (neg, nw), prefetch = self._negatives_for_step(B, W, K)
+        L = batch.u_item_idxs.shape[1]
         self.item_table.reserve_stage(2 * B * (L + 2 + K))                       # collective on first use only
-        self.word_table.reserve_stage(2 * B * (query_word_idxs.shape[1] + W * (1 + K)))
+        self.word_table.reserve_stage(2 * B * (qw.shape[1] + W * (1 + K)))
         self.peer.barrier(0)       # every owner has finished last step's optimizer update / staging reads
-        # the item rows travel on a side stream while the word rows are fetched and the queries pooled
-        if getattr(self, "_fetch_stream", None) is None:
-            self._fetch_stream = torch.cuda.Stream(device=self.peer.device)
-        items, (tgt, neg, hist), item_pad = self.item_table.fetch([target_prod_idxs, neg_item_idxs, u_item_idxs],
-                                                                  stream=self._fetch_stream)
-        words, (qw, pw, nw), word_pad = self.word_table.fetch([query_word_idxs, pos_iword_idxs, neg_word_idxs])
-        isink, wsink = self.item_table.sink, self.word_table.sink
-        cur = torch.cuda.current_stream(self.peer.device)
-        # query pooling on a side stream: the encoder call below enqueues its plan / weight transposes first and
-        # waits for the pooled queries only before the kernel that reads them (psb_encoder_cfg_t.first_ready)
-        if getattr(self, "_q_stream", None) is None:
-            self._q_stream = torch.cuda.Stream(device=self.peer.device)
-            self._q_ready = torch.cuda.Event()
-            self._iw_stream = torch.cuda.Stream(device=self.peer.device)
-        q_emb = self.query_encoder.encode_indices(words, qw, wsink, pad_idx=word_pad, stream=self._q_stream)
-        self._q_ready.record(self._q_stream)
-        wb = self.word_bias
-        bias_mini = None
-        if wb is not None:     # bias values at the mini positions (the bias vector itself is replicated)
-            bias_mini = _BiasAtFn.apply(wb, self.word_table.sink.ids)
-        cur.wait_stream(self._fetch_stream)      # join: the item rows are needed by both branches below
-        # the item -> word objective shares nothing with the encoder: a parallel branch, joined before the sum
-        self._iw_stream.wait_stream(cur)
-        anchor = F_.gather_rows(items, tgt, isink, stream=self._iw_stream)
-        il = F_.ns_loss(anchor, words, pw, nw.view(B, W, K), wsink, bias=bias_mini, pad_idx=word_pad,
-                        stream=self._iw_stream)
-        out_pos = -1 if self.args.use_item_pos else 0
-        stochastic = self.training and self.args.dropout > 0
-        copies = 1 + K if stochastic else 1
-        out = self.transformer_encoder.encode_position(first=q_emb.contiguous(), table=items, idx=hist, sink=isink,
-                                                       pad_idx=item_pad, use_pos=self.args.use_pos_emb,
-                                                       out_pos=out_pos, copies=copies, first_ready=self._q_ready)
-        pos_weight = float(K) if self.args.pos_weight else 1.0
-        if stochastic and K <= 7 and self.embedding_size <= 128:
-            # ranking loss on the encoder's output block in place + loss combination: two launches (see the base class)
-            cur.wait_stream(self._iw_stream)
-            if self._ps_acc is None:
-                self._ps_acc = torch.zeros((), device=out.device)
-                self._item_acc = torch.zeros((), device=out.device)
-            self._join_negative_prefetch(cur)
-            loss = F_.tem_tail(out.view(B, 1 + K, -1), il, items, tgt, neg, isink, pos_weight=pos_weight,
-                               acc_ps=self._ps_acc, acc_il=self._item_acc,
-                               src_rows=self._tail_src_rows(B, K, out.device))
-            F_.RowGradSink.mark_forward_end(out.device)
-            return loss
-        self._join_negative_prefetch(cur)
-        if stochastic:
-            out = out.view(B, 1 + K, -1)
-            pos_out = out[:, 0].contiguous()
-            neg_out = out[:, 1:].reshape(B * K, -1)
-        else:
-            pos_out = out
-            neg_out = pos_out.unsqueeze(1).expand(-1, K, -1).reshape(B * K, -1)
-        ps = F_.ns_loss(pos_out.contiguous(), items, tgt.view(B, 1), neg.view(B, 1, K), isink,
-                        anchor_b=neg_out.contiguous(), pos_weight=pos_weight)
-        ps_loss = ps.mean()
-        cur.wait_stream(self._iw_stream)
-        item_loss = il.mean()
-        with torch.no_grad():
-            if self._ps_acc is None:
-                self._ps_acc = torch.zeros((), device=ps_loss.device)
-                self._item_acc = torch.zeros((), device=ps_loss.device)
-            self._ps_acc.add_(ps_loss.detach())
-            self._item_acc.add_(item_loss.detach())
-        F_.RowGradSink.mark_forward_end(ps_loss.device)
-        return ps_loss + item_loss
+        fetch = self._side_stream("_fetch_stream")
+        items, (tgt, neg, hist), item_pad = self.item_table.fetch([batch.target_prod_idxs, neg, batch.u_item_idxs],
+                                                                  stream=fetch)
+        words, (qw, pw, nw), word_pad = self.word_table.fetch([qw, pw, nw])
+        return self._rows(item_w=items, item_sink=self.item_table.sink, item_pad=item_pad, word_w=words,
+                          word_sink=self.word_table.sink, word_pad=word_pad, tgt=tgt, neg=neg, hist=hist, qw=qw, pw=pw,
+                          nw=nw, fetch=fetch, join=prefetch)
 
     # The sharded step needs the sampled negatives before anything else (their rows are part of the peer fetch), so the
     # two torch.multinomial chains (~70 us of serialised kernels) would sit at the head of its critical path.  The
@@ -571,10 +558,10 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
     # longer) into a second pair of buffers and copied into the live pair at the start of step t + 1.  Same generator,
     # same draw order (items, words, items, words, ...); each draw is merely issued one step early.
     def _negatives_for_step(self, B, W, K):
+        """((item negatives, word negatives), the side stream of the next step's draws to join before the ranking loss
+        or None)."""
         if self.injected_negatives is not None or not self.training:
-            self._neg_fork = None
-            ni, nw = self._draw_negatives(B, W, K)
-            return ni, nw
+            return self._draw_negatives(B, W, K), None
         dev = self.peer.device
         key = (B, W, K)
         if getattr(self, "_neg_key", None) != key:
@@ -599,14 +586,7 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
             self._neg_next[0].copy_(ni)
             self._neg_next[1].copy_(nw)
         self._neg_ready = True
-        self._neg_fork = st
-        return self._neg_cur
-
-    def _join_negative_prefetch(self, cur):
-        st = getattr(self, "_neg_fork", None)
-        if st is not None:
-            cur.wait_stream(st)
-            self._neg_fork = None
+        return self._neg_cur, st
 
     def sync_grads(self, optim=None):
         """Between ``loss.backward()`` and ``optim.step()`` (all ranks): fold the peers' gradient lists into the
@@ -697,68 +677,15 @@ class PeerShardedItemTransformerRanker(ItemTransformerRanker):
                                                    _lib.stream_ptr()), "psb_peer_sum_sqnorm")
 
     # ---- evaluation -----------------------------------------------------------------------------------------
-    def encode_queries(self, query_word_idxs, u_item_idxs, copies=1, hist=None):
+    def _eval_rows(self, query_word_idxs, item_idxs):
         with torch.no_grad():
-            items, (h,), item_pad = self.item_table.fetch([u_item_idxs])
+            items, idx, item_pad = self.item_table.fetch(item_idxs)
             words, (qw,), word_pad = self.word_table.fetch([query_word_idxs])
-            q_emb = self.query_encoder.encode_indices(words, qw, None, pad_idx=word_pad)
-            out_pos = -1 if self.args.use_item_pos else 0
-            return self.transformer_encoder.encode_position(first=q_emb.contiguous(), table=items, idx=h, sink=None,
-                                                            pad_idx=item_pad, use_pos=self.args.use_pos_emb,
-                                                            out_pos=out_pos, copies=copies)
-
-    def test_dotproduct(self, batch_data):
-        with torch.no_grad():
-            q = self.encode_queries(batch_data.query_word_idxs, batch_data.u_item_idxs).contiguous()
-            items, (cand,), _ = self.item_table.fetch([batch_data.candi_prod_idxs])
-            return ops.score_rows(q, items, cand, None)
-
-    def _shard_topk(self, q, k, n_local, id_base, id_stride, mode):
-        """Top-k of this rank's shard; TOPK_TC16 uses a cached fp16 copy of the shard (rebuilt when it changes)."""
-        w = self.item_table.weight.detach()
-        prepared = None
-        if mode == _lib.TOPK_TC16:
-            key = (w.data_ptr(), self.item_table.weight._version, n_local, _lib.PARAM_EPOCH[0])
-            if getattr(self, "_shard_prep", (None, None))[0] != key:
-                self._shard_prep = (key, ops.catalog_prepare_f16(w, n_local))
-            prepared = self._shard_prep[1]
-            if not prepared.fits:
-                mode, prepared = _lib.TOPK_TC, None
-        return ops.catalog_topk(q, w, k, n_items=n_local, id_base=id_base, id_stride=id_stride, mode=mode,
-                                prepared=prepared)
+        return self._rows(item_w=items, item_sink=None, item_pad=item_pad, word_w=words, word_sink=None,
+                          word_pad=word_pad, qw=qw), idx
 
     def rank_catalog(self, batch_or_queries, k=100, mode=_lib.TOPK_TC16):
-        """Sharded full-catalog top-k: every rank scores the all-gathered queries against its shard
-        (id = rank + G * local row), the per-shard lists are all-gathered and merged (psb_topk_merge).
-        Every mode returns the exact mode's lists (the shortlists are rescored in fp32)."""
-        import torch.distributed as dist
-        with torch.no_grad():
-            q = batch_or_queries if torch.is_tensor(batch_or_queries) else self.encode_queries(
-                batch_or_queries.query_word_idxs, batch_or_queries.u_item_idxs)
-            q = q.contiguous()
-            G, r = self.peer.world, self.peer.rank
-            n_local = max(0, (self.prod_pad_idx - r + G - 1) // G)
-            if G == 1:
-                return self._shard_topk(q, k, n_local, 0, 1, mode)
-            # every collective lands in its final layout (all_gather_into_tensor): no list gathers, no cat / stack
-            m = torch.tensor([q.shape[0]], device=q.device)
-            ms = torch.empty(G, dtype=m.dtype, device=q.device)
-            dist.all_gather_into_tensor(ms, m, group=self.peer.group)
-            m_max = int(ms.max())
-            q_pad = q
-            if q.shape[0] != m_max:
-                q_pad = q.new_zeros((m_max, q.shape[1]))
-                q_pad[:q.shape[0]] = q
-            q_all = torch.empty((G * m_max, q.shape[1]), dtype=q.dtype, device=q.device)
-            dist.all_gather_into_tensor(q_all, q_pad, group=self.peer.group)
-            ids, sc = self._shard_topk(q_all, k, n_local, r, G, mode)
-            ids_all = torch.empty((G, G * m_max, k), dtype=ids.dtype, device=q.device)
-            sc_all = torch.empty((G, G * m_max, k), dtype=sc.dtype, device=q.device)
-            dist.all_gather_into_tensor(ids_all.view(-1, k), ids, group=self.peer.group)
-            dist.all_gather_into_tensor(sc_all.view(-1, k), sc, group=self.peer.group)
-            mi, ms_ = ops.topk_merge(ids_all, sc_all)
-            lo = r * m_max
-            return mi[lo:lo + q.shape[0]], ms_[lo:lo + q.shape[0]]
+        return self._rank_shards(batch_or_queries, k, mode, self.peer.group)
 
 
 class _BiasAtFn(torch.autograd.Function):

@@ -15,7 +15,7 @@ Duplicated ids (popular items) cross NVLink once per rank per step instead of on
 
 Evaluation: every rank scores the (all-gathered) queries against its shard with
 ``psb_catalog_topk`` (id_base = rank, id_stride = G), the per-shard top-k lists are all-gathered
-and merged by ``psb_topk_merge`` (``sharded_rank_catalog``).
+and merged by ``psb_topk_merge`` (``sharded_rank_catalog``; the peer-sharded model uses it too).
 
 The exchange logic is backend-agnostic: row gather / gradient fold are injected callables, so the
 CPU test-suite drives it with gloo (world_size 2) while the product passes the CUDA ops.
@@ -92,10 +92,6 @@ class ShardedTable(object):
             t.weight.copy_(full[t.rank::t.world].to(device))
         return t
 
-    def local_item_count(self, n_items):
-        """Number of local rows whose global id is < n_items (catalog candidates on this shard)."""
-        return max(0, (n_items - self.rank + self.world - 1) // self.world)
-
     def fetch(self, index_tensors):
         """Unique the ids of ``index_tensors``, fetch their rows from the owners.
         Returns (mini_table [u, d] leaf tensor, remapped index tensors, remapped pad index or -1)."""
@@ -134,23 +130,30 @@ class ShardedTable(object):
         self._last = None
 
 
-def sharded_rank_catalog(queries, table, n_items, k, topk_fn, merge_fn, bias_local=None):
-    """Full-catalog top-k over a row-sharded table.  queries [m_local, d] of this rank.
-    topk_fn(q, weight, k, n_local, id_base, id_stride, bias) -> (ids, scores); merge_fn(ids[g,m,k], scores)."""
-    world, rank = table.world, table.rank
-    m_counts = [None] * world
-    dist.all_gather_object(m_counts, int(queries.shape[0]), group=table.group)
-    m_max = max(m_counts)
-    q_pad = queries.new_zeros((m_max, queries.shape[1]))
-    q_pad[:queries.shape[0]] = queries
-    gathered = [torch.empty_like(q_pad) for _ in range(world)]
-    dist.all_gather(gathered, q_pad, group=table.group)
-    q_all = torch.cat(gathered, dim=0)                                 # [world * m_max, d]
-    ids, scores = topk_fn(q_all, table.weight.detach(), k, table.local_item_count(n_items), rank, world, bias_local)
-    ids_all = [torch.empty_like(ids) for _ in range(world)]
-    sc_all = [torch.empty_like(scores) for _ in range(world)]
-    dist.all_gather(ids_all, ids, group=table.group)
-    dist.all_gather(sc_all, scores, group=table.group)
-    mi, ms = merge_fn(torch.stack(ids_all), torch.stack(sc_all))       # [world * m_max, k]
+def sharded_rank_catalog(queries, k, shard_topk, merge_fn, group=None):
+    """Full-catalog top-k over a row-sharded table (owner = id % G).  queries [m, d]: this rank's, m may differ from
+    rank to rank.  Every rank scores the queries of all ranks against its shard,
+    ``shard_topk(q_all, k, id_base=rank, id_stride=G) -> (ids, scores)``; the per-shard lists are gathered into
+    [G, G * m_max, k] and merged, ``merge_fn(ids, scores) -> (ids, scores)`` [G * m_max, k].  Every collective lands
+    in its final layout (all_gather_into_tensor): no host pickles, no list gathers, no cat / stack copies."""
+    world, rank = _world(group)
+    if world == 1:
+        return shard_topk(queries, k, 0, 1)
+    m = torch.tensor([queries.shape[0]], device=queries.device)
+    ms = torch.empty(world, dtype=m.dtype, device=queries.device)
+    dist.all_gather_into_tensor(ms, m, group=group)
+    m_max = int(ms.max())
+    q_pad = queries
+    if queries.shape[0] != m_max:
+        q_pad = queries.new_zeros((m_max, queries.shape[1]))
+        q_pad[:queries.shape[0]] = queries
+    q_all = queries.new_empty((world * m_max, queries.shape[1]))
+    dist.all_gather_into_tensor(q_all, q_pad, group=group)
+    ids, sc = shard_topk(q_all, k, rank, world)
+    ids_all = ids.new_empty((world, world * m_max, k))
+    sc_all = sc.new_empty((world, world * m_max, k))
+    dist.all_gather_into_tensor(ids_all.view(-1, k), ids, group=group)
+    dist.all_gather_into_tensor(sc_all.view(-1, k), sc, group=group)
+    mi, ms_ = merge_fn(ids_all, sc_all)
     lo = rank * m_max
-    return mi[lo:lo + queries.shape[0]], ms[lo:lo + queries.shape[0]]
+    return mi[lo:lo + queries.shape[0]], ms_[lo:lo + queries.shape[0]]

@@ -78,15 +78,19 @@ def _worker(rank, world, port, out):
         qtab[10:20] = qtab[3]
         t2b = sharded.ShardedTable.from_full(qtab, None, _cpu_gather, _cpu_fold, "cpu", pad_idx=P)
 
-        def topk(qa, w, kk, n_local, base, stride, bias):
+        def topk(qa, kk, base, stride):
+            assert (base, stride) == (rank, world)
+            n_local = (P - base + stride - 1) // stride
+            w = t2b.weight.detach()
             ids = base + stride * torch.arange(n_local)
             i, s_ = oracle.topk_lower_id_first((qa @ w[:n_local].t()).numpy(), kk, np.tile(ids.numpy(), (qa.shape[0], 1)))
             return torch.from_numpy(i), torch.from_numpy(s_)
 
         def merge(ids, sc):
+            assert ids.shape == (world, world * (3 + world - 1), k)
             i, s_ = oracle.merge_shard_topk(list(ids.numpy()), list(sc.numpy()), k)
             return torch.from_numpy(i), torch.from_numpy(s_)
-        ids, sc = sharded.sharded_rank_catalog(q, t2b, P, k, topk, merge)
+        ids, sc = sharded.sharded_rank_catalog(q, k, topk, merge)
         ref_i, ref_s = oracle.topk_lower_id_first((q @ qtab[:P].t()).numpy(), k)
         assert np.array_equal(ids.numpy(), ref_i) and np.array_equal(sc.numpy(), ref_s)
         # replicated-parameter gradient averaging
@@ -106,7 +110,7 @@ def _worker(rank, world, port, out):
 
 
 @pytest.mark.timeout(180)
-def test_sharded_table_world2_gloo():
+def test_sharded_table_and_ranking_world2_gloo():
     world = 2
     ctx = mp.get_context("spawn")
     out = ctx.Queue()

@@ -309,7 +309,11 @@ int psb_topk_merge(const int64_t* ids, const float* scores, int64_t g, int64_t m
  * Dropout uses Philox4x32-10 keyed by *seed_dev (device uint64; a CUDA-graph replay sees the new
  * seed), stream 1..4 = {attention, context, ff inner, ff output}, element index as laid out
  * above; p_drop == 0 disables it.  All arithmetic fp32 (FFMA), fixed summation order.
- * Shapes supported: d % 4 == 0, d <= 128, ff % 4 == 0, ff <= 1024, T <= 64, d % heads == 0. */
+ * Shapes supported: d % 4 == 0, d <= 128, ff % 4 == 0, ff <= 1024, T <= 64, d % heads == 0, heads <= 32,
+ * copies <= 24.  The backward tail keeps the attention scores of a tile of R >= copies rows (R in {16, 20, 24}) in
+ * shared memory, which bounds heads * T; past it the calls return PSB_E_UNSUPPORTED.  At d = 128, ff = 512 the
+ * bound is heads * T <= 847 for copies <= 16, <= 511 for copies <= 20 and <= 282 for copies <= 24 (8 heads: any
+ * T <= 64 up to 20 copies, T <= 35 at 21..24 copies). */
 typedef struct psb_encoder_params {
   /* nn.Linear layout [out, in]; names follow models/neural.py / models/transformer.py */
   const float *wq, *bq, *wk, *bk, *wv, *bv, *wo, *bo;

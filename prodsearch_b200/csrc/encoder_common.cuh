@@ -271,8 +271,8 @@ __device__ __forceinline__ float gelu_tanh_grad(float x) {
 // ------------------------------------------------------------------ problem dimensions + saved state
 struct Dims {
   int S, T, d, H, dh, F, C, o, pre_ln;
-  int R;     // tile rows of the per-copy kernels (16 or 24)
-  int spt;   // sequences per tile = R / C (>= 1)
+  int R;     // tile rows of the per-copy kernels (16, 20 or 24)
+  int spt;   // sequences per tile: R / C, or fewer where shared memory runs out (dims_from_cfg; >= 1)
   int ntile; // ceil(S / spt)
   float eps, qscale;
   uint32_t thr;

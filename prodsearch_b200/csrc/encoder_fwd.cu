@@ -46,23 +46,30 @@ int dims_from_cfg(const psb_encoder_cfg_t* c, Dims* D) {
   // tile rows R (whole sequences per tile, spt = R / copies): the tail kernels run one CTA per SM whose time is
   // ~ (fixed latency + R), so pick the R in {16, 20, 24} with the least waves * (R + 10).  At the reference's
   // 1 + 5 copies and batch 384: R = 20 -> 128 tiles in one wave (R = 24: 96 tiles on 148 SMs; R = 16: two waves).
+  // Long sequences or many heads (e.g. T >= 57 at d = 128, ff = 512, 8 heads, 1 copy) can leave no R whose backward
+  // tail holds R / copies sequences' scores in shared memory: only then does each R take as many sequences as fit
+  // (rused = spt * C < R), so every shape accepted at full spt keeps its tiling.
   const size_t smem_cap = 227 * 1024;
-  int best_R = 0;
+  int best_R = 0, best_spt = 0;
   long best_cost = 0;
-  for (int R = 16; R <= 24; R += 4) {
-    const int spt = R / D->C;
-    if (spt == 0) continue;
-    if (tail_bwd_smem_floats(R, D->d, D->F, D->H, D->T, spt) * sizeof(float) > smem_cap) continue;
-    const long tiles = (D->S + spt - 1) / spt;
-    const long cost = ((tiles + kNumSMs - 1) / kNumSMs) * (R + 10);
-    if (best_R == 0 || cost < best_cost) {
-      best_R = R;
-      best_cost = cost;
+  for (int lowered = 0; lowered < 2 && best_R == 0; ++lowered) {
+    for (int R = 16; R <= 24; R += 4) {
+      int spt = R / D->C;
+      auto fits = [&](int n) { return tail_bwd_smem_floats(R, D->d, D->F, D->H, D->T, n) * sizeof(float) <= smem_cap; };
+      while (lowered && spt > 0 && !fits(spt)) --spt;
+      if (spt == 0 || !fits(spt)) continue;
+      const long tiles = (D->S + spt - 1) / spt;
+      const long cost = ((tiles + kNumSMs - 1) / kNumSMs) * (R + 10);
+      if (best_R == 0 || cost < best_cost) {
+        best_R = R;
+        best_spt = spt;
+        best_cost = cost;
+      }
     }
   }
   if (best_R == 0) return PSB_E_UNSUPPORTED;
   D->R = best_R;
-  D->spt = best_R / D->C;
+  D->spt = best_spt;
   D->ntile = (D->S + D->spt - 1) / D->spt;
   D->eps = c->ln_eps;
   D->qscale = 1.f / sqrtf(static_cast<float>(D->dh));

@@ -414,8 +414,12 @@ int psb_grad_sqnorm(const psb_adam_tensor_t* tensors /* host; only g and n are r
  * a step touches, with DENSE-EQUIVALENT results: a row that rests for k steps is brought up to date when it is next read or
  * updated -- with a zero gradient its moments decay geometrically, so the skipped updates are a series with
  * independent terms: the first min(k, psb_adam_catchup_steps) are summed with each step's own coefficients (they
- * shrink like (b1/sqrt(b2))^j and are below 1e-9 of the first one after that), the moments decay in closed form.  weight_decay is not supported here (use psb_adam_step).  The global clip norm is taken over the dense
- * tensors' gradients plus the compact row gradients (all other rows have gradient zero). */
+ * shrink like (b1/sqrt(b2))^j and are below 1e-9 of the first one after that), the moments decay in closed form by
+ * the factors a dense step applies, (1 - fl(1-b1))^k and fl(b2)^k.  A step in which a table has no row list (it is
+ * not passed, or has no valid entry) is a zero-gradient step for all of its rows, as in a dense step with a zero
+ * gradient.  last_step == 0 means "never updated, moments zero": a caller that restores moments from a checkpoint
+ * taken at step t stamps every row with t.  weight_decay is not supported here (use psb_adam_step).  The global clip
+ * norm is taken over the dense tensors' gradients plus the compact row gradients (all other rows have gradient zero). */
 typedef struct psb_adam_rows {
   float* p;                /* [table_rows, d] the table                                                      */
   float* m;                /* [table_rows, d] exp_avg                                                        */
@@ -444,7 +448,8 @@ int64_t psb_adam_sparse_workspace_bytes(const psb_adam_tensor_t* dense /* host *
                                         const psb_adam_rows_t* tables /* host */, int32_t n_tables);
 /* One optimizer step: dense tensors exactly as psb_adam_step, tables through their row lists.  coef_hist: device
  * array of coef_cap float2 (8-byte aligned) the call appends this step's (lr_t / (1 - b1^t), 1 / sqrt(1 - b2^t)) to
- * and reads earlier steps' values from (steps >= coef_cap are recomputed on the fly); may be NULL.  norm_given as in
+ * -- also when n_tables == 0 -- and reads earlier steps' values from (steps >= coef_cap are recomputed on the fly);
+ * may be NULL.  Every step of a run that catches rows up through coef_hist must pass it.  norm_given as in
  * psb_adam_step. */
 int psb_adam_sparse_step(const psb_adam_tensor_t* dense /* host */, int32_t n_dense,
                          const psb_adam_rows_t* tables /* host */, int32_t n_tables, double lr, double beta1,

@@ -9,6 +9,7 @@ namespace psb {
 struct AdamHyper {  // the reference's hyper-parameters are Python doubles: 1 - beta is formed in double, then rounded
   double lr, beta1, beta2;
   float b1, b2, omb1, omb2, eps, max_norm, weight_decay;
+  float l2b1;        // log2(1 - omb1) of the exact double: m decays by 1 - omb1 per zero-gradient step (lerp), not b1
   int noam;
   float warmup;
 };
@@ -49,7 +50,7 @@ __device__ __forceinline__ StepCoef load_coef(const AdamHyper& h, const float2* 
 __device__ __forceinline__ float4 catchup_series4(const float4& m, const float4& v, int64_t from, int nterm,
                                                   const AdamHyper& h, const float2* __restrict__ hist, int64_t hist_cap) {
   const int lane = threadIdx.x & 31;
-  const float l2b1 = log2f(h.b1), hl2b2 = 0.5f * log2f(h.b2);
+  const float l2b1 = h.l2b1, hl2b2 = 0.5f * log2f(h.b2);
   const float4 s = make_float4(sqrtf(v.x), sqrtf(v.y), sqrtf(v.z), sqrtf(v.w));
   float4 acc = zero4();
   for (int j0 = 0; j0 < nterm; j0 += 32) {
@@ -84,6 +85,7 @@ inline AdamHyper make_adam_hyper(double lr, double beta1, double beta2, double e
   h.b2 = static_cast<float>(beta2);
   h.omb1 = static_cast<float>(1.0 - beta1);
   h.omb2 = static_cast<float>(1.0 - beta2);
+  h.l2b1 = static_cast<float>(log2(1.0 - static_cast<double>(h.omb1)));
   h.eps = static_cast<float>(eps);
   h.max_norm = static_cast<float>(max_grad_norm);
   h.weight_decay = static_cast<float>(weight_decay);

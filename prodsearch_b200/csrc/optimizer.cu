@@ -175,7 +175,7 @@ __global__ void __launch_bounds__(256) adam_kernel(const AdamTensors T, const Ad
 // are summed with the per-step coefficients of the history table (they fall like (b1 / sqrt(b2))^j: 1e-9 of the first
 // one after catchup_max = 198 steps at the reference's betas, far below fp32 resolution of the parameter), the
 // moments decay in closed form over the whole rest.  The result equals the dense sweep within fp32 rounding
-// (tests/test_gpu_sparse_adam.py holds it to the same tolerance as the dense kernel against torch.optim.Adam).
+// (tests/test_gpu_adam_fp64.py holds it to a float64 replay of the dense steps).
 // weight_decay must be 0 (a decayed row never rests).
 struct RowTables {
   psb_adam_rows_t t[PSB_ADAM_MAX_ROW_TABLES];
@@ -196,9 +196,10 @@ __device__ void catchup_row(const psb_adam_rows_t& t, int64_t r, int64_t from, i
   const int d4 = static_cast<int>(t.d >> 2);
   const int64_t gap = to - from;
   const int nterm = static_cast<int>(gap < catchup_max ? gap : catchup_max);
-  const float m_dec = static_cast<float>(pow(h.beta1, static_cast<double>(gap)));
-  const float v_dec = static_cast<float>(pow(h.beta2, static_cast<double>(gap)));
-  const float l2b1 = log2f(h.b1), hl2b2 = 0.5f * log2f(h.b2);
+  // the bases the dense step applies: m *= 1 - fl(1 - beta1) (lerp), v *= fl(beta2)
+  const float m_dec = static_cast<float>(pow(1.0 - static_cast<double>(h.omb1), static_cast<double>(gap)));
+  const float v_dec = static_cast<float>(pow(static_cast<double>(h.b2), static_cast<double>(gap)));
+  const float l2b1 = h.l2b1, hl2b2 = 0.5f * log2f(h.b2);
   float4* p4 = reinterpret_cast<float4*>(t.p + r * t.d);
   float4* m4 = reinterpret_cast<float4*>(t.m + r * t.d);
   float4* v4 = reinterpret_cast<float4*>(t.v + r * t.d);
@@ -367,7 +368,7 @@ __device__ __forceinline__ AdamCoef make_coef(const AdamHyper& h, const float* s
 // The update of the step's touched rows: one warp per list entry.  The row is first caught up to step - 1 (normally
 // a no-op: the forward pass read the row, so psb_adam_rows_catchup has already run for it), then takes the ordinary
 // Adam update with its reduced gradient and is stamped with the new step.  Block 0 also appends the step's
-// coefficients to the history table.
+// coefficients to the history table (also when no table has a list this step: the launch then has one block).
 __global__ void __launch_bounds__(256) adam_rows_kernel(const RowTables R, const AdamHyper h,
                                                         const float* __restrict__ sqnorm,
                                                         const int64_t* __restrict__ step_dev, float2* __restrict__ hist,
@@ -474,19 +475,7 @@ extern "C" int psb_adam_step(const psb_adam_tensor_t* tensors, int32_t n_tensors
     sqnorm_final_kernel<<<1, 256, 0, s>>>(partial, static_cast<int>(chunks), sqnorm_dev, step_dev);
     if ((st = launch_status()) != PSB_OK) return st;
   }
-  AdamHyper h;
-  h.lr = lr;
-  h.beta1 = beta1;
-  h.beta2 = beta2;
-  h.b1 = static_cast<float>(beta1);
-  h.b2 = static_cast<float>(beta2);
-  h.omb1 = static_cast<float>(1.0 - beta1);
-  h.omb2 = static_cast<float>(1.0 - beta2);
-  h.eps = static_cast<float>(eps);
-  h.max_norm = static_cast<float>(max_grad_norm);
-  h.weight_decay = static_cast<float>(weight_decay);
-  h.noam = noam;
-  h.warmup = static_cast<float>(warmup_steps);
+  const AdamHyper h = make_adam_hyper(lr, beta1, beta2, eps, weight_decay, max_grad_norm, noam, warmup_steps);
   PSB_PROF("adam_kernel", s);
   adam_kernel<<<static_cast<int>(chunks), 256, 0, s>>>(T, h, sqnorm_dev, step_dev);
   return launch_status();
@@ -616,6 +605,9 @@ extern "C" int psb_adam_sparse_step(const psb_adam_tensor_t* dense, int32_t n_de
     adam_kernel<<<static_cast<int>(chunks), 256, 0, s>>>(T, h, sqnorm_dev, step_dev);
     if ((st = launch_status()) != PSB_OK) return st;
   }
+  // A step in which a table has no row list is a zero-gradient step for all its rows: its coefficients still go into
+  // the history (block 0 writes them; a block without a table returns), or a later catch-up would skip that step.
+  if (ublocks == 0 && coef_hist != nullptr) ublocks = 1;
   if (ublocks > 0) {
     PSB_PROF("adam_rows_kernel", s);
     adam_rows_kernel<<<static_cast<int>(ublocks), 256, 0, s>>>(R, h, sqnorm_dev, step_dev,

@@ -91,18 +91,20 @@ class GraphedTrainStep(object):
                 p.copy_(v)
             opt = getattr(self.optim, "optimizer", None)
             if opt is not None and hasattr(opt, "_step_dev"):
-                for p, st in opt.state.items():
-                    old = snap["opt_state"].get(p) or {}
-                    for k, v in st.items():          # exp_avg, exp_avg_sq, (row-sparse tables) last_step
-                        if k in old:
-                            v.copy_(old[k])
-                        else:
-                            v.zero_()
                 if opt._step_dev is not None:
                     if snap["opt_step"] is None:
                         opt._step_dev.zero_()
                     else:
                         opt._step_dev.copy_(snap["opt_step"])
+                for p, st in opt.state.items():
+                    old = snap["opt_state"].get(p) or {}
+                    for k, v in st.items():          # exp_avg, exp_avg_sq, (row-sparse tables) last_step
+                        if k in old:
+                            v.copy_(old[k])
+                        elif k == "last_step":       # created by the warm-up: every row is current at the restored step
+                            v.copy_(opt._step_dev.expand_as(v))
+                        else:
+                            v.zero_()
             elif opt is not None:
                 opt.load_state_dict(snap["opt_state"])
             if hasattr(self.optim, "_step"):

@@ -11,7 +11,10 @@ device memory (CUDA-graph replayable):
     within fp32 rounding; the step costs O(rows touched), not O(table).
 
 Known difference from torch.optim.Adam: ONE step counter for all tensors (torch keeps one per parameter; they only
-differ for a parameter that receives its first gradient later than the others -- none does in these models)."""
+differ for a parameter that receives its first gradient later than the others -- none does in these models).
+A step in which a row-sparse table receives no row list (its gradient is None) is a zero-gradient step for every row of
+that table -- its moments decay and its rows move, as in a dense step with a zero gradient -- whereas torch.optim.Adam
+would leave a parameter without a gradient untouched."""
 import torch
 from torch.nn.utils import clip_grad_norm_
 
@@ -79,7 +82,9 @@ class FusedAdam(object):
         """psb_adam_rows_t of table parameter ``p`` (+ the bias vector indexed like it) and the tensors it points to."""
         st = self._state_of(p)
         if "last_step" not in st:
-            st["last_step"] = torch.zeros(p.shape[0], dtype=torch.int32, device=p.device)
+            # every row is current at the optimizer's step: 0 in a fresh run, the checkpoint's step after a resume (a
+            # stamp of 0 would read as "never updated" and the row's resting steps would not be replayed)
+            st["last_step"] = self._step_stamps(p.shape[0], p.device)
         bias = getattr(p, "_psb_row_bias", None)
         if bias is not None and not bias.requires_grad:
             bias = None
@@ -105,6 +110,11 @@ class FusedAdam(object):
                 R.bias_grad = bg[1].data_ptr()
                 keep.append(bg[1])
         return R, keep, bias
+
+    def _step_stamps(self, n, device):
+        """int32 [n] holding the current step: a stream-ordered copy of the device counter, no host sync."""
+        self._ensure(device)
+        return self._step_dev.to(torch.int32).expand(n).clone()
 
     def _hyper(self):
         g = self.param_groups[0]
